@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — candidates/s of the DAN forward (BASELINE.json metric) on N B200s, one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--precision bf16|fp32] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--precision bf16|fp32] [--batch B] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (encoder -> conv stack -> pooling -> FC -> heads, dl4vc/model.py:434-961) over one
 batch of B synthetic PROD-shaped pileup candidates (100 reads x 201 positions, all read rows populated = the dense
@@ -18,6 +18,14 @@ worst case). Candidates are independent, so N GPUs shard by candidate with no co
 
 The per-step batch (default 4144 candidates = 252 MB of uint8 input) is larger than the 126 MB L2, so no L2 flush is
 needed between timed iterations.
+
+--dump-outputs DIR writes the (B,27) fp32 head matrix of the last timed `value` step to DIR/heads.npy (DIR/heads_rank<r>.npy
+per rank under torchrun). Inputs and weights are seeded, so two builds run with the same arguments can be compared output for
+output. The dump stays within 64 MB in all: a rank's head matrix above 64 MB / N (N ranks) is cut to a fixed, seeded sample of its
+rows (the same rows in every run of that batch size and rank count).
+
+--steps K times K steps in every region that times this project's code (value, e2e, the profile pass, the fp32 and train blocks);
+the CPU and torch-eager samples of the reference op sequence are baselines of fixed size.
 """
 from __future__ import annotations
 
@@ -345,6 +353,19 @@ def train_step_block(cfg, sd, dev, dist, world, rank, timed, batch=32, steps=3, 
             "last_losses[bin,vt,af,cov,vb,vr,total,n_close]": loss}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, name, arr, limit=DUMP_LIMIT_BYTES):
+    """arr (rows x cols float32, host) -> out_dir/<name>.npy, above `limit` bytes a seeded row sample in ascending row order."""
+    import numpy as np
+    if arr.nbytes > limit:
+        keep = limit // (arr.shape[1] * arr.itemsize)
+        arr = arr[np.sort(np.random.default_rng(0).choice(arr.shape[0], keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(arr, dtype=np.float32))
+
+
 def run_b200(args):
     import numpy as np
     import torch
@@ -442,8 +463,11 @@ def run_b200(args):
             dist.destroy_process_group()
         return 0
 
+    last = {}
+
     def step_resident():
-        return model.forward_heads(d_r, d_ref, d_q, d_s, d_rm, d_vm)
+        last["heads"] = model.forward_heads(d_r, d_ref, d_q, d_s, d_rm, d_vm)
+        return last["heads"]
 
     def step_e2e():
         # pinned host uint8 -> chunked H2D on the library's side stream, overlapped with the kernels -> D2H of the (B,27) result
@@ -456,12 +480,14 @@ def run_b200(args):
     sampler.start()
     ms = timed(step_resident, args.steps)
     launches = model.last_launch_count * args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "heads" if world == 1 else f"heads_rank{rank}", last["heads"].cpu().numpy(), DUMP_LIMIT_BYTES // world)
     for _ in range(2):
         step_e2e()
     ms_e2e = timed(step_e2e, args.steps)
     # dominant-kernel timing: the same steps with the library's event hook on
     lib.dan_profile_enable(1)
-    prof_steps = min(args.steps, 3)
+    prof_steps = args.steps
     timed(step_resident, prof_steps)
     import ctypes as C
     ms_cls = (C.c_double * _lib.PROF_NUM_CLASSES)()
@@ -470,7 +496,7 @@ def run_b200(args):
     lib.dan_profile_enable(0)
     clocks = sampler.stop()
 
-    train_block = None if args.no_train else train_step_block(cfg, sd, dev, dist, world, rank, timed)
+    train_block = None if args.no_train else train_step_block(cfg, sd, dev, dist, world, rank, timed, steps=args.steps)
     total_cands = B * world * args.steps
     value = total_cands / (ms * 1e-3)
     e2e_value = total_cands / (ms_e2e * 1e-3)
@@ -538,7 +564,7 @@ def run_b200(args):
     }
     line["train"] = train_block
     if world == 1 and args.precision == "bf16" and not args.no_fp32:
-        line["fp32"] = fp32_block(model, sample, dev, cfg, clocks)
+        line["fp32"] = fp32_block(model, sample, dev, cfg, clocks, steps=args.steps)
     if world == 1 and not args.no_cpu_baseline:
         cores = os.cpu_count() or 1
         nb, reps = 64, 10                  # BASELINE.md §5: >= 640 timed candidates
@@ -557,7 +583,8 @@ def run_b200(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of every region that times this project's code (value, e2e, "
+                    "profile pass, fp32 and train blocks); the CPU and torch-eager baseline samples keep their fixed sizes")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--precision", default="bf16", choices=["bf16", "fp32"])
@@ -569,7 +596,12 @@ def main():
     ap.add_argument("--no-eager-baseline", action="store_true", help="skip the torch-eager-on-this-GPU sample of the reference op sequence")
     ap.add_argument("--no-fp32", action="store_true", help="skip the fp32 1e-4-parity path block (BASELINE configs[1])")
     ap.add_argument("--no-train", action="store_true", help="skip the training-step block (BASELINE configs[4])")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the head matrix of the last timed step to DIR/heads.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.mode != "forward"):
+        ap.error("--dump-outputs applies to the forward benchmark of --impl b200")
     if args.impl == "reference":
         return run_reference(args)
     return run_b200(args)

@@ -1,6 +1,8 @@
 """CPU: the drop-in module keeps the reference's interface — names, shapes, init RNG stream, error behaviour —
 and the C-ABI library loads and exports every symbol include/dan_b200.h declares (no compute without a GPU)."""
 import ctypes
+import hashlib
+import json
 import os
 import re
 
@@ -8,15 +10,12 @@ import pytest
 import torch
 
 from dl4vc_b200 import _lib
-from dl4vc_b200.config import prod_config, min_config, small_config, state_dict_spec
+from dl4vc_b200.config import prod_config, small_config, state_dict_spec
 from dl4vc_b200.factory import ctor_kwargs
 from dl4vc_b200.model import Basic2DNet
-from oracle import ref_shim
+from oracle.interface_configs import CONFIGS
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CONFIGS = {"prod_small": small_config(), "min_small": min_config(layer_sizes=(64, 32), pool_combine_dimension=96),
-           "variant": small_config(total_conv_layers=4, residual_layer_start=3, conv_1d_pool_layers=(1, 3), concat_hw_reads=False,
-                                   skip_final_maxpool=True, use_strands=False, hidden_dropout=0.0)}
 
 
 @pytest.mark.parametrize("name", sorted(CONFIGS))
@@ -43,22 +42,24 @@ def test_prod_parameter_count():
     assert prod_config().macs_per_candidate() == 8_059_296_000
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="/root/reference not mounted")
 @pytest.mark.parametrize("name", sorted(CONFIGS))
 def test_same_names_shapes_and_init_as_reference(name):
-    cfg = CONFIGS[name]
+    """State-dict names and order, shapes, dtypes and the initial values drawn under torch.manual_seed(1) (bitwise, by SHA-256), and the
+    named_parameters() order, against tests/golden/init_state.json; a checkpoint of the recorded layout loads unchanged.
+    Provenance of the values (the file's "source" field): recorded from this module at commit 68cf6ee, whose initial values this test had
+    found bit-identical to the reference dl4vc/model.py when it still compared with a reference checkout directly. oracle/make_init_golden.py
+    re-records them from the reference itself."""
+    with open(os.path.join(ROOT, "tests", "golden", "init_state.json")) as f:
+        want = json.load(f)["configs"][name]
     torch.manual_seed(1)
-    ref_model, _ = ref_shim.build_reference_model(cfg)
-    torch.manual_seed(1)
-    mine = Basic2DNet(**ctor_kwargs(cfg))
-    a, b = ref_model.state_dict(), mine.state_dict()
-    assert list(a.keys()) == list(b.keys())
-    for k in a:
-        assert a[k].shape == b[k].shape and a[k].dtype == b[k].dtype, k
-        assert torch.equal(a[k], b[k]), f"init differs for {k}"
-    # a reference checkpoint loads unchanged
-    mine.load_state_dict(ref_model.state_dict())
-    assert [n for n, _ in mine.named_parameters()] == [n for n, _ in ref_model.named_parameters()]
+    mine = Basic2DNet(**ctor_kwargs(CONFIGS[name]))
+    sd = mine.state_dict()
+    assert list(sd.keys()) == [k for k, _, _, _ in want["state"]]
+    for k, shape, dtype, digest in want["state"]:
+        assert list(sd[k].shape) == shape and sd[k].dtype == getattr(torch, dtype), k
+        assert hashlib.sha256(sd[k].contiguous().numpy().tobytes()).hexdigest() == digest, f"init differs for {k}"
+    mine.load_state_dict({k: torch.zeros(shape, dtype=getattr(torch, dtype)) for k, shape, dtype, _ in want["state"]})
+    assert [n for n, _ in mine.named_parameters()] == want["parameters"]
 
 
 def test_unsupported_options_raise_clearly():
