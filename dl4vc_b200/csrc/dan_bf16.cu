@@ -11,7 +11,7 @@
 //                      shared memory, read-axis max / sum by TMA bulk reductions — the PROD path.
 //   dan_layer_kernel   (dan_layerwise.cuh) one conv layer per launch: fallback for shapes the fused kernel does not take.
 //   tma_gemm_kernel    (dan_gemm.cuh) TMA-fed batched GEMM: highway compression (1x201) conv as one K=6432 GEMM over reads,
-//                      pool bias map, FC trunk, heads.
+//                      pool bias map, post-pool Linear (pool_combine_dimension > 0), FC trunk, heads.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -163,8 +163,9 @@ __global__ void __launch_bounds__(64) pool_groups_im2col_kernel(const uint4* __r
   if (pp >= P - dil) row0[(long)pp * (3 * kKC) + 2 * kKC] = make_uint4(0, 0, 0, 0);         // tap 2 reaches behind it
 }
 
-// read-mean of the final layer (model.py:826) -> mean block of the FC input; the max block next to it (model.py:825) is written by
-// the stack kernel itself (bulk max-reductions) after fcin_max_init_kernel has set it to -inf
+// read-mean of the final layer (model.py:826) -> mean block of the pooled features; the max block next to it (model.py:825) is written
+// by the stack kernel itself (bulk max-reductions) after fcin_max_init_kernel has set it to -inf. The pooled block is the head of the
+// FC input, or a buffer of its own when the post-pool Linear follows (dan_bf16_forward).
 __global__ void __launch_bounds__(64) fcin_mean_kernel(const uint4* __restrict__ sums, int P, int R, uint4* __restrict__ fcin, long fc_kstride, long mean_piece0, int cand0) {
   const int cand = blockIdx.y, kc = blockIdx.z;
   const int pp = blockIdx.x * blockDim.x + threadIdx.x;
@@ -229,7 +230,7 @@ __global__ void add_pool_bf16_kernel(const uint4* __restrict__ h, const float* _
   }
 }
 
-// layer-wise fallback path: final max ‖ mean over reads -> FC input pieces (bf16 feature order of both paths: max (c/8, p, c%8) | mean likewise)
+// layer-wise fallback path: final max ‖ mean over reads -> pooled-feature pieces (bf16 feature order of both paths: max (c/8, p, c%8) | mean likewise)
 __global__ void __launch_bounds__(64) pool_final_bf16_kernel(const uint4* __restrict__ h, long kstride, uint4* __restrict__ fcin, long fc_kstride,
                                        int cand0, RowGeom g, int skip_max) {
   const int cand = blockIdx.y, kc = blockIdx.z;
@@ -260,7 +261,7 @@ __global__ void __launch_bounds__(64) pool_final_bf16_kernel(const uint4* __rest
   }
 #pragma unroll
   for (int j = 0; j < 8; ++j) s[j] /= (float)g.R;
-  uint4* row = fcin + (long)(cand0 + cand) * fc_kstride;          // fc_kstride = pieces per FC-input row
+  uint4* row = fcin + (long)(cand0 + cand) * fc_kstride;          // fc_kstride = pieces per row of the pooled-feature buffer
   if (skip_max) {
     row[(long)kc * g.P + pp] = pack8(s);
   } else {
@@ -316,10 +317,37 @@ __global__ void pack_conv_bf16_kernel(const float* __restrict__ w, uint4* __rest
     store_bf16(out, ((long)tap * kc_in + kc) * kC + n, j, c < Cin ? w[((long)n * Cin + c) * 3 + tap] : 0.f);
   }
 }
+// Feature order of the bf16 path's FC input (and of the post-pool Linear's input) against the reference's (model.py:833-859):
+//   * pooled max | mean features: the kernels keep (block, c / 8, p, c % 8) — one 16-byte piece per (c / 8, p), the unit of the stack
+//     kernel's bulk reductions — where the reference flattens (block, c, p);
+//   * post-pool Linear outputs (pool_combine_dimension > 0): the reference's order;
+//   * highway features: the kernels keep (layer, read, o), the reference (layer, o, read).
+// Column k of such an input -> the reference's column. The leading `permuted` columns are pooled features, columns up to `hw_base` are
+// in the reference's order, the rest is the highway block. Weight packers and the FC-input test hook both go through this map.
+__device__ __forceinline__ long fc_ref_column(long k, long permuted, long hw_base, int P, int C, int R, int bott) {
+  if (k < permuted) {
+    const long blk = k / ((long)P * C);            // 0 = max block (or mean when skip_max), 1 = mean block
+    const long rem = k - blk * P * C;
+    const int kc8 = (int)(rem / (P * 8)), pp = (int)((rem / 8) % P), c = kc8 * 8 + (int)(rem % 8);
+    return (blk * C + c) * (long)P + pp;
+  }
+  if (k < hw_base) return k;
+  const long h = k - hw_base;
+  const int o = (int)(h % bott); const long lr = h / bott;
+  const int r = (int)(lr % R); const int l = (int)(lr / R);
+  return hw_base + (long)l * bott * R + (long)o * R + r;
+}
+// where the blocks of the FC input sit: pooled features at the head (pool_combine_dimension 0), or the post-pool Linear's D outputs
+struct FcInLayout { long permuted, hw_base; };
+inline FcInLayout fc_in_layout(const dan_model* m) {
+  const int D = m->cfg.pool_combine_dimension;
+  return D > 0 ? FcInLayout{0, D} : FcInLayout{m->pooled, m->pooled};
+}
+
 // linear-like (N, K) fp32 with optional source-column map -> bf16 row-major [Npad][Kpad] (mode 3: UMMA chunk image [kc][Npad][8])
 __global__ void pack_linear_bf16_kernel(const float* __restrict__ w, uint4* __restrict__ out, int N, int Npad, int K, int Kpad,
-                                        int mode, int P, int C, int R, int bott, int L, int pooled, int skip_max) {
-  // mode 0: identity columns. mode 1: FC1 feature permutation (see dan_bf16_forward). mode 2: compression (O, Cb, 1, P): k = ((c/8)*P + p)*8 + c%8
+                                        int mode, int P, int C, int R, int bott, long permuted, long hw_base) {
+  // mode 0: identity columns. mode 1: FC-input feature order (fc_ref_column). mode 2: compression (O, Cb, 1, P): k = ((c/8)*P + p)*8 + c%8
   // mode 4: conv weight (Cout, C, 1, 3) with k = tap*C + cin
   const long total = (long)(Kpad / 8) * Npad * 8;
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
@@ -330,17 +358,7 @@ __global__ void pack_linear_bf16_kernel(const float* __restrict__ w, uint4* __re
     if (n < N && k < K) {
       long src = k;
       if (mode == 1) {
-        if (k < pooled) {
-          const long blk = k / ((long)P * C);            // 0 = max block (or mean when skip_max), 1 = mean block
-          const long rem = k - blk * P * C;               // pooled feature order of the kernels: (c / 8, p, c % 8)
-          const int kc8 = (int)(rem / (P * 8)), pp = (int)((rem / 8) % P), c = kc8 * 8 + (int)(rem % 8);
-          src = (blk * C + c) * (long)P + pp;
-        } else {
-          const long h = k - pooled;
-          const int o = (int)(h % bott); const long lr = h / bott;
-          const int r = (int)(lr % R); const int l = (int)(lr / R);
-          src = pooled + (long)l * bott * R + (long)o * R + r;
-        }
+        src = fc_ref_column(k, permuted, hw_base, P, C, R, bott);
       } else if (mode == 2) {                             // K order of the T matrix: (c / 8, p, c % 8)
         const int g = (int)(k / (P * 8)), rem = (int)(k % (P * 8));
         const int pp = rem / 8, c = g * 8 + rem % 8;
@@ -373,6 +391,7 @@ struct Bf16Weights {
   uint4* wconv[DAN_MAX_LAYERS]; uint4* wres[DAN_MAX_LAYERS]; uint4* wbott[DAN_MAX_LAYERS]; uint4* wcomp[DAN_MAX_LAYERS];
   uint4* wcomp_all;                   // all layers' compression weights, [L][bott][P*bott] bf16 (one batched GEMM operand)
   uint4* fcw[DAN_MAX_FC]; uint4* headw;
+  uint4* postw;                       // post-pool Linear (pool_combine_dimension > 0): [D][pooledPad] bf16, columns in pooled-feature order
   uint4* wbmap[DAN_MAX_LAYERS];       // layers fed by a read-mean pool-add: conv weight as a row-major GEMM operand [cout][tap*C + cin] bf16 (pool bias map)
   const float** comp_bias_ptrs;       // device array of L pointers
   uint8_t* wstream[DAN_MAX_LAYERS];   // conv | residual | bottleneck operand images of a layer, contiguous (dan_stack.cuh); kWeightReplicas copies
@@ -417,7 +436,8 @@ struct Bf16Plan {
   long hw_layer_stride;
   long t_layer_pieces;               // uint4 pieces of one layer's T matrix
   int fcKC;                          // FC input pieces
-  size_t off_zero_begin, off_x0, off_h[3], off_zero_end, off_t, off_pool, off_sums, off_im2col, off_bmapg, off_bmap, off_hw, off_part, off_fcin, off_fcx[DAN_MAX_FC], total;
+  int poolKC;                        // pieces per row of the pooled-feature buffer (pool_combine_dimension > 0)
+  size_t off_zero_begin, off_x0, off_h[3], off_zero_end, off_t, off_pool, off_sums, off_im2col, off_bmapg, off_bmap, off_hw, off_part, off_pooled, off_fcin, off_fcx[DAN_MAX_FC], total;
   int maxN;
 };
 
@@ -450,6 +470,9 @@ Bf16Plan make_plan(const dan_model* m, int batch) {
   pl.hw_layer_stride = pl.readsPad * bott;
   pl.off_hw = take((size_t)m->L * pl.hw_layer_stride * 4);
   pl.off_part = take((size_t)kCompSplits * m->L * pl.readsPad * bott * 4);     // split-K partials of the compression GEMM
+  // with the post-pool Linear (model.py:841-843) the pooled max | mean block (wider than the FC input) is its own GEMM operand
+  pl.poolKC = m->pooledPad / 8;
+  pl.off_pooled = take(m->cfg.pool_combine_dimension > 0 ? (size_t)pl.poolKC * pl.BcPad * 16 : 0);     // [BcPad][pooledPad] bf16
   pl.off_fcin = take((size_t)pl.fcKC * pl.BcPad * 16);           // [BcPad][fcInPad] bf16, row-major
   pl.maxN = DAN_HEAD_PAD;
   for (int i = 0; i < m->cfg.num_fc; ++i) {
@@ -463,18 +486,23 @@ Bf16Plan make_plan(const dan_model* m, int batch) {
 }  // namespace
 
 // ----------------------------------------------------------------------------------------------------------
-int dan_bf16_supported(const dan_model* m) {
-  if (m->C != kC) return 0;
-  if (m->cfg.pool_combine_dimension != 0) return 0;
-  if (m->cfg.highway && !(m->bott == 32 || m->bott == 64)) return 0;
-  if (m->geom.gap > kLead) return 0;
-  if (m->CinPad % 16) return 0;
-  for (int i = 0; i < m->cfg.num_fc; ++i) if (m->cfg.fc_sizes[i] % 32) return 0;
-  return 1;
+const char* dan_bf16_unsupported_reason(const dan_model* m) {
+  if (m->C != kC) return "the bf16 kernels are built for 128 conv channels";
+  // N of the post-pool GEMM and of the FC trunk's GEMMs is cut into 32- or 64-wide tiles (run_gemm2)
+  if (m->cfg.pool_combine_dimension % 32) return "pool_combine_dimension must be a multiple of 32";
+  if (m->cfg.highway && !(m->bott == 32 || m->bott == 64)) return "the highway bottleneck must be 32 or 64 wide";
+  if (m->geom.gap > kLead) return "dilation above 8";
+  if (m->CinPad % 16) return "padded input channels must be a multiple of 16";
+  for (int i = 0; i < m->cfg.num_fc; ++i) if (m->cfg.fc_sizes[i] % 32) return "FC widths must be multiples of 32";
+  return nullptr;
 }
+int dan_bf16_supported(const dan_model* m) { return dan_bf16_unsupported_reason(m) == nullptr; }
 
 size_t dan_bf16_workspace_bytes(const dan_model* m, int batch) {
-  if (!dan_bf16_supported(m)) return 0;
+  if (const char* why = dan_bf16_unsupported_reason(m)) {
+    dan_set_error("bf16 tcgen05 path does not cover this configuration: %s", why);
+    return 0;
+  }
   return make_plan(m, batch).total;
 }
 
@@ -507,32 +535,39 @@ int dan_bf16_pack(dan_model* m, const dan_weights* w, cudaStream_t st) {
     pack_conv_bf16_kernel<<<grid_for((long)3 * kc_in * kC * 8), 256, 0, st>>>(w->conv_w[l], bw->wconv[l], cin, kc_in);
     if (l > 0 && m->cfg.pool_after[l - 1]) {
       if ((rc = alloc(&bw->wbmap[l], (size_t)kC * 3 * kC / 8))) return rc;
-      pack_linear_bf16_kernel<<<grid_for((long)3 * kC * kC), 256, 0, st>>>(w->conv_w[l], bw->wbmap[l], kC, kC, 3 * kC, 3 * kC, 4, P, kC, R, bott, L, 0, 0);
+      pack_linear_bf16_kernel<<<grid_for((long)3 * kC * kC), 256, 0, st>>>(w->conv_w[l], bw->wbmap[l], kC, kC, 3 * kC, 3 * kC, 4, P, kC, R, bott, 0, 0);
     }
     if (m->cfg.is_residual[l]) {
-      pack_linear_bf16_kernel<<<grid_for((long)kKC * kC * 8), 256, 0, st>>>(w->res_w[l], bw->wres[l], kC, kC, kC, kC, 3, P, kC, R, bott, L, 0, 0);
+      pack_linear_bf16_kernel<<<grid_for((long)kKC * kC * 8), 256, 0, st>>>(w->res_w[l], bw->wres[l], kC, kC, kC, kC, 3, P, kC, R, bott, 0, 0);
     }
     if (m->cfg.highway) {
-      pack_linear_bf16_kernel<<<grid_for((long)kKC * bott * 8), 256, 0, st>>>(w->bott_w[l], bw->wbott[l], bott, bott, kC, kC, 3, P, kC, R, bott, L, 0, 0);
+      pack_linear_bf16_kernel<<<grid_for((long)kKC * bott * 8), 256, 0, st>>>(w->bott_w[l], bw->wbott[l], bott, bott, kC, kC, 3, P, kC, R, bott, 0, 0);
       const int K = P * bott;
       if ((rc = alloc(&bw->wcomp_all, (size_t)L * (K / 8) * bott))) return rc;
       bw->wcomp[l] = bw->wcomp_all + (size_t)l * (K / 8) * bott;
-      pack_linear_bf16_kernel<<<grid_for((long)K * bott), 256, 0, st>>>(w->comp_w[l], bw->wcomp[l], bott, bott, K, K, 2, P, kC, R, bott, L, 0, 0);
+      pack_linear_bf16_kernel<<<grid_for((long)K * bott), 256, 0, st>>>(w->comp_w[l], bw->wcomp[l], bott, bott, K, K, 2, P, kC, R, bott, 0, 0);
     }
     // epilogue constants (the fp32 packer already folded BatchNorm on this stream)
     chan_table_kernel<<<1, kC, 0, st>>>(m->convB[l], m->cfg.use_batchnorm ? m->bnScale[l] : nullptr, m->cfg.use_batchnorm ? m->bnShift[l] : nullptr,
                                         m->cfg.is_residual[l] ? m->resB[l] : nullptr, bw->chan_dev + (size_t)l * kChanRows * kC);
   }
+  const int D = m->cfg.pool_combine_dimension;
+  if (D > 0) {      // post_pool_conv1D (D, pooled): its input columns are the pooled features in the kernels' order
+    if ((rc = alloc(&bw->postw, (size_t)(m->pooledPad / 8) * D))) return rc;
+    pack_linear_bf16_kernel<<<grid_for((long)m->pooledPad * D), 256, 0, st>>>(w->post_pool_w, bw->postw, D, D, m->pooled, m->pooledPad, 1, P, kC, R, bott,
+                                                                              m->pooled, m->pooled);
+  }
+  const FcInLayout fl = fc_in_layout(m);
   int K = m->fcIn, Kpad = m->fcInPad;
   for (int i = 0; i < m->cfg.num_fc; ++i) {
     const int N = m->cfg.fc_sizes[i];
     if ((rc = alloc(&bw->fcw[i], (size_t)(Kpad / 8) * N))) return rc;
     pack_linear_bf16_kernel<<<grid_for((long)Kpad * N), 256, 0, st>>>(w->fc_w[i], bw->fcw[i], N, N, K, Kpad, i == 0 ? 1 : 0, P, kC, R, bott,
-                                                                      m->cfg.concat_hw_reads ? L : 1, m->pooled, m->cfg.skip_final_maxpool);
+                                                                      fl.permuted, fl.hw_base);
     K = N; Kpad = N;
   }
   if ((rc = alloc(&bw->headw, (size_t)(m->hidden / 8) * DAN_HEAD_PAD))) return rc;
-  pack_linear_bf16_kernel<<<grid_for((long)m->hidden * DAN_HEAD_PAD), 256, 0, st>>>(w->head_w, bw->headw, DAN_NUM_HEAD_OUTPUTS, DAN_HEAD_PAD, m->hidden, m->hidden, 0, P, kC, R, bott, L, 0, 0);
+  pack_linear_bf16_kernel<<<grid_for((long)m->hidden * DAN_HEAD_PAD), 256, 0, st>>>(w->head_w, bw->headw, DAN_NUM_HEAD_OUTPUTS, DAN_HEAD_PAD, m->hidden, m->hidden, 0, P, kC, R, bott, 0, 0);
   for (int l = 0; l < L; ++l)
     for (int r = 1; r < kWeightReplicas; ++r)
       DAN_CUDA_TRY(cudaMemcpyAsync(bw->wstream[l] + (size_t)r * bw->wstream_bytes[l], bw->wstream[l], bw->wstream_bytes[l], cudaMemcpyDeviceToDevice, st));
@@ -558,6 +593,7 @@ void dan_bf16_free(dan_model* m) {
   cudaFree(bw->enc_tab);
   for (int i = 0; i < DAN_MAX_FC; ++i) cudaFree(bw->fcw[i]);
   cudaFree(bw->headw);
+  cudaFree(bw->postw);
   cudaFree(bw->comp_bias_ptrs);
   delete bw;
   m->bf16_store = nullptr;
@@ -581,9 +617,14 @@ int dan_bf16_forward(dan_model* m, const DevInputs& in, int batch, float* heads_
   uint4* BMAP = reinterpret_cast<uint4*>(base + pl.off_bmap);
   float* HW = reinterpret_cast<float*>(base + pl.off_hw);
   uint4* FCIN = reinterpret_cast<uint4*>(base + pl.off_fcin);
+  const int D = m->cfg.pool_combine_dimension;
+  // pooled max | mean pieces: the head of the FC input, or (post-pool Linear, model.py:841-843) the A operand of the post-pool GEMM
+  uint4* POOLED = D > 0 ? reinterpret_cast<uint4*>(base + pl.off_pooled) : FCIN;
+  const long pool_kstride = D > 0 ? pl.poolKC : pl.fcKC;
+  const FcInLayout fl = fc_in_layout(m);
   const bool fused = stack_fused(m);
   const bool enc_in_kernel = fused && stack_encodes(m) && bw->enc_tab != nullptr;
-  const long mean_piece0 = m->cfg.skip_final_maxpool ? 0 : (long)kKC * P;      // FC-input pieces: max block | mean block | highway
+  const long mean_piece0 = m->cfg.skip_final_maxpool ? 0 : (long)kKC * P;      // pooled pieces: max block | mean block
   // highway compression (model.py:776) of every layer of a pass as ONE batched GEMM: HW[l][read][o] = T[l][read][:] . Wc[l][o][:]
   auto run_compression = [&](int l0, int nl, int reads) -> int {
     const long K = (long)P * bott;
@@ -613,7 +654,7 @@ int dan_bf16_forward(dan_model* m, const DevInputs& in, int batch, float* heads_
     else { sp.in_mode = kStkInPlanes; sp.in = seg_in; sp.in_kstride = pl.kstride; }
     sp.out = seg_out; sp.out_kstride = pl.kstride;
     if (want_sums || final_seg) { sp.sums = SUMS; sp.groups_per_cand = sum_groups_per_cand(m); }
-    if (final_seg && !m->cfg.skip_final_maxpool) { sp.maxv = FCIN + (long)s0 * pl.fcKC; sp.max_stride = pl.fcKC; }
+    if (final_seg && !m->cfg.skip_final_maxpool) { sp.maxv = POOLED + (long)s0 * pool_kstride; sp.max_stride = pool_kstride; }
     sp.bmap = with_bmap ? BMAP : nullptr;
     sp.cands = ns; sp.R = R; sp.P = P; sp.pitch = g.pitch; sp.highway = m->cfg.highway; sp.num_layers = l_end - l;
     for (int k = l; k < l_end; ++k) {
@@ -703,7 +744,7 @@ int dan_bf16_forward(dan_model* m, const DevInputs& in, int batch, float* heads_
           const bool pool_next = !final_seg;             // segments end where a read-mean pool-add follows (or at the last layer)
           uint4* next = final_seg ? nullptr : H[hsel ^ 1];
           if (final_seg && !m->cfg.skip_final_maxpool) {
-            { DanProfScope ps(DAN_PROF_POOL, st); fcin_max_init_kernel<<<grid_for((long)ns * kKC * P), 256, 0, st>>>(FCIN, pl.fcKC, s0, ns, kKC * P); }
+            { DanProfScope ps(DAN_PROF_POOL, st); fcin_max_init_kernel<<<grid_for((long)ns * kKC * P), 256, 0, st>>>(POOLED, pool_kstride, s0, ns, kKC * P); }
             dan_count_launch();
           }
           if ((rc = launch_segment(l, l_end, (long)c0 + s0, cur, next, with_bmap, pool_next, final_seg, s0, ns))) return rc;
@@ -723,7 +764,7 @@ int dan_bf16_forward(dan_model* m, const DevInputs& in, int batch, float* heads_
             with_bmap = true;
             cur = next; hsel ^= 1;
           } else {
-            { DanProfScope ps(DAN_PROF_POOL, st); fcin_mean_kernel<<<dim3((P + 63) / 64, ns, kKC), 64, 0, st>>>(SUMS, P, R, FCIN, pl.fcKC, mean_piece0, s0); }
+            { DanProfScope ps(DAN_PROF_POOL, st); fcin_mean_kernel<<<dim3((P + 63) / 64, ns, kKC), 64, 0, st>>>(SUMS, P, R, POOLED, pool_kstride, mean_piece0, s0); }
             dan_count_launch();
             DAN_CUDA_TRY(cudaGetLastError());
           }
@@ -767,17 +808,27 @@ int dan_bf16_forward(dan_model* m, const DevInputs& in, int batch, float* heads_
           }
           cur = next; hsel = (hsel + 1) % 3;
         }
-        { DanProfScope ps(DAN_PROF_POOL, st); pool_final_bf16_kernel<<<dim3((P + 63) / 64, ns, kKC), 64, 0, st>>>(cur, pl.kstride, FCIN, pl.fcKC, s0, g, m->cfg.skip_final_maxpool); }
+        { DanProfScope ps(DAN_PROF_POOL, st); pool_final_bf16_kernel<<<dim3((P + 63) / 64, ns, kKC), 64, 0, st>>>(cur, pl.kstride, POOLED, pool_kstride, s0, g, m->cfg.skip_final_maxpool); }
         dan_count_launch();
         DAN_CUDA_TRY(cudaGetLastError());
       }
       if (m->cfg.highway) {
         const int Lh = m->cfg.concat_hw_reads ? L : 1;
         { DanProfScope ps(DAN_PROF_POOL, st); highway_finish_bf16_kernel<<<grid_for((long)ns * Lh * R * (bott / 8)), 256, 0, st>>>(
-            HW, pl.hw_layer_stride, bw->comp_bias_ptrs, L, bott, R, m->cfg.concat_hw_reads, FCIN, pl.fcKC, m->pooled / 8, s0, ns); }
+            HW, pl.hw_layer_stride, bw->comp_bias_ptrs, L, bott, R, m->cfg.concat_hw_reads, FCIN, pl.fcKC, fl.hw_base / 8, s0, ns); }
         dan_count_launch();
         DAN_CUDA_TRY(cudaGetLastError());
       }
+    }
+    if (D > 0) {
+      // ---- post_pool_conv1D + ReLU (model.py:841-843) -> FC-input columns [0, D). One K = pooled contraction per row, unsplit: a row's
+      // sum runs in the same order whatever the batch shape ----
+      Gemm2Operand A{POOLED, nb, (long)pl.poolKC * 16, 0};
+      Gemm2Operand B{bw->postw, D, (long)pl.poolKC * 16, 0};
+      Gemm2Params gp{};
+      gp.M = nb; gp.N = D; gp.K = m->pooled; gp.mode = kG2BiasReluBf16; gp.bias = m->postB;
+      gp.out_bf16 = reinterpret_cast<__nv_bfloat16*>(FCIN); gp.ld_bf16 = m->fcInPad;
+      if ((rc = run_gemm2(A, B, gp, 1, bw->num_sms, st))) return rc;
     }
     // ---- FC trunk + heads (model.py:917-958) ----
     const uint4* x = FCIN; int K = m->fcInPad;
@@ -837,22 +888,12 @@ int dan_bf16_encode_reference_order(dan_model* m, const DevInputs& in, int batch
 // FC input in the REFERENCE feature order (fp32), undoing the bf16 path's feature permutation (test hook)
 namespace {
 __global__ void fcin_to_reference_order_kernel(const uint4* __restrict__ fcin, long kstride, int rows, float* __restrict__ out,
-                                               int fcIn, int pooled, int P, int C, int R, int bott) {
+                                               int fcIn, long permuted, long hw_base, int P, int C, int R, int bott) {
   const long total = (long)rows * fcIn;
   for (long i = blockIdx.x * (long)blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
-    const int f = (int)(i % fcIn); const long m = i / fcIn;
-    long k;
-    if (f < pooled) {
-      const int blk = f / (C * P), rem = f % (C * P);
-      const int c = rem / P, pp = rem % P;
-      k = (long)blk * P * C + ((long)(c / 8) * P + pp) * 8 + c % 8;
-    } else {
-      const int h = f - pooled;
-      const int l = h / (bott * R), rem = h % (bott * R);
-      const int o = rem / R, r = rem % R;
-      k = pooled + ((long)l * R + r) * bott + o;
-    }
-    out[i] = __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(fcin + m * kstride)[k]);      // kstride = pieces per row
+    const int k = (int)(i % fcIn); const long m = i / fcIn;
+    out[m * fcIn + fc_ref_column(k, permuted, hw_base, P, C, R, bott)] =
+        __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(fcin + m * kstride)[k]);      // kstride = pieces per row
   }
 }
 }  // namespace
@@ -861,7 +902,9 @@ int dan_bf16_debug_fc_input(dan_model* m, int batch, const void* ws, float* out,
   const Bf16Plan pl = make_plan(m, batch);
   const int nb = batch % pl.Bc == 0 ? pl.Bc : batch % pl.Bc;
   const uint4* FCIN = reinterpret_cast<const uint4*>(static_cast<const char*>(ws) + pl.off_fcin);
-  fcin_to_reference_order_kernel<<<grid_for((long)nb * m->fcIn), 256, 0, st>>>(FCIN, pl.fcKC, nb, out, m->fcIn, m->pooled, m->P, kC, m->R, m->bott > 0 ? m->bott : 1);
+  const FcInLayout fl = fc_in_layout(m);
+  fcin_to_reference_order_kernel<<<grid_for((long)nb * m->fcIn), 256, 0, st>>>(FCIN, pl.fcKC, nb, out, m->fcIn, fl.permuted, fl.hw_base, m->P, kC, m->R,
+                                                                               m->bott > 0 ? m->bott : 1);
   DAN_CUDA_TRY(cudaGetLastError());
   return nb;
 }

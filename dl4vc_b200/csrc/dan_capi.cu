@@ -192,7 +192,10 @@ static int check_forward_args(dan_model* m, int precision, const uint8_t* reads,
   if (batch > 0 && m->cfg.use_strands && !s) { dan_set_error("model uses strands but strands is null (model.py:549)"); return DAN_E_INVALID; }
   if (batch > 0 && m->cfg.use_reads_ref_var_mask && (!rm || !vm)) { dan_set_error("model uses ref/var masks but a mask pointer is null (model.py:576)"); return DAN_E_INVALID; }
   if (precision != DAN_PRECISION_FP32 && precision != DAN_PRECISION_BF16) { dan_set_error("unknown precision %d", precision); return DAN_E_INVALID; }
-  if (precision == DAN_PRECISION_BF16 && !dan_bf16_supported(m)) { dan_set_error("bf16 tcgen05 path does not cover this configuration"); return DAN_E_UNSUPPORTED; }
+  if (precision == DAN_PRECISION_BF16 && !dan_bf16_supported(m)) {
+    dan_set_error("bf16 tcgen05 path does not cover this configuration: %s", dan_bf16_unsupported_reason(m));
+    return DAN_E_UNSUPPORTED;
+  }
   return DAN_OK;
 }
 
@@ -324,9 +327,10 @@ static int check_train_args(dan_model* m, const dan_weights* params, const uint8
   if (!params) { dan_set_error("null parameter struct"); return DAN_E_INVALID; }
   if (batch < 1) { dan_set_error("training needs at least one candidate"); return DAN_E_INVALID; }
   if (!(dropout_p >= 0.f && dropout_p < 1.f)) { dan_set_error("dropout probability %g outside [0, 1)", dropout_p); return DAN_E_INVALID; }
-  if (!dan_train_supported(m)) { dan_set_error("training kernels do not cover this configuration (pool_combine_dimension > 0)"); return DAN_E_UNSUPPORTED; }
+  if (!dan_train_supported(m)) { dan_set_error("training kernels do not cover this configuration (channels must be a multiple of 4, at most 1024)"); return DAN_E_UNSUPPORTED; }
   for (int l = 0; l < m->L; ++l)
     if (m->cfg.use_batchnorm && (!params->bn_w[l] || !params->bn_b[l] || !params->bn_mean[l] || !params->bn_var[l])) { dan_set_error("missing BatchNorm tensors of layer %d", l + 1); return DAN_E_INVALID; }
+  if (m->cfg.pool_combine_dimension > 0 && (!params->post_pool_w || !params->post_pool_b)) { dan_set_error("missing post_pool_w / post_pool_b"); return DAN_E_INVALID; }
   return DAN_OK;
 }
 
@@ -349,6 +353,7 @@ int dan_backward(dan_model* m, const dan_weights* params, const uint8_t* reads, 
   int rc = check_train_args(m, params, reads, q_scores, strands, ref, ref_masks, var_masks, batch, heads_out, dropout_p);
   if (rc) return rc;
   if (!tape || !dheads || !grads) { dan_set_error("null tape / gradient pointer"); return DAN_E_INVALID; }
+  if (m->cfg.pool_combine_dimension > 0 && (!grads->post_pool_w || !grads->post_pool_b)) { dan_set_error("missing post_pool_w / post_pool_b gradient tensors"); return DAN_E_INVALID; }
   DevInputs in{reads, q_scores, strands, ref, ref_masks, var_masks};
   return dan_backward_impl(m, params, in, removed, batch, dropout_p, seed, dheads, heads_out, grads, tape, tape_bytes, static_cast<cudaStream_t>(stream));
 }

@@ -131,6 +131,7 @@ int dan_bf16_encode_reference_order(dan_model* m, const DevInputs& in, int batch
 int dan_bf16_pack(dan_model* m, const dan_weights* w, cudaStream_t st);
 void dan_bf16_free(dan_model* m);
 int dan_bf16_supported(const dan_model* m);
+const char* dan_bf16_unsupported_reason(const dan_model* m);     // nullptr when the bf16 path takes the configuration
 
 // training path (dan_train.cu)
 int dan_train_supported(const dan_model* m);

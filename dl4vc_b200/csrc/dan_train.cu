@@ -375,8 +375,8 @@ constexpr int kLinearMaxSplits = 40;
 struct TrainPlan {
   long rows, rowsAlloc, readsPad, hw_layer_stride;
   int BPad, chunks;
-  size_t x0, u[DAN_MAX_LAYERS], y[DAN_MAX_LAYERS], h[DAN_MAX_LAYERS], inp[DAN_MAX_LAYERS], t[DAN_MAX_LAYERS], pool, hw, fcin, xd[DAN_MAX_FC + 1], act[DAN_MAX_FC],
-      heads, stats, red, ga, gb, gt, dhw, dfc[2], dz_heads, tnpart, wtmp, embpart, embcnt, total;
+  size_t x0, u[DAN_MAX_LAYERS], y[DAN_MAX_LAYERS], h[DAN_MAX_LAYERS], inp[DAN_MAX_LAYERS], t[DAN_MAX_LAYERS], pool, hw, pooled, fcin, xd[DAN_MAX_FC + 1], act[DAN_MAX_FC],
+      heads, stats, red, ga, gb, gt, dhw, dfc[2], dpooled, dz_heads, tnpart, wtmp, embpart, embcnt, total;
   size_t tn_part_floats;
 };
 
@@ -403,6 +403,8 @@ TrainPlan make_train_plan(const dan_model* m, int B) {
   }
   pl.pool = take((size_t)B * m->P * C * 4);
   pl.hw = take((size_t)L * pl.hw_layer_stride * 4);
+  const size_t pooled_bytes = m->cfg.pool_combine_dimension > 0 ? (size_t)pl.BPad * m->pooledPad * 4 : 0;
+  pl.pooled = take(pooled_bytes);                                  // input of the post-pool Linear (model.py:841-843); without it the pooled block heads FCIN
   pl.fcin = take((size_t)pl.BPad * m->fcInPad * 4);
   int K = m->fcInPad;
   for (int i = 0; i <= m->cfg.num_fc; ++i) {
@@ -417,6 +419,7 @@ TrainPlan make_train_plan(const dan_model* m, int B) {
   pl.gt = m->cfg.highway ? take(((size_t)pl.rowsAlloc + (size_t)128 * g.pitch) * bott * 4) : 0;
   pl.dhw = take((size_t)L * pl.hw_layer_stride * 4);
   pl.dfc[0] = take((size_t)pl.BPad * m->fcInPad * 4); pl.dfc[1] = take((size_t)pl.BPad * m->fcInPad * 4);
+  pl.dpooled = take(pooled_bytes);
   pl.dz_heads = take((size_t)pl.BPad * DAN_HEAD_PAD * 4);
   pl.tn_part_floats = (size_t)296 * 128 * 128 + (size_t)64 * bott * g.pitch * bott;      // conv-shaped problems | compression (I = bott, J = P*bott)
   const size_t fc_part = (size_t)kLinearMaxSplits * pl.BPad * 1024;                          // split-K partials of the small-M FC products (tr_linear)
@@ -497,7 +500,6 @@ int tr_colsum(const float* X, int ldx, long rows, int C, float* out, double* red
 size_t dan_train_tape_bytes_impl(const dan_model* m, int batch) { return make_train_plan(m, batch).total; }
 
 int dan_train_supported(const dan_model* m) {
-  if (m->cfg.pool_combine_dimension != 0) return 0;
   if (m->C % 4 || m->C > 1024) return 0;
   return 1;
 }
@@ -600,10 +602,19 @@ int dan_train_forward_impl(dan_model* m, const dan_weights* w, const DevInputs& 
   }
   float* FCIN = reinterpret_cast<float*>(base + pl.fcin);
   DAN_CUDA_TRY(cudaMemsetAsync(FCIN, 0, (size_t)pl.BPad * m->fcInPad * 4, st));
-  pool_final_kernel<<<dim3(g.P, B), 128, 0, st>>>(cur, C, FCIN, m->fcInPad, C, g, m->cfg.skip_final_maxpool);
+  const int Dp = m->cfg.pool_combine_dimension;
+  float* POOLED = Dp > 0 ? reinterpret_cast<float*>(base + pl.pooled) : FCIN;
+  const int pooled_ld = Dp > 0 ? m->pooledPad : m->fcInPad;
+  if (Dp > 0) DAN_CUDA_TRY(cudaMemsetAsync(POOLED, 0, (size_t)pl.BPad * m->pooledPad * 4, st));
+  pool_final_kernel<<<dim3(g.P, B), 128, 0, st>>>(cur, C, POOLED, pooled_ld, C, g, m->cfg.skip_final_maxpool);
   dan_count_launch();
+  if (Dp > 0) {      // post_pool_conv1D + ReLU (model.py:841-843) -> FC-input columns [0, D)
+    if ((rc = tr_linear(POOLED, m->pooledPad, B, m->pooledPad, m->postW, Dp, Dp, m->postB, 1, nullptr, 0, FCIN, m->fcInPad,
+                        reinterpret_cast<float*>(base + pl.tnpart), pl.tn_part_floats, st))) return rc;
+  }
   if (m->cfg.highway) {
-    highway_assemble_kernel<<<grid_for((long)B * m->hwFeat), 256, 0, st>>>(HW, pl.hw_layer_stride, L, bott, m->R, m->cfg.concat_hw_reads, FCIN + m->pooled, m->fcInPad, B);
+    highway_assemble_kernel<<<grid_for((long)B * m->hwFeat), 256, 0, st>>>(HW, pl.hw_layer_stride, L, bott, m->R, m->cfg.concat_hw_reads, FCIN + (Dp > 0 ? Dp : m->pooled),
+                                                                          m->fcInPad, B);
     dan_count_launch();
   }
   // FC trunk: [Dropout] Linear ReLU Dropout ... (model.py:369-377), then the heads on the dropped-out last activation
@@ -691,16 +702,32 @@ int dan_backward_impl(dan_model* m, const dan_weights* w, const DevInputs& in, c
   // dA = d(dropped-out FC input) [B][fcInPad]: undo dropout 0
   dropout_kernel<<<grid1d((long)B * m->fcInPad), 256, 0, st>>>(dA, dA, (long)B * m->fcInPad, dropout_p, seed, 0u);
   dan_count_launch();
+  // ---- post-pool Linear: dA[:, 0:D) through its ReLU, weight / bias gradients, data gradient into the pooled features ----
+  const int Dp = m->cfg.pool_combine_dimension;
+  const float* dpooled = dA;
+  int dpooled_ld = m->fcInPad;
+  if (Dp > 0) {
+    relu_mask_kernel<<<grid1d((long)B * m->fcInPad), 256, 0, st>>>(dA, FCIN, (long)B * m->fcInPad);      // the highway block is masked alike below
+    dan_count_launch();
+    const float* POOLED = reinterpret_cast<const float*>(base + pl.pooled);
+    if ((rc = tr_wgrad(dA, m->fcInPad, POOLED, m->pooledPad, B, 0, Dp, m->pooledPad, m->pooled, G_(grads->post_pool_w), m->pooled, 1, TNP, pl.tn_part_floats, st))) return rc;
+    if ((rc = tr_colsum(dA, m->fcInPad, B, Dp, G_(grads->post_pool_b), RED, st))) return rc;
+    float* DP = reinterpret_cast<float*>(base + pl.dpooled);
+    // d(pooled) = dpre . W_post: the torch weight (D, pooled) row-major is the K-major operand of this product
+    if ((rc = tr_linear(dA, m->fcInPad, B, Dp, w->post_pool_w, m->pooled, m->pooled, nullptr, 0, nullptr, 0, DP, m->pooledPad, TNP, pl.tn_part_floats, st))) return rc;
+    dpooled = DP; dpooled_ld = m->pooledPad;
+  }
   // ---- highway features and final pools ----
   if (m->cfg.highway) {
-    highway_bwd_kernel<<<grid1d((long)B * L * bott * m->R), 256, 0, st>>>(HW, pl.hw_layer_stride, L, bott, m->R, m->cfg.concat_hw_reads, FCIN + m->pooled, dA + m->pooled,
+    const int hw0 = Dp > 0 ? Dp : m->pooled;
+    highway_bwd_kernel<<<grid1d((long)B * L * bott * m->R), 256, 0, st>>>(HW, pl.hw_layer_stride, L, bott, m->R, m->cfg.concat_hw_reads, FCIN + hw0, dA + hw0,
                                                                          m->fcInPad, DHW, B);
     dan_count_launch();
   }
   float* GA = R_(pl.ga, C);      // d(layer output) of the layer being processed
   float* GB = R_(pl.gb, C);
   DAN_CUDA_TRY(cudaMemsetAsync(base + pl.ga, 0, pl.dhw - pl.ga, st));      // gap rows of the gradient row matrices
-  pool_final_bwd_kernel<<<dim3(g.P, B), 128, 0, st>>>(R_(pl.h[L - 1], C), C, dA, m->fcInPad, GA, C, g, m->cfg.skip_final_maxpool);
+  pool_final_bwd_kernel<<<dim3(g.P, B), 128, 0, st>>>(R_(pl.h[L - 1], C), C, dpooled, dpooled_ld, GA, C, g, m->cfg.skip_final_maxpool);
   dan_count_launch();
   DAN_CUDA_TRY(cudaGetLastError());
   float* POOLG = reinterpret_cast<float*>(base + pl.pool);      // forward's pool table is dead by now: reused for the pool-add backward

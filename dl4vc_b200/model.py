@@ -357,7 +357,8 @@ class Basic2DNet(nn.Module):
         lib = _lib.load_library()
         need = (lib.dan_workspace_bytes_host if host else lib.dan_workspace_bytes)(st.handle, batch, prec)
         if need == 0:
-            raise NotImplementedError("precision '%s' is not available for this configuration" % self.precision)
+            raise NotImplementedError("precision '%s' is not available for this configuration: %s"
+                                      % (self.precision, lib.dan_last_error().decode(errors="replace")))
         key = (prec, host)
         ws = st.workspace.get(key)
         if ws is None or ws.numel() < need:
@@ -466,6 +467,8 @@ class Basic2DNet(nn.Module):
             if cfg.highway:
                 out += [(f"bott_w.{l}", self.conv1D_bottleneck_layers[l].weight), (f"bott_b.{l}", self.conv1D_bottleneck_layers[l].bias),
                         (f"comp_w.{l}", self.conv1D_compression_layers[l].weight), (f"comp_b.{l}", self.conv1D_compression_layers[l].bias)]
+        if cfg.pool_combine_dimension > 0:
+            out += [("post_pool_w", self.post_pool_conv1D.weight), ("post_pool_b", self.post_pool_conv1D.bias)]
         for i, idx in enumerate(cfg.fc_indices):
             out += [(f"fc_w.{i}", self.conv2hidden[idx].weight), (f"fc_b.{i}", self.conv2hidden[idx].bias)]
         for n in HEAD_NAMES:
@@ -487,7 +490,7 @@ class Basic2DNet(nn.Module):
 
         for name, t in tensors.items():
             field, _, idx = name.partition(".")
-            if field in ("embeddings", "head_w", "head_b"):
+            if field in ("embeddings", "post_pool_w", "post_pool_b", "head_w", "head_b"):
                 setattr(w, field, ptr(t))
             else:
                 getattr(w, field)[int(idx)] = ptr(t)

@@ -3,9 +3,10 @@ reference's nn.DataParallel replicas, main.py:117), ONE bucketed gradient all-re
 broadcast + reduce_add to GPU 0, and an all-reduce(max) of the per-example "close" table so that every rank's AdjustableDataSampler
 (dl4vc/dataset.py:697-746) draws the same epoch list, which is then strided by rank.
 
-The native backward produces the FC-trunk gradients first (97 % of the bytes: conv2hidden.1 is 302 MB): `allreduce_gradients` sends that
-bucket off on a side stream as soon as the backward call has been enqueued, the small conv-stack bucket afterwards; torch.distributed
-(NCCL over NVLink on the GPU box, gloo in the CPU tests) is plumbing only."""
+The native backward produces the FC-trunk gradients first (97 % of the bytes: conv2hidden.1 is 302 MB), then, with pool_combine_dimension > 0,
+the post-pool Linear's (105 M parameters at D = 2048, more than PROD's whole FC trunk): `allreduce_gradients` sends that bucket off on a side
+stream as soon as the backward call has been enqueued, the small conv-stack bucket afterwards; torch.distributed (NCCL over NVLink on the GPU
+box, gloo in the CPU tests) is plumbing only."""
 from __future__ import annotations
 
 import torch
@@ -30,7 +31,7 @@ def sync_close_table(table: torch.Tensor, group=None):
 
 
 class GradientAllReducer:
-    """Averages .grad over the ranks in two flat buckets: [FC trunk + heads] and [everything else]."""
+    """Averages .grad over the ranks in two flat buckets: [FC trunk + heads + post-pool Linear] and [everything else]."""
 
     def __init__(self, model, group=None):
         self.group = group
@@ -39,7 +40,7 @@ class GradientAllReducer:
         for name, p in m.named_parameters():
             if not p.requires_grad:
                 continue
-            (big if name.startswith(("conv2hidden", "fcHidden2")) else small).append(p)
+            (big if name.startswith(("conv2hidden", "fcHidden2", "post_pool_conv1D")) else small).append(p)
         self.buckets = [big, small]
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.side = torch.cuda.Stream() if torch.cuda.is_available() and any(p.is_cuda for p in big + small) else None

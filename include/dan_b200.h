@@ -194,7 +194,8 @@ int dan_make_mask_vectors(const char* const* ref_alleles, const char* const* var
  *
  * dan_backward: d(loss)/d(heads) (batch*27, w.r.t. the returned, activated outputs) -> gradient of every parameter tensor, written
  * (not accumulated) into the tensors `grads` points to (same layout as `params`; head_w / head_b as the 27-row concatenation;
- * entries may be NULL to skip embeddings). Must follow dan_train_forward on the same tape, inputs, seed and dropout_p. */
+ * embeddings may be NULL to skip the embedding table; post_pool_w / post_pool_b are required, in params and in grads, when
+ * pool_combine_dimension > 0). Must follow dan_train_forward on the same tape, inputs, seed and dropout_p. */
 size_t dan_train_tape_bytes(const dan_model* m, int batch);
 int dan_train_forward(dan_model* m, const dan_weights* params, const uint8_t* reads, const uint8_t* q_scores, const uint8_t* strands,
                       const uint8_t* ref, const uint8_t* ref_masks, const uint8_t* var_masks, const uint8_t* removed, int batch,
@@ -266,8 +267,8 @@ int dan_encode_bf16(dan_model* m, const uint8_t* reads, const uint8_t* q_scores,
                     const uint8_t* ref, const uint8_t* ref_masks, const uint8_t* var_masks, int batch,
                     float* x0_out, void* stream);
 
-/* Test hook: after a dan_forward call on `workspace`, copy the FC input vector (pooled max|mean|relu(highway),
- * dl4vc/model.py:838-912) of the LAST internal pass to out (rows x fc_in_features fp32, DEVICE pointer).
+/* Test hook: after a dan_forward call on `workspace`, copy the FC input vector (pooled max|mean, or relu(post_pool(pooled)) when
+ * pool_combine_dimension > 0, then relu(highway); dl4vc/model.py:838-912) of the LAST internal pass to out (rows x fc_in_features fp32, DEVICE pointer).
  * Returns the number of rows written, or a negative error. */
 int dan_debug_fc_input(dan_model* m, int precision, int batch, const void* workspace, float* out, void* stream);
 
