@@ -493,10 +493,13 @@ const char* dan_bf16_unsupported_reason(const dan_model* m) {
   if (m->cfg.highway && !(m->bott == 32 || m->bott == 64)) return "the highway bottleneck must be 32 or 64 wide";
   if (m->geom.gap > kLead) return "dilation above 8";
   if (m->CinPad % 16) return "padded input channels must be a multiple of 16";
+  // a layer-1 input tile slot (dan_layerwise.cuh) and the fused kernel's read buffer (kStkBuf) hold kKC = 16 channel planes
+  if (m->CinPad > kC) return "more than 128 padded input channels (embed_dim 62-64 with q-scores, strands and masks)";
   for (int i = 0; i < m->cfg.num_fc; ++i) if (m->cfg.fc_sizes[i] % 32) return "FC widths must be multiples of 32";
   return nullptr;
 }
 int dan_bf16_supported(const dan_model* m) { return dan_bf16_unsupported_reason(m) == nullptr; }
+int dan_bf16_route(const dan_model* m) { return dan_bf16_unsupported_reason(m) ? 0 : stack_fused(m) ? 1 : 2; }
 
 size_t dan_bf16_workspace_bytes(const dan_model* m, int batch) {
   if (const char* why = dan_bf16_unsupported_reason(m)) {

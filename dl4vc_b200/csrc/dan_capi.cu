@@ -176,6 +176,11 @@ int dan_model_set_flags(dan_model* m, int flags) {
   return DAN_OK;
 }
 
+int dan_model_bf16_route(const dan_model* m) {
+  if (!m) { dan_set_error("null model"); return DAN_E_INVALID; }
+  return dan_bf16_route(m);
+}
+
 size_t dan_workspace_bytes(const dan_model* m, int batch, int precision) {
   if (!m || batch < 0) return 0;
   if (precision == DAN_PRECISION_BF16) return dan_bf16_workspace_bytes(m, batch);
@@ -316,7 +321,11 @@ int dan_encode_bf16(dan_model* m, const uint8_t* reads, const uint8_t* q_scores,
 }
 
 size_t dan_train_tape_bytes(const dan_model* m, int batch) {
-  if (!m || batch < 1 || !dan_train_supported(m)) return 0;
+  if (!m || batch < 1) return 0;
+  if (const char* why = dan_train_unsupported_reason(m)) {
+    dan_set_error("training kernels do not cover this configuration: %s", why);
+    return 0;
+  }
   return dan_train_tape_bytes_impl(m, batch);
 }
 
@@ -327,7 +336,7 @@ static int check_train_args(dan_model* m, const dan_weights* params, const uint8
   if (!params) { dan_set_error("null parameter struct"); return DAN_E_INVALID; }
   if (batch < 1) { dan_set_error("training needs at least one candidate"); return DAN_E_INVALID; }
   if (!(dropout_p >= 0.f && dropout_p < 1.f)) { dan_set_error("dropout probability %g outside [0, 1)", dropout_p); return DAN_E_INVALID; }
-  if (!dan_train_supported(m)) { dan_set_error("training kernels do not cover this configuration (channels must be a multiple of 4, at most 1024)"); return DAN_E_UNSUPPORTED; }
+  if (const char* why = dan_train_unsupported_reason(m)) { dan_set_error("training kernels do not cover this configuration: %s", why); return DAN_E_UNSUPPORTED; }
   for (int l = 0; l < m->L; ++l)
     if (m->cfg.use_batchnorm && (!params->bn_w[l] || !params->bn_b[l] || !params->bn_mean[l] || !params->bn_var[l])) { dan_set_error("missing BatchNorm tensors of layer %d", l + 1); return DAN_E_INVALID; }
   if (m->cfg.pool_combine_dimension > 0 && (!params->post_pool_w || !params->post_pool_b)) { dan_set_error("missing post_pool_w / post_pool_b"); return DAN_E_INVALID; }

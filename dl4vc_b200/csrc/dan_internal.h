@@ -132,9 +132,10 @@ int dan_bf16_pack(dan_model* m, const dan_weights* w, cudaStream_t st);
 void dan_bf16_free(dan_model* m);
 int dan_bf16_supported(const dan_model* m);
 const char* dan_bf16_unsupported_reason(const dan_model* m);     // nullptr when the bf16 path takes the configuration
+int dan_bf16_route(const dan_model* m);                          // dan_model_bf16_route
 
 // training path (dan_train.cu)
-int dan_train_supported(const dan_model* m);
+const char* dan_train_unsupported_reason(const dan_model* m);    // nullptr when the training kernels take the configuration
 size_t dan_train_tape_bytes_impl(const dan_model* m, int batch);
 int dan_train_forward_impl(dan_model* m, const dan_weights* w, const DevInputs& in, const uint8_t* removed, int batch, float dropout_p, uint64_t seed,
                            float* heads_out, void* tape, size_t tape_bytes, cudaStream_t st);

@@ -395,7 +395,7 @@ TrainPlan make_train_plan(const dan_model* m, int B) {
   const size_t rowC = (size_t)pl.rowsAlloc * C * 4;
   pl.x0 = take((size_t)pl.rowsAlloc * m->CinPad * 4);
   for (int l = 0; l < L; ++l) {
-    pl.u[l] = take(rowC);
+    pl.u[l] = take(l == 0 && m->CinPad > C ? (size_t)pl.rowsAlloc * m->CinPad * 4 : rowC);      // the backward writes d(x0) into U of layer 1
     pl.y[l] = m->cfg.use_batchnorm ? take(rowC) : pl.u[l];
     pl.h[l] = m->cfg.is_residual[l] ? take(rowC) : pl.y[l];
     pl.inp[l] = (l > 0 && m->cfg.pool_after[l - 1]) ? take(rowC) : 0;
@@ -499,9 +499,13 @@ int tr_colsum(const float* X, int ldx, long rows, int C, float* out, double* red
 
 size_t dan_train_tape_bytes_impl(const dan_model* m, int batch) { return make_train_plan(m, batch).total; }
 
-int dan_train_supported(const dan_model* m) {
-  if (m->C % 4 || m->C > 1024) return 0;
-  return 1;
+const char* dan_train_unsupported_reason(const dan_model* m) {
+  if (m->C % 4 || m->C > 1024) return "channels must be a multiple of 4, at most 1024";
+  // the gradient of a residual layer fed by a pool-add (its residual bypasses the pool term, model.py:732 vs :742) is not implemented;
+  // rejected here, before dan_train_forward has moved the BatchNorm running statistics
+  for (int l = 1; l < m->L; ++l)
+    if (m->cfg.pool_after[l - 1] && m->cfg.is_residual[l]) return "a residual layer directly behind a pool-add";
+  return nullptr;
 }
 
 int dan_train_forward_impl(dan_model* m, const dan_weights* w, const DevInputs& in, const uint8_t* removed, int batch, float dropout_p, uint64_t seed,
@@ -804,7 +808,7 @@ int dan_backward_impl(dan_model* m, const dan_weights* w, const DevInputs& in, c
     dan_count_launch();
     {
       // d(conv_in)[m][cin] = sum_tap dZ[m - (t-1) d][:] . w[:, cin, tap]: the same tap-gathering GEMM with mirrored offsets
-      float* DIN = (l == 0) ? R_(pl.u[0], C) : GA;      // layer 1: its (dead) U matrix takes d(x0) (CinPad <= C columns)
+      float* DIN = (l == 0) ? R_(pl.u[0], m->CinPad) : GA;      // layer 1: its (dead) U matrix takes d(x0) (sized for max(C, CinPad) columns)
       GemmParams q{};
       q.A = DZl; q.lda = C; q.a_rows = pl.rowsAlloc - 2 * lead; q.M = (int)rows;
       q.ntaps = 3; q.tap_off[0] = d; q.tap_off[1] = 0; q.tap_off[2] = -d; q.Kc = C;

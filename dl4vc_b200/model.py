@@ -280,6 +280,14 @@ class Basic2DNet(nn.Module):
                 _lib.check(_lib.load_library().dan_model_set_flags(st.handle, self._flags), "set_flags")
         return self
 
+    def bf16_route(self) -> int:
+        """Test hook: the route a bf16 forward takes with the current flags (dan_model_bf16_route): 0 the bf16 path rejects the
+        configuration, 1 the fused conv-stack kernel, 2 layer by layer."""
+        dev = self._device()
+        with torch.cuda.device(dev):
+            st = self._state(dev)
+            return _lib.check(_lib.load_library().dan_model_bf16_route(st.handle), "dan_model_bf16_route")
+
     def _device(self) -> torch.device:
         dev = self.embeddings.weight.device
         if dev.type != "cuda":
@@ -531,7 +539,7 @@ class Basic2DNet(nn.Module):
             B = int(u8[0].shape[0])
             need = lib.dan_train_tape_bytes(st.handle, B)
             if need == 0:
-                raise NotImplementedError("the training kernels do not cover this configuration")
+                raise NotImplementedError(lib.dan_last_error().decode(errors="replace"))
             tape = torch.empty(int(need), dtype=torch.uint8, device=dev)
             keep = []
             names = dict(self._train_params())

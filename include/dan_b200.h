@@ -108,6 +108,12 @@ int dan_model_set_pass_candidates(dan_model* m, int candidates);
 enum { DAN_FLAG_LAYERWISE = 1 };
 int dan_model_set_flags(dan_model* m, int flags);
 
+/* Test hook: which route dan_forward takes at DAN_PRECISION_BF16 with the handle's current flags. 0: the bf16 path does not cover the
+ * configuration (dan_forward returns DAN_E_UNSUPPORTED naming the reason), 1: the fused conv-stack kernel (dan_stack.cuh), 2: layer by
+ * layer (dan_layerwise.cuh). */
+enum { DAN_BF16_ROUTE_NONE = 0, DAN_BF16_ROUTE_FUSED = 1, DAN_BF16_ROUTE_LAYERWISE = 2 };
+int dan_model_bf16_route(const dan_model* m);
+
 /* Bytes of device scratch dan_forward needs for a batch of `batch` candidates at `precision`. */
 size_t dan_workspace_bytes(const dan_model* m, int batch, int precision);
 

@@ -1,18 +1,17 @@
 """pool_combine_dimension (post_pool_conv1D, model.py:841-843) on the bf16 tensor-core path and in training.
 
 GPU tests (-m gpu) run the kernels against the real reference's goldens, the fp32 path, the numpy oracle and torch autograd over the
-op sequence of oracle/dan_torch_cpu.py in float64; the bucket test runs on the CPU."""
+op sequence of oracle/dan_torch_ref.py in float64; the bucket test runs on the CPU."""
 import numpy as np
 import pytest
 import torch
-import torch.nn.functional as F
 
 from conftest import load_golden, rel_err
-from dl4vc_b200.config import BN_EPS, HEAD_NAMES, Q_SCORE_SCALE_FACTOR, STRAND_ENCODE_FACTOR, min_config, small_config
+from dl4vc_b200.config import min_config, small_config
 from dl4vc_b200.factory import build_model, ctor_kwargs
 from dl4vc_b200.synth import make_pileups
 from dl4vc_b200.weights import synth_state_dict
-from oracle import dan_oracle
+from oracle import dan_oracle, dan_torch_ref
 
 BF16_TOL = 3e-2          # the bf16 bar of tests/test_gpu_parity.py: heads within 3e-2 of the largest |logit|
 GRAD_TOL = 5e-3          # the training bar of tests/test_gpu_train.py: per tensor, relative to its largest |gradient|
@@ -131,75 +130,8 @@ def test_bf16_rejects_a_pool_combine_dimension_the_kernels_do_not_take():
 
 
 # ---------------------------------------------------------------------------------------------------------------- training
-_NOT_TRAINED = ("pe", "bin_output_weights", "vt_output_weights")
-
-
-def _train_reference(cfg, sd, arrays, dtype, dev):
-    """Training-mode forward (batch-statistics BatchNorm with running-statistics update, dropout 0) of the op sequence of
-    oracle/dan_torch_cpu.forward under torch autograd. Returns heads, {name: leaf parameter} and {name: updated running buffer}."""
-    params = {k: v.to(dev, dtype).clone().requires_grad_(True) for k, v in sd.items()
-              if k not in _NOT_TRAINED and "running_" not in k and "num_batches" not in k}
-    bufs = {k: v.to(dev, dtype).clone() for k, v in sd.items() if "running_" in k}
-    reads, q_scores, strands, ref, ref_masks, var_masks = (torch.from_numpy(np.ascontiguousarray(a)).to(dev) for a in arrays)
-    reads, ref = reads.long(), ref.long()
-    E, pe = params["embeddings.weight"], sd["pe"].to(dev, dtype)
-    B, P, R = reads.shape
-    reads_emb = F.embedding(reads, E, padding_idx=0, scale_grad_by_freq=True) + pe.unsqueeze(2)       # nn.Embedding of model.py:143-145
-    ref_emb = (F.embedding(ref, E, padding_idx=0, scale_grad_by_freq=True) + pe).unsqueeze(2).expand(-1, -1, R, -1)
-    x = torch.cat((reads_emb, ref_emb), dim=3)
-    if cfg.use_q_scores:
-        x = torch.cat((x, (q_scores.to(dtype) * Q_SCORE_SCALE_FACTOR).unsqueeze(3)), dim=3)
-    if cfg.use_strands:
-        x = torch.cat((x, (strands.to(dtype) * STRAND_ENCODE_FACTOR).unsqueeze(3)), dim=3)
-    if cfg.use_reads_ref_var_mask:
-        chans, nzs = [], []
-        for m in (ref_masks, var_masks):
-            m = m.long().unsqueeze(2)
-            nz = (m != 0).long()
-            agree = ((reads * nz) == m).long().sum(dim=1) == P
-            chans.append((nz * agree.unsqueeze(1).long()).to(dtype))
-            nzs.append(nz)
-        chans.append(nzs[0].expand(-1, -1, R).to(dtype))
-        x = torch.cat([x] + [c.unsqueeze(3) for c in chans], dim=3)
-    h = x.permute(0, 3, 2, 1)
-    pool, hw, res_i = None, [], 0
-    for l in range(1, cfg.total_conv_layers + 1):
-        resid = h
-        if pool is not None:
-            h = h + pool
-            pool = None
-        d = cfg.dilation(l)
-        h = F.relu(F.conv2d(h, params[f"conv1D_layers.{l-1}.weight"], params[f"conv1D_layers.{l-1}.bias"], padding=(0, d), dilation=d))
-        if cfg.use_batchnorm:
-            p = f"bn1D_layers.{l-1}."
-            h = F.batch_norm(h, bufs[p + "running_mean"], bufs[p + "running_var"], params[p + "weight"], params[p + "bias"],
-                             training=True, momentum=0.1, eps=BN_EPS)
-        if cfg.is_residual(l):
-            h = F.conv2d(h, params[f"residual_conv_layers.{res_i}.weight"], params[f"residual_conv_layers.{res_i}.bias"]) + resid
-            res_i += 1
-        if l in cfg.conv_1d_pool_layers:
-            pool = F.avg_pool2d(h, kernel_size=(R, 1), ceil_mode=True)
-        if cfg.highway:
-            t = F.relu(F.conv2d(h, params[f"conv1D_bottleneck_layers.{l-1}.weight"], params[f"conv1D_bottleneck_layers.{l-1}.bias"]))
-            o = F.conv2d(t, params[f"conv1D_compression_layers.{l-1}.weight"], params[f"conv1D_compression_layers.{l-1}.bias"])
-            hw.append(o.reshape(B, -1))
-    mean = F.avg_pool2d(h, kernel_size=(R, 1), ceil_mode=True)
-    if cfg.skip_final_maxpool:
-        pooled = mean.reshape(B, -1)
-    else:
-        pooled = torch.cat((F.max_pool2d(h, kernel_size=(R, 1), ceil_mode=True), mean), dim=1).reshape(B, -1)
-    if cfg.pool_combine_dimension > 0:
-        pooled = F.relu(F.linear(pooled, params["post_pool_conv1D.weight"], params["post_pool_conv1D.bias"]))
-    if cfg.highway:
-        hwv = torch.cat(hw, dim=1) if cfg.concat_hw_reads else torch.stack(hw, 0).mean(0)
-        pooled = torch.cat((pooled, F.relu(hwv)), dim=1)
-    xh = pooled
-    for idx in cfg.fc_indices:
-        xh = F.relu(F.linear(xh, params[f"conv2hidden.{idx}.weight"], params[f"conv2hidden.{idx}.bias"]))
-    outs = [F.linear(xh, params[n + ".weight"], params[n + ".bias"]) for n in HEAD_NAMES]
-    outs[2] = torch.sigmoid(outs[2])
-    outs[3] = F.leaky_relu(outs[3], 0.01)
-    return torch.cat(outs, dim=1), params, bufs
+_NOT_TRAINED = dan_torch_ref.NOT_TRAINED
+_train_reference = dan_torch_ref.train_reference
 
 
 def _sampled(a):

@@ -57,3 +57,20 @@ def test_torch_cpu_port_matches_reference_goldens(golden):
     reads, q, s, ref, rm, vm = golden["arrays"]
     heads = dan_torch_cpu.forward(cfg, sd, reads, ref, q, s, rm, vm).numpy()
     assert rel_err(heads, golden["heads"]) < 5e-6
+
+
+def test_float64_torch_reference_matches_reference_goldens(golden):
+    """oracle/dan_torch_ref.py, the float64 yardstick of the GPU configuration sweep, gives the reference's results: heads and the
+    sampled FC input of candidate 0, with its FC-input blocks tiling the whole vector."""
+    import torch
+
+    from oracle import dan_torch_ref
+
+    cfg = golden["cfg"]
+    sd = synth_state_dict(cfg, seed=golden["seed"])
+    res = dan_torch_ref.forward(cfg, sd, golden["arrays"], dtype=torch.float64)
+    assert res.heads.dtype == torch.float64
+    assert rel_err(res.heads.numpy(), golden["heads"]) < 5e-6
+    fc_in = res.fc_in.numpy()
+    np.testing.assert_allclose(fc_in[0][::37], golden["fc_in_cand0_sample"], rtol=1e-3, atol=1e-4)
+    assert np.array_equal(np.concatenate([b.numpy() for b in res.blocks.values()], axis=1), fc_in)
