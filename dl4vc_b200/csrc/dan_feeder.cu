@@ -93,6 +93,181 @@ int parse_vcf_record(const std::string& rec_in, VcfInfo* out, std::string* ref_a
   return DAN_REC_OK;
 }
 
+// ---- header pass: everything of the decode that is not tile bytes (host, shared by the host and the device decode) --------------
+// Row window + sample_single_reads selection, parse_vcf, allele counts at the proposal column over the chosen rows, coverage /
+// allele_freq, proposal masks, blacklist and status. Writes the scalars of record i into `out` (each may be NULL), the masks into
+// rm / vm, and the chosen stored rows into *h. `key` seeds the draw of deep pileups (the record's index in its file).
+int header_pass(const uint8_t* rec, int64_t key, const dan_feeder_config* cfg, int R, int S, const dan_record_batch* out, int i,
+                uint8_t* rm, uint8_t* vm, dan_record_header* h) {
+  int32_t num_reads;
+  memcpy(&num_reads, rec + kOffNumReads, 4);
+  // A. window of stored rows (dataset.py:517-521), B. at most R of them (sample_single_reads, dataset.py:256-287)
+  const int middle = (num_reads > S ? num_reads : S) / 2;
+  int start = (int)((double)middle - (double)S / 2.0);
+  if (start < 0) start = 0;
+  const int avail = start < kRecRows ? (kRecRows - start < S ? kRecRows - start : S) : 0;      // columns of the transposed window
+  const int max_reads = R < avail ? R : avail;
+  int perm[kRecRows];
+  if (max_reads >= num_reads) {
+    for (int j = 0; j < max_reads; ++j) perm[j] = j;                                              // the first max_reads columns, deterministic
+  } else {
+    // a sorted random subset of the first min(avail, num_reads) columns: the reference draws it with an unseeded np.random.choice
+    // (its inference is not reproducible for deep pileups, SURVEY App. G); here the draw is a function of (seed, record index)
+    const int total = avail < num_reads ? avail : num_reads;
+    uint64_t st = cfg->seed ^ (0xD1B54A32D192ED03ull * (uint64_t)(key + 1));
+    int pool[kRecRows];
+    for (int j = 0; j < total; ++j) pool[j] = j;
+    for (int j = 0; j < max_reads; ++j) { const int k = j + (int)(splitmix(st) % (uint64_t)(total - j)); const int t = pool[j]; pool[j] = pool[k]; pool[k] = t; }
+    bool take[kRecRows] = {};
+    for (int j = 0; j < max_reads; ++j) take[pool[j]] = true;
+    for (int j = 0, k = 0; j < total; ++j) if (take[j]) perm[k++] = j;
+  }
+  memset(h, 0, sizeof(*h));
+  h->window_start = start;
+  h->num_rows = max_reads;
+  for (int j = 0; j < max_reads; ++j) h->rows[j] = (uint8_t)(start + perm[j]);      // start + perm[j] < start + avail <= kRecRows
+  const uint8_t* ref = rec + kOffRefBases;
+  if (out->label) out->label[i] = rec[kOffLabel];
+  if (out->num_reads) out->num_reads[i] = num_reads;
+  // vcfrec: S128, trailing NULs stripped like numpy does
+  size_t len = 128;
+  while (len > 0 && rec[kOffVcf + len - 1] == 0) --len;
+  const std::string vcf(reinterpret_cast<const char*>(rec + kOffVcf), len);
+  VcfInfo vi{};
+  std::string xa, ya;
+  int status = parse_vcf_record(vcf, &vi, &xa, &ya);
+  h->ref_len = (int32_t)xa.size();
+  h->var_len = (int32_t)ya.size();
+  memset(rm, 0, kRecP); memset(vm, 0, kRecP);
+  int blacklist = 0;
+  if (status == DAN_REC_OK) {
+    // coverage / allele frequency from the sampled reads at the proposal column (count_variants_from_single_reads, dataset.py:340-362);
+    // tile column j of the reads holds stored row h->rows[j], so the column is read from the record itself
+    int ref_base; int col;
+    if (vi.var_mode == 1) { ref_base = ref[100]; col = 100; }
+    else if (vi.var_mode == 3) { ref_base = ref[101]; col = 101; }
+    else { ref_base = 8; col = 101; }
+    int agree = 0, disagree = 0;
+    for (int j = 0; j < max_reads; ++j) {
+      const int t = rec[kOffSingle + (size_t)h->rows[j] * kRecP + col];
+      if (t == ref_base) ++agree;
+      else if (t == 1 || t == 2 || t == 3 || t == 4 || t == 5 || t == 8 || t == 9) ++disagree;      // real_base_keys_set: A T C G - M noinsert
+    }
+    // columns beyond max_reads do not exist in the reference's slice: only the chosen rows count
+    const int cover = agree + disagree;
+    int coverage = vi.coverage; double af = vi.allele_freq;
+    if (cover > 0) { coverage = cover; if (!cfg->keep_candidate_af) af = (double)disagree / (double)cover; }
+    if (out->is_snp) out->is_snp[i] = (uint8_t)vi.is_snp;
+    if (out->var_type) out->var_type[i] = vi.var_type;
+    if (out->allele_freq) out->allele_freq[i] = (float)af;
+    if (out->coverage) out->coverage[i] = coverage;
+    if (out->var_base_enum) out->var_base_enum[i] = vi.var_base;
+    if (out->var_ref_enum) out->var_ref_enum[i] = vi.ref_base;
+    // proposal masks (get_read_mask_vectors); an AssertionError there blacklists the example and leaves all-pad masks (dataset.py:644-664)
+    const int mcode = mask_one(xa.c_str(), ya.c_str(), ref, rm, vm);
+    if (mcode != DAN_MASK_OK) {
+      memset(rm, 0, kRecP); memset(vm, 0, kRecP);
+      if (mcode == DAN_MASK_E_SHAPE || mcode == DAN_MASK_E_REF_MISMATCH) blacklist = 1;      // assert -> caught
+      else status = DAN_REC_E_MASK;                                                            // KeyError / ValueError / UnboundLocalError propagate in the reference
+    }
+  }
+  if (out->blacklist) out->blacklist[i] = (uint8_t)blacklist;
+  if (out->status) out->status[i] = status;
+  return status;
+}
+
+// host tile pass: tile column j = stored row h.rows[j] transposed to [position][read]; columns past num_rows stay zero
+void host_tiles(const uint8_t* rec, const dan_record_header& h, const dan_feeder_config* cfg, int R, const dan_record_batch* out, int i) {
+  const size_t tile = (size_t)kRecP * R;
+  uint8_t* reads = out->reads + (size_t)i * tile;
+  uint8_t* q = out->q_scores ? out->q_scores + (size_t)i * tile : nullptr;
+  uint8_t* sd = out->strands ? out->strands + (size_t)i * tile : nullptr;
+  memset(reads, 0, tile);
+  if (q) memset(q, 0, tile);
+  if (sd) memset(sd, 0, tile);
+  for (int j = 0; j < h.num_rows; ++j) {
+    const uint8_t* row = rec + kOffSingle + (size_t)h.rows[j] * kRecP;
+    const uint8_t* qrow = rec + kOffQ + (size_t)h.rows[j] * kRecP;
+    const uint8_t* srow = rec + kOffStrand + (size_t)h.rows[j] * kRecP;
+    for (int p = 0; p < kRecP; ++p) {
+      reads[(size_t)p * R + j] = row[p];
+      if (q && cfg->use_q_scores) q[(size_t)p * R + j] = qrow[p];
+      if (sd && cfg->use_strands) sd[(size_t)p * R + j] = srow[p];
+    }
+  }
+  memcpy(out->ref + (size_t)i * kRecP, rec + kOffRefBases, kRecP);
+}
+
+int check_feeder_config(const dan_feeder_config* cfg, int* R, int* S) {
+  *R = cfg->max_reads; *S = cfg->store_max_reads < kRecRows ? cfg->store_max_reads : kRecRows;
+  if (*R < 1 || *R > kRecRows || *S < 1) { dan_set_error("max_reads %d / store_max_reads %d out of range", *R, cfg->store_max_reads); return DAN_E_INVALID; }
+  return DAN_OK;
+}
+
+// ---- device tile pass ------------------------------------------------------------------------------------------------------------
+// Layout of the device workspace, and of the pinned host staging buffer it is copied from in one piece:
+//   [n records, DAN_RECORD_BYTES apart][pad to 16][n dan_record_header][n*201 ref_masks][n*201 var_masks]
+struct StagingLayout { size_t hdr, rm, vm, total; };
+StagingLayout staging_layout(int n) {
+  StagingLayout l;
+  l.hdr = ((size_t)n * kRecBytes + 15) & ~(size_t)15;
+  l.rm = l.hdr + (size_t)n * sizeof(dan_record_header);
+  l.vm = l.rm + (size_t)n * kRecP;
+  l.total = ((l.vm + (size_t)n * kRecP) + 15) & ~(size_t)15;
+  return l;
+}
+
+constexpr int kTileThreads = 256;
+
+// grid (n, 3): block (i, t) writes tile t (0 reads, 1 q-scores, 2 strands) of record i. The chosen rows are gathered into a
+// [position][read] image of the tile in shared memory (zero past num_rows, or everywhere for a tile the config leaves unused),
+// placed at the output address's offset mod 16, so the tile leaves shared memory in aligned 16-byte stores; only the bytes before
+// the first and after the last 16-byte boundary of the record's range go out one by one. Blocks of tile 0 also copy ref_bases
+// and the header pass's masks.
+__global__ void decode_tiles_kernel(const uint8_t* __restrict__ ws, int n, int R, int use_q, int use_s,
+                                                                      size_t hdr_off, size_t rm_off, size_t vm_off,
+                                                                      uint8_t* __restrict__ reads, uint8_t* __restrict__ q, uint8_t* __restrict__ sd,
+                                                                      uint8_t* __restrict__ ref, uint8_t* __restrict__ ref_masks, uint8_t* __restrict__ var_masks) {
+  extern __shared__ uint4 tile_smem[];
+  __shared__ uint8_t rows[kRecRows];
+  const int i = blockIdx.x, t = blockIdx.y, tid = threadIdx.x;
+  uint8_t* dst_base = t == 0 ? reads : t == 1 ? q : sd;
+  if (!dst_base) return;
+  const int T = kRecP * R;
+  uint8_t* dst = dst_base + (size_t)i * T;
+  const int mis = (int)((uintptr_t)dst & 15);
+  uint8_t* s = reinterpret_cast<uint8_t*>(tile_smem) + mis;
+  const dan_record_header* h = reinterpret_cast<const dan_record_header*>(ws + hdr_off) + i;
+  const int num_rows = h->num_rows;
+  const bool fill = t == 0 || (t == 1 && use_q) || (t == 2 && use_s);
+  for (int k = tid; k < (T + 31) / 16; k += kTileThreads) tile_smem[k] = make_uint4(0, 0, 0, 0);
+  if (tid < num_rows) rows[tid] = h->rows[tid];
+  __syncthreads();
+  if (fill) {
+    const uint8_t* src = ws + (size_t)i * kRecBytes + (t == 0 ? kOffSingle : t == 1 ? kOffQ : kOffStrand);
+    for (int e = tid; e < num_rows * kRecP; e += kTileThreads) {        // consecutive threads read consecutive bytes of one stored row
+      const int j = e / kRecP, p = e - j * kRecP;
+      s[p * R + j] = src[rows[j] * kRecP + p];
+    }
+  }
+  __syncthreads();
+  const int head = min((16 - mis) & 15, T);
+  const int chunks = (T - head) >> 4;
+  for (int k = tid; k < head; k += kTileThreads) dst[k] = s[k];
+  const uint4* s4 = reinterpret_cast<const uint4*>(s + head);
+  uint4* d4 = reinterpret_cast<uint4*>(dst + head);
+  for (int k = tid; k < chunks; k += kTileThreads) d4[k] = s4[k];
+  for (int k = head + chunks * 16 + tid; k < T; k += kTileThreads) dst[k] = s[k];
+  if (t == 0) {
+    const uint8_t* rb = ws + (size_t)i * kRecBytes + kOffRefBases;
+    for (int k = tid; k < kRecP; k += kTileThreads) {
+      ref[(size_t)i * kRecP + k] = rb[k];
+      ref_masks[(size_t)i * kRecP + k] = ws[rm_off + (size_t)i * kRecP + k];
+      var_masks[(size_t)i * kRecP + k] = ws[vm_off + (size_t)i * kRecP + k];
+    }
+  }
+}
+
 }  // namespace
 
 extern "C" {
@@ -102,101 +277,63 @@ int dan_decode_records(const void* records, size_t record_stride, const int64_t*
   if (n == 0) return DAN_OK;
   if (!records || !indices || !cfg || !out || !out->reads || !out->ref || !out->ref_masks || !out->var_masks) { dan_set_error("null pointer"); return DAN_E_INVALID; }
   if (record_stride < DAN_RECORD_BYTES) { dan_set_error("record stride %zu below the %d-byte record", record_stride, DAN_RECORD_BYTES); return DAN_E_INVALID; }
-  const int R = cfg->max_reads, S = cfg->store_max_reads < kRecRows ? cfg->store_max_reads : kRecRows;
-  if (R < 1 || R > kRecRows || S < 1) { dan_set_error("max_reads %d / store_max_reads %d out of range", R, cfg->store_max_reads); return DAN_E_INVALID; }
-  const size_t tile = (size_t)kRecP * R;
+  int R, S;
+  if (check_feeder_config(cfg, &R, &S) != DAN_OK) return DAN_E_INVALID;
   int failed = 0;
   for (int i = 0; i < n; ++i) {
     const uint8_t* rec = static_cast<const uint8_t*>(records) + (size_t)indices[i] * record_stride;
-    int32_t num_reads;
-    memcpy(&num_reads, rec + kOffNumReads, 4);
-    // A. window of stored rows (dataset.py:517-521), B. at most R of them (sample_single_reads, dataset.py:256-287)
-    const int middle = (num_reads > S ? num_reads : S) / 2;
-    int start = (int)((double)middle - (double)S / 2.0);
-    if (start < 0) start = 0;
-    const int avail = start < kRecRows ? (kRecRows - start < S ? kRecRows - start : S) : 0;      // columns of the transposed window
-    const int max_reads = R < avail ? R : avail;
-    int perm[kRecRows];
-    if (max_reads >= num_reads) {
-      for (int j = 0; j < max_reads; ++j) perm[j] = j;                                              // the first max_reads columns, deterministic
-    } else {
-      // a sorted random subset of the first min(avail, num_reads) columns: the reference draws it with an unseeded np.random.choice
-      // (its inference is not reproducible for deep pileups, SURVEY App. G); here the draw is a function of (seed, record index)
-      const int total = avail < num_reads ? avail : num_reads;
-      uint64_t st = cfg->seed ^ (0xD1B54A32D192ED03ull * (uint64_t)(indices[i] + 1));
-      int pool[kRecRows];
-      for (int j = 0; j < total; ++j) pool[j] = j;
-      for (int j = 0; j < max_reads; ++j) { const int k = j + (int)(splitmix(st) % (uint64_t)(total - j)); const int t = pool[j]; pool[j] = pool[k]; pool[k] = t; }
-      bool take[kRecRows] = {};
-      for (int j = 0; j < max_reads; ++j) take[pool[j]] = true;
-      for (int j = 0, k = 0; j < total; ++j) if (take[j]) perm[k++] = j;
-    }
-    uint8_t* reads = out->reads + (size_t)i * tile;
-    uint8_t* q = out->q_scores ? out->q_scores + (size_t)i * tile : nullptr;
-    uint8_t* sd = out->strands ? out->strands + (size_t)i * tile : nullptr;
-    memset(reads, 0, tile);
-    if (q) memset(q, 0, tile);
-    if (sd) memset(sd, 0, tile);
-    for (int j = 0; j < max_reads; ++j) {
-      const uint8_t* row = rec + kOffSingle + (size_t)(start + perm[j]) * kRecP;
-      const uint8_t* qrow = rec + kOffQ + (size_t)(start + perm[j]) * kRecP;
-      const uint8_t* srow = rec + kOffStrand + (size_t)(start + perm[j]) * kRecP;
-      for (int p = 0; p < kRecP; ++p) {
-        reads[(size_t)p * R + j] = row[p];
-        if (q && cfg->use_q_scores) q[(size_t)p * R + j] = qrow[p];
-        if (sd && cfg->use_strands) sd[(size_t)p * R + j] = srow[p];
-      }
-    }
-    uint8_t* ref = out->ref + (size_t)i * kRecP;
-    memcpy(ref, rec + kOffRefBases, kRecP);
-    if (out->label) out->label[i] = rec[kOffLabel];
-    if (out->num_reads) out->num_reads[i] = num_reads;
-    // vcfrec: S128, trailing NULs stripped like numpy does
-    size_t len = 128;
-    while (len > 0 && rec[kOffVcf + len - 1] == 0) --len;
-    const std::string vcf(reinterpret_cast<const char*>(rec + kOffVcf), len);
-    VcfInfo vi{};
-    std::string xa, ya;
-    int status = parse_vcf_record(vcf, &vi, &xa, &ya);
-    uint8_t* rm = out->ref_masks + (size_t)i * kRecP;
-    uint8_t* vm = out->var_masks + (size_t)i * kRecP;
-    memset(rm, 0, kRecP); memset(vm, 0, kRecP);
-    int blacklist = 0;
-    if (status == DAN_REC_OK) {
-      // coverage / allele frequency from the sampled reads at the proposal column (count_variants_from_single_reads, dataset.py:340-362)
-      int ref_base; int col;
-      if (vi.var_mode == 1) { ref_base = ref[100]; col = 100; }
-      else if (vi.var_mode == 3) { ref_base = ref[101]; col = 101; }
-      else { ref_base = 8; col = 101; }
-      int agree = 0, disagree = 0;
-      for (int j = 0; j < max_reads; ++j) {
-        const int t = reads[(size_t)col * R + j];
-        if (t == ref_base) ++agree;
-        else if (t == 1 || t == 2 || t == 3 || t == 4 || t == 5 || t == 8 || t == 9) ++disagree;      // real_base_keys_set: A T C G - M noinsert
-      }
-      // columns beyond max_reads do not exist in the reference's slice; pad columns (token 0) count for neither side unless ref_base is 0
-      if (ref_base == 0 && R > max_reads) { /* the reference's array has exactly max_reads columns */ }
-      const int cover = agree + disagree;
-      int coverage = vi.coverage; double af = vi.allele_freq;
-      if (cover > 0) { coverage = cover; if (!cfg->keep_candidate_af) af = (double)disagree / (double)cover; }
-      if (out->is_snp) out->is_snp[i] = (uint8_t)vi.is_snp;
-      if (out->var_type) out->var_type[i] = vi.var_type;
-      if (out->allele_freq) out->allele_freq[i] = (float)af;
-      if (out->coverage) out->coverage[i] = coverage;
-      if (out->var_base_enum) out->var_base_enum[i] = vi.var_base;
-      if (out->var_ref_enum) out->var_ref_enum[i] = vi.ref_base;
-      // proposal masks (get_read_mask_vectors); an AssertionError there blacklists the example and leaves all-pad masks (dataset.py:644-664)
-      const int mcode = mask_one(xa.c_str(), ya.c_str(), ref, rm, vm);
-      if (mcode != DAN_MASK_OK) {
-        memset(rm, 0, kRecP); memset(vm, 0, kRecP);
-        if (mcode == DAN_MASK_E_SHAPE || mcode == DAN_MASK_E_REF_MISMATCH) blacklist = 1;      // assert -> caught
-        else status = DAN_REC_E_MASK;                                                            // KeyError / ValueError / UnboundLocalError propagate in the reference
-      }
-    }
-    if (out->blacklist) out->blacklist[i] = (uint8_t)blacklist;
-    if (out->status) out->status[i] = status;
-    if (status != DAN_REC_OK) ++failed;
+    dan_record_header h;
+    if (header_pass(rec, indices[i], cfg, R, S, out, i, out->ref_masks + (size_t)i * kRecP, out->var_masks + (size_t)i * kRecP, &h) != DAN_REC_OK) ++failed;
+    host_tiles(rec, h, cfg, R, out, i);
   }
+  if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
+  return DAN_OK;
+}
+
+int dan_decode_record_headers(const void* records, size_t record_stride, const int64_t* indices, int n, const dan_feeder_config* cfg,
+                              const dan_record_batch* out, dan_record_header* headers) {
+  if (n < 0) { dan_set_error("negative record count"); return DAN_E_INVALID; }
+  if (n == 0) return DAN_OK;
+  if (!records || !indices || !cfg || !out || !out->ref_masks || !out->var_masks || !headers) { dan_set_error("null pointer"); return DAN_E_INVALID; }
+  if (record_stride < DAN_RECORD_BYTES) { dan_set_error("record stride %zu below the %d-byte record", record_stride, DAN_RECORD_BYTES); return DAN_E_INVALID; }
+  int R, S;
+  if (check_feeder_config(cfg, &R, &S) != DAN_OK) return DAN_E_INVALID;
+  int failed = 0;
+  for (int i = 0; i < n; ++i) {
+    const uint8_t* rec = static_cast<const uint8_t*>(records) + (size_t)indices[i] * record_stride;
+    if (header_pass(rec, indices[i], cfg, R, S, out, i, out->ref_masks + (size_t)i * kRecP, out->var_masks + (size_t)i * kRecP, headers + i) != DAN_REC_OK) ++failed;
+  }
+  if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
+  return DAN_OK;
+}
+
+size_t dan_decode_records_device_workspace_bytes(int n, const dan_feeder_config* cfg) {
+  int R, S;
+  if (n < 0 || !cfg || check_feeder_config(cfg, &R, &S) != DAN_OK) return 0;
+  return staging_layout(n).total;
+}
+
+int dan_decode_records_device(void* staging, size_t staging_bytes, const int64_t* indices, int n, const dan_feeder_config* cfg,
+                              const dan_record_batch* out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (n < 0) { dan_set_error("negative record count"); return DAN_E_INVALID; }
+  if (n == 0) return DAN_OK;
+  if (!staging || !indices || !cfg || !out || !out->reads || !out->ref || !out->ref_masks || !out->var_masks || !workspace) { dan_set_error("null pointer"); return DAN_E_INVALID; }
+  int R, S;
+  if (check_feeder_config(cfg, &R, &S) != DAN_OK) return DAN_E_INVALID;
+  const StagingLayout l = staging_layout(n);
+  if (staging_bytes < l.total) { dan_set_error("staging buffer of %zu bytes is below the %zu bytes %d records need", staging_bytes, l.total, n); return DAN_E_WORKSPACE; }
+  if (workspace_bytes < l.total) { dan_set_error("device workspace of %zu bytes is below the %zu bytes %d records need", workspace_bytes, l.total, n); return DAN_E_WORKSPACE; }
+  uint8_t* st = static_cast<uint8_t*>(staging);
+  dan_record_header* hdr = reinterpret_cast<dan_record_header*>(st + l.hdr);
+  int failed = 0;
+  for (int i = 0; i < n; ++i)
+    if (header_pass(st + (size_t)i * kRecBytes, indices[i], cfg, R, S, out, i, st + l.rm + (size_t)i * kRecP, st + l.vm + (size_t)i * kRecP, hdr + i) != DAN_REC_OK) ++failed;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  DAN_CUDA_TRY(cudaMemcpyAsync(workspace, staging, l.total, cudaMemcpyHostToDevice, s));
+  const int smem = ((kRecP * R + 31) / 16) * 16;
+  decode_tiles_kernel<<<dim3(n, 3), kTileThreads, smem, s>>>(static_cast<const uint8_t*>(workspace), n, R, cfg->use_q_scores != 0, cfg->use_strands != 0,
+                                                             l.hdr, l.rm, l.vm, out->reads, out->q_scores, out->strands, out->ref, out->ref_masks, out->var_masks);
+  DAN_CUDA_TRY(cudaGetLastError());
   if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
   return DAN_OK;
 }

@@ -11,10 +11,14 @@ scores_on_device   the same post-ops as one CUDA kernel behind the C-ABI (`dan_s
 RecordFile / decode_records  raw fixed-record pileup file (the reference's HDF5 compound type as a flat np.memmap: h5py is not in the image) and
                    the batched C decode of `ContextDatasetFromNumpy._get_generator` (`dataset.py:500-680`: row window, sample_single_reads,
                    parse_vcf, count_variants_from_single_reads, proposal masks) straight into a pinned HostBatch — no per-item Python.
+decode_records_device  the same decode with the tile pass on the GPU (`dan_decode_records_device`): host header pass (parse, sampling,
+                   masks), one H2D copy of the staged raw records, a kernel that writes the device tiles `dan_forward` reads.
+call_record_file   record file -> scored VCF lines and genotype calls, streamed in batches through a ring of pinned slots.
 format_vcf_info    the `BP=..;NV=..;HV=..;OV=..` field `utils.append_vcf_records` splices into VCF column 3 (`utils.py:162-178`).
 """
 from __future__ import annotations
 
+import ctypes as C
 from collections import deque
 
 import numpy as np
@@ -225,7 +229,10 @@ def format_vcf_info_native(scores) -> list:
 
 def splice_vcf_records(vcf_records, bin_score, vt_probs):
     """Records with the score field spliced in, one per line, as append_vcf_records would append them (utils.py:166-178)."""
-    info = format_vcf_info(bin_score, vt_probs)
+    return _splice_info(vcf_records, format_vcf_info(bin_score, vt_probs))
+
+
+def _splice_info(vcf_records, info):
     if len(info) != len(vcf_records):
         raise AssertionError("mis-match between results and VCF to save")          # utils.py:165
     out = []
@@ -264,45 +271,301 @@ class RecordFile:
     def field(self, idx, name):
         return self.raw[idx].view(RECORD_DTYPE)[0][name]
 
+    def read_block(self, start: int, count: int, out):
+        """Copy records [start, start + count) into the first count * RECORD_BYTES bytes of `out` (a uint8 numpy array or CPU tensor,
+        typically pinned staging) with one memcpy; nothing is decoded."""
+        if start < 0 or count < 0 or start + count > len(self):
+            raise IndexError(f"records [{start}, {start + count}) outside the file's {len(self)}")
+        dst = _byte_view(out, count)
+        np.copyto(dst, self.raw[start:start + count].reshape(-1))
+
+    def gather(self, indices, out):
+        """Copy the records `indices` (any order, repeats allowed) back to back into `out`, like read_block does for a range."""
+        idx = np.ascontiguousarray(np.asarray(indices, dtype=np.int64))
+        if len(idx) and (idx.min() < 0 or idx.max() >= len(self)):
+            raise IndexError("record index out of range")
+        dst = _byte_view(out, len(idx))
+        np.take(self.raw, idx, axis=0, out=dst.reshape(len(idx), RECORD_BYTES))
+
+
+def _byte_view(out, count):
+    a = out.numpy() if isinstance(out, torch.Tensor) else out
+    if a.dtype != np.uint8 or a.ndim != 1 or not a.flags.c_contiguous:
+        raise ValueError("out must be a contiguous 1-D uint8 buffer")
+    if a.size < count * RECORD_BYTES:
+        raise ValueError(f"out holds {a.size} bytes, {count} records need {count * RECORD_BYTES}")
+    return a[:count * RECORD_BYTES]
+
+
+class _FeederCfg(C.Structure):
+    _fields_ = [("max_reads", C.c_int32), ("store_max_reads", C.c_int32), ("use_q_scores", C.c_int32), ("use_strands", C.c_int32),
+                ("keep_candidate_af", C.c_int32), ("seed", C.c_uint64)]
+
+
+_SCALARS = (("label", np.uint8), ("num_reads", np.int32), ("is_snp", np.uint8), ("var_type", np.int32), ("allele_freq", np.float32),
+            ("coverage", np.int32), ("var_base_enum", np.int32), ("var_ref_enum", np.int32), ("blacklist", np.uint8), ("status", np.int32))
+
+
+class _RecordBatchC(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("reads", "q_scores", "strands", "ref", "ref_masks", "var_masks")] + [(n, C.c_void_p) for n, _ in _SCALARS]
+
+
+# dan_record_header (include/dan_b200.h): tile column j < num_rows of every tile is stored row rows[j]
+RECORD_HEADER_DTYPE = np.dtype([("window_start", np.int32), ("num_rows", np.int32), ("ref_len", np.int32), ("var_len", np.int32),
+                                ("rows", np.uint8, (200,))])
+assert RECORD_HEADER_DTYPE.itemsize == 216
+
+
+def _feeder_cfg(max_reads, store_max_reads, use_q_scores, use_strands, keep_candidate_af, seed):
+    return _FeederCfg(max_reads, store_max_reads, int(use_q_scores), int(use_strands), int(keep_candidate_af), int(seed))
+
+
+def _record_indices(records, indices):
+    idx = np.ascontiguousarray(np.asarray(indices, dtype=np.int64)).reshape(-1)
+    if len(idx) and (idx.min() < 0 or idx.max() >= len(records)):
+        raise IndexError(f"record index out of range [0, {len(records)})")
+    return idx
+
+
+def _scalars(n):
+    return {k: np.zeros(n, t) for k, t in _SCALARS}
+
+
+def _batch_struct(tiles, sc):
+    ptr = lambda t: None if t is None else t.data_ptr() if isinstance(t, torch.Tensor) else t.ctypes.data
+    return _RecordBatchC(*[ptr(t) for t in tiles], *[sc[k].ctypes.data for k, _ in _SCALARS])
+
+
+def _raise_failed(idx, sc):
+    bad = np.flatnonzero(sc["status"])
+    raise ValueError(f"{len(bad)} records cannot be decoded (the reference loader raises on them): " +
+                     ", ".join(f"#{int(idx[b])}: {REC_STATUS.get(int(sc['status'][b]), '?')}" for b in bad[:5]))
+
 
 def decode_records(records: RecordFile, indices, batch: HostBatch | None = None, use_q_scores=True, use_strands=True, keep_candidate_af=False, seed=0,
                    max_reads=100, store_max_reads=200, strict=True):
     """Decode `indices` of a RecordFile into a (pinned) HostBatch + the per-example scalars the trainer reads (dataset.py:672-680).
     Returns (batch, scalars dict of numpy arrays incl. `status` / `blacklist`). strict: raise if the reference's loader would."""
-    import ctypes as C
-
     from . import _lib
     lib = _lib.load_library()
-
-    class Cfg(C.Structure):
-        _fields_ = [("max_reads", C.c_int32), ("store_max_reads", C.c_int32), ("use_q_scores", C.c_int32), ("use_strands", C.c_int32),
-                    ("keep_candidate_af", C.c_int32), ("seed", C.c_uint64)]
-
-    class Out(C.Structure):
-        _fields_ = [(n, C.c_void_p) for n in ("reads", "q_scores", "strands", "ref", "ref_masks", "var_masks", "label", "num_reads", "is_snp", "var_type",
-                                              "allele_freq", "coverage", "var_base_enum", "var_ref_enum", "blacklist", "status")]
-
-    idx = np.ascontiguousarray(np.asarray(indices, dtype=np.int64))
+    idx = _record_indices(records, indices)
     n = len(idx)
-    if n and (idx.min() < 0 or idx.max() >= len(records)):
-        raise IndexError("record index out of range")
     if batch is None:
         batch = HostBatch(max(n, 1), num_reads=max_reads)
     if n > batch.capacity:
         raise ValueError(f"{n} records > capacity {batch.capacity}")
-    sc = {"label": np.zeros(n, np.uint8), "num_reads": np.zeros(n, np.int32), "is_snp": np.zeros(n, np.uint8), "var_type": np.zeros(n, np.int32),
-          "allele_freq": np.zeros(n, np.float32), "coverage": np.zeros(n, np.int32), "var_base_enum": np.zeros(n, np.int32),
-          "var_ref_enum": np.zeros(n, np.int32), "blacklist": np.zeros(n, np.uint8), "status": np.zeros(n, np.int32)}
-    out = Out(batch.reads.data_ptr(), batch.q.data_ptr(), batch.strands.data_ptr(), batch.ref.data_ptr(), batch.ref_masks.data_ptr(),
-              batch.var_masks.data_ptr(), *[sc[k].ctypes.data for k in ("label", "num_reads", "is_snp", "var_type", "allele_freq", "coverage",
-                                                                         "var_base_enum", "var_ref_enum", "blacklist", "status")])
-    cfg = Cfg(max_reads, store_max_reads, int(use_q_scores), int(use_strands), int(keep_candidate_af), int(seed))
-    lib.dan_decode_records.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(Cfg), C.POINTER(Out)]
+    sc = _scalars(n)
+    out = _batch_struct((batch.reads, batch.q, batch.strands, batch.ref, batch.ref_masks, batch.var_masks), sc)
+    cfg = _feeder_cfg(max_reads, store_max_reads, use_q_scores, use_strands, keep_candidate_af, seed)
+    lib.dan_decode_records.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(_FeederCfg), C.POINTER(_RecordBatchC)]
     rc = lib.dan_decode_records(records.raw.ctypes.data, RECORD_BYTES, idx.ctypes.data, n, C.byref(cfg), C.byref(out))
     batch.size = n
     batch.meta = [(bytes(records.field(int(i), "name")).decode(), bytes(records.field(int(i), "vcfrec")).decode()) for i in idx]
     if rc < 0 and strict:
-        bad = np.flatnonzero(sc["status"])
-        raise ValueError(f"{len(bad)} records cannot be decoded (the reference loader raises on them): " +
-                         ", ".join(f"#{int(idx[b])}: {REC_STATUS.get(int(sc['status'][b]), '?')}" for b in bad[:5]))
+        _raise_failed(idx, sc)
     return batch, sc
+
+
+def decode_record_headers(records: RecordFile, indices, use_q_scores=True, use_strands=True, keep_candidate_af=False, seed=0, max_reads=100,
+                          store_max_reads=200):
+    """The header pass of the decode alone (`dan_decode_record_headers`, host code): -> (headers, scalars, ref_masks, var_masks).
+    headers is a RECORD_HEADER_DTYPE array; scalars and masks are what decode_records returns for the same arguments."""
+    from . import _lib
+    lib = _lib.load_library()
+    idx = _record_indices(records, indices)
+    n = len(idx)
+    sc = _scalars(n)
+    rm, vm = np.zeros((n, 201), np.uint8), np.zeros((n, 201), np.uint8)
+    hdr = np.zeros(n, RECORD_HEADER_DTYPE)
+    out = _batch_struct((None, None, None, None, rm, vm), sc)
+    cfg = _feeder_cfg(max_reads, store_max_reads, use_q_scores, use_strands, keep_candidate_af, seed)
+    lib.dan_decode_record_headers.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(_FeederCfg), C.POINTER(_RecordBatchC), C.c_void_p]
+    rc = lib.dan_decode_record_headers(records.raw.ctypes.data, RECORD_BYTES, idx.ctypes.data, n, C.byref(cfg), C.byref(out), hdr.ctypes.data)
+    if rc < 0 and not sc["status"].any():
+        _lib.check(rc, "dan_decode_record_headers")
+    return hdr, sc, rm, vm
+
+
+def _staging_bytes(n, max_reads):
+    from . import _lib
+    lib = _lib.load_library()
+    lib.dan_decode_records_device_workspace_bytes.argtypes = [C.c_int, C.POINTER(_FeederCfg)]
+    lib.dan_decode_records_device_workspace_bytes.restype = C.c_size_t
+    cfg = _feeder_cfg(max_reads, 200, 1, 1, 0, 0)
+    need = int(lib.dan_decode_records_device_workspace_bytes(n, C.byref(cfg)))
+    if need == 0 and n > 0:
+        raise ValueError(f"max_reads {max_reads} out of range 1..200")
+    return need
+
+
+class DeviceBatch:
+    """Decoded batch on the GPU (`dan_decode_records_device`): device uint8 tiles in the layout dan_forward takes, the pinned host
+    staging buffer the raw records are read into, and the device workspace they are copied to. The decoded tiles exist only on
+    the device."""
+
+    def __init__(self, capacity: int, num_reads: int = 100, device=None, read_len: int = 201):
+        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        self.capacity, self.num_reads, self.device, self.size = capacity, num_reads, dev, 0
+        nbytes = _staging_bytes(capacity, num_reads)
+        self.staging = torch.empty(nbytes, dtype=torch.uint8).pin_memory()
+        self.workspace = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        mk = lambda *shape: torch.empty(shape, dtype=torch.uint8, device=dev)
+        self.reads, self.q, self.strands = (mk(capacity, read_len, num_reads) for _ in range(3))
+        self.ref, self.ref_masks, self.var_masks = (mk(capacity, read_len) for _ in range(3))
+        self.meta = []
+
+    def tensors(self):
+        n = self.size
+        return self.reads[:n], self.ref[:n], self.q[:n], self.strands[:n], self.ref_masks[:n], self.var_masks[:n]
+
+    def headers(self):
+        """Header-pass descriptors of the last decode (RECORD_HEADER_DTYPE, a view into the staging buffer)."""
+        n = self.size
+        off = (n * RECORD_BYTES + 15) & ~15
+        return self.staging.numpy()[off:off + n * RECORD_HEADER_DTYPE.itemsize].view(RECORD_HEADER_DTYPE)
+
+
+def decode_records_device(records: RecordFile, indices, batch: DeviceBatch | None = None, use_q_scores=True, use_strands=True,
+                          keep_candidate_af=False, seed=0, max_reads=100, store_max_reads=200, strict=True, stream=None):
+    """decode_records with the tile pass on the GPU (`dan_decode_records_device`). The records go into the batch's pinned staging
+    buffer (one memcpy from the file for a contiguous ascending range, an index gather otherwise), the header pass runs on the host,
+    then one H2D copy and the tile kernel run on `stream` (default: the current stream). Returns (batch, scalars) with the same
+    outputs as decode_records, byte for byte. Asynchronous: the batch's tensors are ready once `stream` has passed the call, and
+    the batch may be decoded into again only after that."""
+    from . import _lib
+    lib = _lib.load_library()
+    idx = _record_indices(records, indices)
+    n = len(idx)
+    if batch is None:
+        batch = DeviceBatch(max(n, 1), num_reads=max_reads)
+    if n > batch.capacity:
+        raise ValueError(f"{n} records > capacity {batch.capacity}")
+    if batch.num_reads != max_reads:
+        raise ValueError(f"batch holds {batch.num_reads} reads per candidate, max_reads is {max_reads}")
+    if n and np.all(np.diff(idx) == 1):
+        records.read_block(int(idx[0]), n, batch.staging)
+    else:
+        records.gather(idx, batch.staging)
+    sc = _scalars(n)
+    out = _batch_struct((batch.reads, batch.q, batch.strands, batch.ref, batch.ref_masks, batch.var_masks), sc)
+    cfg = _feeder_cfg(max_reads, store_max_reads, use_q_scores, use_strands, keep_candidate_af, seed)
+    lib.dan_decode_records_device.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(_FeederCfg), C.POINTER(_RecordBatchC),
+                                              C.c_void_p, C.c_size_t, C.c_void_p]
+    with torch.cuda.device(batch.device):
+        st = (stream if stream is not None else torch.cuda.current_stream(batch.device)).cuda_stream
+        rc = lib.dan_decode_records_device(batch.staging.data_ptr(), batch.staging.numel(), idx.ctypes.data, n, C.byref(cfg), C.byref(out),
+                                           batch.workspace.data_ptr(), batch.workspace.numel(), st)
+    batch.size = n
+    raw = batch.staging.numpy()[:n * RECORD_BYTES].reshape(n, RECORD_BYTES)
+    names = raw[:, :16].copy().view("S16").reshape(-1)
+    vcfrecs = raw[:, _VCF_OFFSET:_VCF_OFFSET + 128].copy().view("S128").reshape(-1)
+    batch.meta = [(a.decode(), b.decode()) for a, b in zip(names.tolist(), vcfrecs.tolist())]
+    if rc == -1 and sc["status"].any():          # DAN_E_INVALID with per-record status: records the reference raises on
+        if strict:
+            _raise_failed(idx, sc)
+    else:
+        _lib.check(rc, "dan_decode_records_device")
+    return batch, sc
+
+
+_VCF_OFFSET = RECORD_DTYPE.fields["vcfrec"][1]
+
+
+class _CallSlot:
+    """One ring slot of call_record_file: a DeviceBatch plus the pinned buffers of its allele lengths and results."""
+
+    def __init__(self, capacity, num_reads, dev):
+        self.batch = DeviceBatch(capacity, num_reads, dev)
+        pin = lambda shape, dt: torch.empty(shape, dtype=dt).pin_memory()
+        self.ref_len, self.var_len = pin(capacity, torch.int32), pin(capacity, torch.int32)
+        self.scores, self.gt, self.q = pin((capacity, 4), torch.float32), pin(capacity, torch.int8), pin(capacity, torch.int32)
+
+
+def call_record_file(model, records, start=0, stop=None, batch_size=1036, depth=2, thresholds=None, strict=True, failed=None, seed=0,
+                     store_max_reads=200, keep_candidate_af=False):
+    """Stream records [start, stop) of a record file (path or RecordFile) to scored VCF records and genotype calls: the whole path of
+    the reference's inference (main.py --test_file -> trainer.test -> append_vcf_records -> tools/format_vcf.py's thresholds) in one call.
+
+    Yields, per batch of up to `batch_size` records in file order, (names, vcf_lines, gt, q): record names, the VCF records with the
+    score field spliced in (exactly what splice_vcf_records writes), and the genotype calls of genotype_calls_on_device (gt int8 numpy:
+    0 dropped, 1 "0/1", 2 "1/1"; q int32 numpy). `thresholds` are genotype_calls' keyword arguments.
+
+    Per batch: the records are read into a pinned ring slot (one memcpy), the header pass runs on the host, and the H2D copy and the
+    device tile pass run on a side stream; forward_heads, dan_scores and dan_genotype_calls follow on the current stream, and only
+    scores (16 bytes) and gt / q per record come back. `depth` slots rotate, so the host work of batch k+1 overlaps the GPU work of
+    batch k; a slot is reused only after its batch's results have been yielded.
+    Records the reference's loader raises on (status != 0): strict=True raises naming them; strict=False leaves them out and appends
+    (record index, status) to `failed` when a list is given."""
+    import os
+    rf = records if isinstance(records, RecordFile) else RecordFile(os.fspath(records))
+    stop = len(rf) if stop is None else int(stop)
+    start = int(start)
+    if not 0 <= start <= stop <= len(rf):
+        raise IndexError(f"record range [{start}, {stop}) outside the file's {len(rf)}")
+    if batch_size < 1 or depth < 1:
+        raise ValueError("batch_size and depth must be >= 1")
+    if model.training:
+        raise RuntimeError("call_record_file runs the eval-mode forward: call .eval() first")
+    dev = model._device()
+    thr = dict(thresholds or {})
+    opts = dict(use_q_scores=model.use_q_scores, use_strands=model.use_strands, keep_candidate_af=keep_candidate_af, seed=seed,
+                max_reads=model.num_single_reads, store_max_reads=store_max_reads)
+    with torch.cuda.device(dev):
+        main, side = torch.cuda.current_stream(dev), torch.cuda.Stream(dev)
+        free = deque(_CallSlot(min(batch_size, max(stop - start, 1)), model.num_single_reads, dev) for _ in range(depth))
+        side.wait_stream(main)          # the slots' device memory may be blocks the current stream freed with work still queued on them
+        pending = deque()
+
+        def submit(b0, n):
+            slot = free.popleft()
+            idx = np.arange(b0, b0 + n, dtype=np.int64)
+            batch, sc = decode_records_device(rf, idx, slot.batch, strict=False, stream=side, **opts)
+            bad = np.flatnonzero(sc["status"])
+            if strict and len(bad):
+                side.synchronize()      # the copy and tile pass just queued still use the slot
+                free.append(slot)
+                _raise_failed(idx, sc)
+            hdr = batch.headers()
+            slot.ref_len[:n].numpy()[:] = hdr["ref_len"]
+            slot.var_len[:n].numpy()[:] = hdr["var_len"]
+            main.wait_stream(side)
+            with torch.cuda.stream(main):
+                heads = model.forward_heads(*batch.tensors())
+                scores = scores_on_device(heads)
+                rl, vl = slot.ref_len[:n].to(dev, non_blocking=True), slot.var_len[:n].to(dev, non_blocking=True)
+                gt, q = genotype_calls_on_device(scores, rl, vl, **thr)
+                slot.scores[:n].copy_(scores, non_blocking=True)
+                slot.gt[:n].copy_(gt, non_blocking=True)
+                slot.q[:n].copy_(q, non_blocking=True)
+                ev = torch.cuda.Event()
+                ev.record(main)
+            pending.append((slot, idx, sc["status"].copy(), batch.meta, ev))
+
+        def finish():
+            slot, idx, status, meta, ev = pending.popleft()
+            ev.synchronize()
+            n = len(idx)
+            good = status == 0
+            if failed is not None:
+                failed.extend((int(idx[b]), int(status[b])) for b in np.flatnonzero(~good))
+            keep = np.flatnonzero(good)
+            scores = slot.scores[:n].numpy()[keep]
+            names = [meta[k][0] for k in keep]
+            lines = _splice_info([meta[k][1] for k in keep], format_vcf_info_native(scores))
+            out = (names, lines, slot.gt[:n].numpy()[keep].copy(), slot.q[:n].numpy()[keep].copy())
+            free.append(slot)
+            return out
+
+        try:
+            for b0 in range(start, stop, batch_size):
+                if not free:
+                    yield finish()
+                submit(b0, min(batch_size, stop - b0))
+            while pending:
+                yield finish()
+        finally:
+            # on an exception or an abandoned generator the slots are freed here: let the device work that uses them finish first
+            # (the raw staging copies are invisible to torch's allocators)
+            side.synchronize()
+            for *_, ev in pending:
+                ev.synchronize()

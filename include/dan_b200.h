@@ -260,6 +260,36 @@ typedef struct dan_record_batch {
 int dan_decode_records(const void* records, size_t record_stride, const int64_t* indices, int n, const dan_feeder_config* cfg,
                        const dan_record_batch* out);
 
+/* The decode in two passes. The header pass (host) does everything that is not tile bytes: row window and read sampling, VCF parse,
+ * allele counts at the proposal column over the chosen rows, coverage / allele frequency, proposal masks, blacklist and status. The
+ * tile pass gathers the chosen stored rows of single_reads / q-scores / strand into the [position][read] tiles. dan_decode_records
+ * runs both on the host; dan_decode_records_device runs the tile pass on the device.
+ * One header per record: tile column j (j < num_rows) is stored row rows[j] of the record; columns from num_rows on are zero.
+ * ref_len / var_len are the lengths of the VCF record's REF / ALT columns (0 if it has too few columns). */
+typedef struct dan_record_header {
+  int32_t window_start;       /* first stored row of the window (dataset.py:517-521) */
+  int32_t num_rows;           /* chosen rows = tile columns holding a read, <= max_reads */
+  int32_t ref_len, var_len;
+  uint8_t rows[200];          /* stored-row indices of tile columns 0 .. num_rows-1, ascending */
+} dan_record_header;
+
+/* Header pass alone (pure host code): same arguments as dan_decode_records; fills headers[n], the masks and the scalars of `out`
+ * (its tile and ref pointers are not used). Returns DAN_E_INVALID if any record failed. */
+int dan_decode_record_headers(const void* records, size_t record_stride, const int64_t* indices, int n, const dan_feeder_config* cfg,
+                              const dan_record_batch* out, dan_record_header* headers);
+
+/* Device decode. `staging` is a pinned HOST buffer of dan_decode_records_device_workspace_bytes(n, cfg) bytes whose first
+ * n * DAN_RECORD_BYTES bytes hold the n records back to back, record i decoding into candidate i; indices[i] is record i's index in its
+ * file, which seeds the read draw exactly as in dan_decode_records. The call runs the header pass on the host, writing the headers and
+ * masks into the rest of `staging` and the scalars of `out` (HOST pointers: label .. status, each may be NULL, valid on return), copies
+ * the staging buffer to `workspace` (DEVICE, same size) in one cudaMemcpyAsync on `stream` and launches the tile pass there, which
+ * writes out->reads / q_scores / strands / ref / ref_masks / var_masks (DEVICE pointers; q_scores / strands may be NULL). Every output
+ * equals dan_decode_records' byte for byte. Asynchronous: neither buffer may be reused before the stream has passed this call.
+ * DAN_E_WORKSPACE (no copy, no launch) if either buffer is too small; DAN_E_INVALID with per-record status as dan_decode_records. */
+size_t dan_decode_records_device_workspace_bytes(int n, const dan_feeder_config* cfg);
+int dan_decode_records_device(void* staging, size_t staging_bytes, const int64_t* indices, int n, const dan_feeder_config* cfg,
+                              const dan_record_batch* out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Test hook for the bit-exact integer/encoding work (dl4vc/model.py:450-627,719): writes the conv-1 input in the
  * reference's logical order (batch, Cin, num_reads, read_len) fp32, DEVICE pointer. */
 int dan_encode(dan_model* m, const uint8_t* reads, const uint8_t* q_scores, const uint8_t* strands,
