@@ -97,10 +97,29 @@ int parse_vcf_record(const std::string& rec_in, VcfInfo* out, std::string* ref_a
 // Row window + sample_single_reads selection, parse_vcf, allele counts at the proposal column over the chosen rows, coverage /
 // allele_freq, proposal masks, blacklist and status. Writes the scalars of record i into `out` (each may be NULL), the masks into
 // rm / vm, and the chosen stored rows into *h. `key` seeds the draw of deep pileups (the record's index in its file).
-int header_pass(const uint8_t* rec, int64_t key, const dan_feeder_config* cfg, int R, int S, const dan_record_batch* out, int i,
+// The pass reads its record through a HeaderView: the scalar fields, ref_bases, and single_reads columns 100 and 101 of the stored rows.
+
+// sidecar layout (include/dan_b200.h): the bytes a HeaderView reads, plus the name
+constexpr size_t kSideName = 0, kSideNumReads = 16, kSideLabel = 20, kSideVcf = 21, kSideRef = kSideVcf + 128, kSideCol100 = kSideRef + kRecP,
+                 kSideCol101 = kSideCol100 + kRecRows, kSideBytes = kSideCol101 + kRecRows;
+static_assert(kSideBytes == DAN_SIDECAR_BYTES, "sidecar layout");
+
+struct HeaderView {
+  const uint8_t *num_reads, *label, *vcf, *ref;
+  const uint8_t* col[2];                      // single_reads columns 100 and 101: stored row r at col[c][r * row_stride]
+  size_t row_stride;
+};
+HeaderView raw_view(const uint8_t* rec) {
+  return {rec + kOffNumReads, rec + kOffLabel, rec + kOffVcf, rec + kOffRefBases, {rec + kOffSingle + 100, rec + kOffSingle + 101}, (size_t)kRecP};
+}
+HeaderView sidecar_view(const uint8_t* sc) {
+  return {sc + kSideNumReads, sc + kSideLabel, sc + kSideVcf, sc + kSideRef, {sc + kSideCol100, sc + kSideCol101}, 1};
+}
+
+int header_pass(const HeaderView& rec, int64_t key, const dan_feeder_config* cfg, int R, int S, const dan_record_batch* out, int i,
                 uint8_t* rm, uint8_t* vm, dan_record_header* h) {
   int32_t num_reads;
-  memcpy(&num_reads, rec + kOffNumReads, 4);
+  memcpy(&num_reads, rec.num_reads, 4);
   // A. window of stored rows (dataset.py:517-521), B. at most R of them (sample_single_reads, dataset.py:256-287)
   const int middle = (num_reads > S ? num_reads : S) / 2;
   int start = (int)((double)middle - (double)S / 2.0);
@@ -126,13 +145,13 @@ int header_pass(const uint8_t* rec, int64_t key, const dan_feeder_config* cfg, i
   h->window_start = start;
   h->num_rows = max_reads;
   for (int j = 0; j < max_reads; ++j) h->rows[j] = (uint8_t)(start + perm[j]);      // start + perm[j] < start + avail <= kRecRows
-  const uint8_t* ref = rec + kOffRefBases;
-  if (out->label) out->label[i] = rec[kOffLabel];
+  const uint8_t* ref = rec.ref;
+  if (out->label) out->label[i] = *rec.label;
   if (out->num_reads) out->num_reads[i] = num_reads;
   // vcfrec: S128, trailing NULs stripped like numpy does
   size_t len = 128;
-  while (len > 0 && rec[kOffVcf + len - 1] == 0) --len;
-  const std::string vcf(reinterpret_cast<const char*>(rec + kOffVcf), len);
+  while (len > 0 && rec.vcf[len - 1] == 0) --len;
+  const std::string vcf(reinterpret_cast<const char*>(rec.vcf), len);
   VcfInfo vi{};
   std::string xa, ya;
   int status = parse_vcf_record(vcf, &vi, &xa, &ya);
@@ -149,7 +168,7 @@ int header_pass(const uint8_t* rec, int64_t key, const dan_feeder_config* cfg, i
     else { ref_base = 8; col = 101; }
     int agree = 0, disagree = 0;
     for (int j = 0; j < max_reads; ++j) {
-      const int t = rec[kOffSingle + (size_t)h->rows[j] * kRecP + col];
+      const int t = rec.col[col - 100][(size_t)h->rows[j] * rec.row_stride];
       if (t == ref_base) ++agree;
       else if (t == 1 || t == 2 || t == 3 || t == 4 || t == 5 || t == 8 || t == 9) ++disagree;      // real_base_keys_set: A T C G - M noinsert
     }
@@ -268,6 +287,31 @@ __global__ void decode_tiles_kernel(const uint8_t* __restrict__ ws, int n, int R
   }
 }
 
+// ---- compressed records ------------------------------------------------------------------------------------------------------------
+// Staging layout for n records (include/dan_b200.h). The device workspace holds [n record images][pad to 16] followed by the staging
+// buffer from `off` on, so every offset past `off` keeps its 16-byte alignment.
+struct CompressedLayout { size_t side, off, len, hdr, rm, vm, data; };
+CompressedLayout compressed_layout(int n) {
+  CompressedLayout l;
+  l.side = 0;
+  l.off = ((size_t)n * kSideBytes + 15) & ~(size_t)15;
+  l.len = l.off + (size_t)n * 8;
+  l.hdr = (l.len + (size_t)n * 4 + 15) & ~(size_t)15;
+  l.rm = l.hdr + (size_t)n * sizeof(dan_record_header);
+  l.vm = l.rm + (size_t)n * kRecP;
+  l.data = (l.vm + (size_t)n * kRecP + 15) & ~(size_t)15;
+  return l;
+}
+size_t images_bytes(int n) { return ((size_t)n * kRecBytes + 15) & ~(size_t)15; }
+
+// a record whose stream failed decodes to nothing: no tile rows (its image is already all zero) and all-zero masks
+__global__ void clear_failed_kernel(uint8_t* ws, int n, size_t hdr_off, size_t rm_off, size_t vm_off, const int32_t* __restrict__ inflate_status) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n || inflate_status[i] == DAN_INFLATE_OK) return;
+  reinterpret_cast<dan_record_header*>(ws + hdr_off)[i].num_rows = 0;
+  for (int k = 0; k < kRecP; ++k) { ws[rm_off + (size_t)i * kRecP + k] = 0; ws[vm_off + (size_t)i * kRecP + k] = 0; }
+}
+
 }  // namespace
 
 extern "C" {
@@ -283,7 +327,7 @@ int dan_decode_records(const void* records, size_t record_stride, const int64_t*
   for (int i = 0; i < n; ++i) {
     const uint8_t* rec = static_cast<const uint8_t*>(records) + (size_t)indices[i] * record_stride;
     dan_record_header h;
-    if (header_pass(rec, indices[i], cfg, R, S, out, i, out->ref_masks + (size_t)i * kRecP, out->var_masks + (size_t)i * kRecP, &h) != DAN_REC_OK) ++failed;
+    if (header_pass(raw_view(rec), indices[i], cfg, R, S, out, i, out->ref_masks + (size_t)i * kRecP, out->var_masks + (size_t)i * kRecP, &h) != DAN_REC_OK) ++failed;
     host_tiles(rec, h, cfg, R, out, i);
   }
   if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
@@ -301,7 +345,7 @@ int dan_decode_record_headers(const void* records, size_t record_stride, const i
   int failed = 0;
   for (int i = 0; i < n; ++i) {
     const uint8_t* rec = static_cast<const uint8_t*>(records) + (size_t)indices[i] * record_stride;
-    if (header_pass(rec, indices[i], cfg, R, S, out, i, out->ref_masks + (size_t)i * kRecP, out->var_masks + (size_t)i * kRecP, headers + i) != DAN_REC_OK) ++failed;
+    if (header_pass(raw_view(rec), indices[i], cfg, R, S, out, i, out->ref_masks + (size_t)i * kRecP, out->var_masks + (size_t)i * kRecP, headers + i) != DAN_REC_OK) ++failed;
   }
   if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
   return DAN_OK;
@@ -327,12 +371,108 @@ int dan_decode_records_device(void* staging, size_t staging_bytes, const int64_t
   dan_record_header* hdr = reinterpret_cast<dan_record_header*>(st + l.hdr);
   int failed = 0;
   for (int i = 0; i < n; ++i)
-    if (header_pass(st + (size_t)i * kRecBytes, indices[i], cfg, R, S, out, i, st + l.rm + (size_t)i * kRecP, st + l.vm + (size_t)i * kRecP, hdr + i) != DAN_REC_OK) ++failed;
+    if (header_pass(raw_view(st + (size_t)i * kRecBytes), indices[i], cfg, R, S, out, i, st + l.rm + (size_t)i * kRecP, st + l.vm + (size_t)i * kRecP, hdr + i) != DAN_REC_OK) ++failed;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   DAN_CUDA_TRY(cudaMemcpyAsync(workspace, staging, l.total, cudaMemcpyHostToDevice, s));
   const int smem = ((kRecP * R + 31) / 16) * 16;
   decode_tiles_kernel<<<dim3(n, 3), kTileThreads, smem, s>>>(static_cast<const uint8_t*>(workspace), n, R, cfg->use_q_scores != 0, cfg->use_strands != 0,
                                                              l.hdr, l.rm, l.vm, out->reads, out->q_scores, out->strands, out->ref, out->ref_masks, out->var_masks);
+  DAN_CUDA_TRY(cudaGetLastError());
+  if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
+  return DAN_OK;
+}
+
+int dan_record_sidecars(const void* records, size_t record_stride, int n, void* out) {
+  if (n < 0) { dan_set_error("negative record count"); return DAN_E_INVALID; }
+  if (n == 0) return DAN_OK;
+  if (!records || !out) { dan_set_error("null pointer"); return DAN_E_INVALID; }
+  if (record_stride < DAN_RECORD_BYTES) { dan_set_error("record stride %zu below the %d-byte record", record_stride, DAN_RECORD_BYTES); return DAN_E_INVALID; }
+  for (int i = 0; i < n; ++i) {
+    const uint8_t* rec = static_cast<const uint8_t*>(records) + (size_t)i * record_stride;
+    uint8_t* sc = static_cast<uint8_t*>(out) + (size_t)i * kSideBytes;
+    memcpy(sc + kSideName, rec + kOffName, 16);
+    memcpy(sc + kSideNumReads, rec + kOffNumReads, 4);
+    sc[kSideLabel] = rec[kOffLabel];
+    memcpy(sc + kSideVcf, rec + kOffVcf, 128);
+    memcpy(sc + kSideRef, rec + kOffRefBases, kRecP);
+    for (int r = 0; r < kRecRows; ++r) {
+      sc[kSideCol100 + r] = rec[kOffSingle + (size_t)r * kRecP + 100];
+      sc[kSideCol101 + r] = rec[kOffSingle + (size_t)r * kRecP + 101];
+    }
+  }
+  return DAN_OK;
+}
+
+int dan_decode_sidecar_headers(const void* sidecars, const int64_t* indices, int n, const dan_feeder_config* cfg, const dan_record_batch* out,
+                               dan_record_header* headers) {
+  if (n < 0) { dan_set_error("negative record count"); return DAN_E_INVALID; }
+  if (n == 0) return DAN_OK;
+  if (!sidecars || !indices || !cfg || !out || !out->ref_masks || !out->var_masks || !headers) { dan_set_error("null pointer"); return DAN_E_INVALID; }
+  int R, S;
+  if (check_feeder_config(cfg, &R, &S) != DAN_OK) return DAN_E_INVALID;
+  int failed = 0;
+  for (int i = 0; i < n; ++i) {
+    const uint8_t* sc = static_cast<const uint8_t*>(sidecars) + (size_t)indices[i] * kSideBytes;
+    if (header_pass(sidecar_view(sc), indices[i], cfg, R, S, out, i, out->ref_masks + (size_t)i * kRecP, out->var_masks + (size_t)i * kRecP, headers + i) != DAN_REC_OK) ++failed;
+  }
+  if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
+  return DAN_OK;
+}
+
+size_t dan_decode_compressed_records_device_staging_bytes(int n, size_t max_stream_bytes) {
+  if (n < 0) return 0;
+  return (compressed_layout(n).data + (size_t)n * max_stream_bytes + 15) & ~(size_t)15;
+}
+
+size_t dan_decode_compressed_records_device_workspace_bytes(int n, size_t max_stream_bytes) {
+  if (n < 0) return 0;
+  return images_bytes(n) + dan_decode_compressed_records_device_staging_bytes(n, max_stream_bytes) - compressed_layout(n).off;
+}
+
+int dan_decode_compressed_records_device(void* staging, size_t staging_bytes, const int64_t* indices, int n, const dan_feeder_config* cfg,
+                                         const dan_record_batch* out, void* workspace, size_t workspace_bytes, int32_t* inflate_status,
+                                         void* stream) {
+  if (n < 0) { dan_set_error("negative record count"); return DAN_E_INVALID; }
+  if (n == 0) return DAN_OK;
+  if (!staging || !indices || !cfg || !out || !out->reads || !out->ref || !out->ref_masks || !out->var_masks || !workspace || !inflate_status) {
+    dan_set_error("null pointer"); return DAN_E_INVALID;
+  }
+  int R, S;
+  if (check_feeder_config(cfg, &R, &S) != DAN_OK) return DAN_E_INVALID;
+  const CompressedLayout l = compressed_layout(n);
+  if (staging_bytes < l.data) { dan_set_error("staging buffer of %zu bytes is below the %zu bytes %d records need", staging_bytes, l.data, n); return DAN_E_WORKSPACE; }
+  uint8_t* st = static_cast<uint8_t*>(staging);
+  const uint64_t* off = reinterpret_cast<const uint64_t*>(st + l.off);
+  const uint32_t* len = reinterpret_cast<const uint32_t*>(st + l.len);
+  const size_t cap = staging_bytes - l.data;
+  size_t used = 0;
+  for (int i = 0; i < n; ++i) {
+    if (off[i] > cap || len[i] > cap - off[i]) {
+      dan_set_error("stream %d ([%llu, +%u)) leaves the %zu-byte streams region of the staging buffer", i, (unsigned long long)off[i], len[i], cap);
+      return DAN_E_INVALID;
+    }
+    if (off[i] + len[i] > used) used = off[i] + len[i];
+  }
+  const size_t copy = l.data - l.off + used, images = images_bytes(n);
+  if (workspace_bytes < images + copy) { dan_set_error("device workspace of %zu bytes is below the %zu bytes %d records need", workspace_bytes, images + copy, n); return DAN_E_WORKSPACE; }
+  dan_record_header* hdr = reinterpret_cast<dan_record_header*>(st + l.hdr);
+  int failed = 0;
+  for (int i = 0; i < n; ++i)
+    if (header_pass(sidecar_view(st + l.side + (size_t)i * kSideBytes), indices[i], cfg, R, S, out, i, st + l.rm + (size_t)i * kRecP,
+                    st + l.vm + (size_t)i * kRecP, hdr + i) != DAN_REC_OK) ++failed;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  const size_t base = images - l.off;                 // workspace offset of staging byte b (b >= l.off) is base + b
+  DAN_CUDA_TRY(cudaMemcpyAsync(ws + images, st + l.off, copy, cudaMemcpyHostToDevice, s));
+  const int rc = dan_inflate_launch(ws + base + l.data, reinterpret_cast<const uint64_t*>(ws + base + l.off),
+                                    reinterpret_cast<const uint32_t*>(ws + base + l.len), n, ws, kRecBytes, inflate_status, s);
+  if (rc != DAN_OK) return rc;
+  clear_failed_kernel<<<(n + 127) / 128, 128, 0, s>>>(ws, n, base + l.hdr, base + l.rm, base + l.vm, inflate_status);
+  DAN_CUDA_TRY(cudaGetLastError());
+  const int smem = ((kRecP * R + 31) / 16) * 16;
+  decode_tiles_kernel<<<dim3(n, 3), kTileThreads, smem, s>>>(ws, n, R, cfg->use_q_scores != 0, cfg->use_strands != 0, base + l.hdr, base + l.rm,
+                                                             base + l.vm, out->reads, out->q_scores, out->strands, out->ref, out->ref_masks,
+                                                             out->var_masks);
   DAN_CUDA_TRY(cudaGetLastError());
   if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
   return DAN_OK;

@@ -15,6 +15,9 @@ static inline int round_up_i(int x, int m) { return (x + m - 1) / m * m; }
 static inline size_t round_up_z(size_t x, size_t m) { return (x + m - 1) / m * m; }
 
 void dan_set_error(const char* fmt, ...);
+// dan_inflate.cu: the launch behind dan_inflate_device, for callers that have checked their arguments (no argument checks)
+int dan_inflate_launch(const uint8_t* src, const uint64_t* offsets, const uint32_t* lengths, int n, uint8_t* dst, uint64_t slot_bytes,
+                       int32_t* status, cudaStream_t stream);
 void dan_count_launch(int n = 1);
 // kernel-class timing spans (no-ops unless dan_profile_enable(1)); classes: DAN_PROF_*
 void dan_prof_begin(int cls, cudaStream_t st);

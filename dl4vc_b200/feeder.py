@@ -13,12 +13,16 @@ RecordFile / decode_records  raw fixed-record pileup file (the reference's HDF5 
                    parse_vcf, count_variants_from_single_reads, proposal masks) straight into a pinned HostBatch — no per-item Python.
 decode_records_device  the same decode with the tile pass on the GPU (`dan_decode_records_device`): host header pass (parse, sampling,
                    masks), one H2D copy of the staged raw records, a kernel that writes the device tiles `dan_forward` reads.
+CompressedRecordFile  the same records as one zlib stream each, with an index and per-record sidecars (the bytes the header pass
+                   reads); write_compressed_records writes one, decode_records_device inflates the records on the GPU (`dan_inflate_device`).
 call_record_file   record file -> scored VCF lines and genotype calls, streamed in batches through a ring of pinned slots.
 format_vcf_info    the `BP=..;NV=..;HV=..;OV=..` field `utils.append_vcf_records` splices into VCF column 3 (`utils.py:162-178`).
 """
 from __future__ import annotations
 
 import ctypes as C
+import os
+import zlib
 from collections import deque
 
 import numpy as np
@@ -251,7 +255,12 @@ RECORD_DTYPE = np.dtype([("name", "S16"), ("ref", np.uint8, (5, 201)), ("reads",
 RECORD_BYTES = 123965
 assert RECORD_DTYPE.itemsize == RECORD_BYTES
 REC_STATUS = {0: "ok", 1: "vcf record has too few columns", 2: "allele letter outside base_enum", 3: "unknown mutation (equal-length non-SNP)",
-              4: "INFO column without AF= / DP=", 5: "proposal masks: the reference raises (not an assertion)"}
+              4: "INFO column without AF= / DP=", 5: "proposal masks: the reference raises (not an assertion)",
+              6: "compressed record is corrupt"}
+REC_CORRUPT = 6
+# dan_inflate_device's per-stream status (DAN_INFLATE_*)
+INFLATE_STATUS = {0: "ok", 1: "bad zlib header", 2: "bad block type", 3: "bad code set", 4: "distance too far back", 5: "input exhausted",
+                  6: "output longer than its slot", 7: "output shorter than its slot", 8: "Adler-32 mismatch"}
 
 
 class RecordFile:
@@ -295,6 +304,192 @@ def _byte_view(out, count):
     if a.size < count * RECORD_BYTES:
         raise ValueError(f"out holds {a.size} bytes, {count} records need {count * RECORD_BYTES}")
     return a[:count * RECORD_BYTES]
+
+
+# ---- compressed record files (layout: include/dan_b200.h) ----------------------------------------------------------------------------
+COMPRESSED_MAGIC = b"DL4VCZR1"
+SIDECAR_BYTES = 750
+_CZ_HEADER = np.dtype([("magic", "S8"), ("version", "<u4"), ("record_bytes", "<u4"), ("count", "<u8"), ("index_off", "<u8"),
+                       ("sidecar_off", "<u8"), ("data_off", "<u8"), ("data_bytes", "<u8"), ("sidecar_bytes", "<u4"), ("reserved", "<u4")])
+_CZ_INDEX = np.dtype([("offset", "<u8"), ("length", "<u4")])
+assert _CZ_HEADER.itemsize == 64 and _CZ_INDEX.itemsize == 12
+# the sidecar as dan_record_sidecars cuts it (include/dan_b200.h); col100 / col101: single_reads columns 100 / 101 of the 200 stored rows
+SIDECAR_DTYPE = np.dtype([("name", "S16"), ("num_reads", "<i4"), ("label", "u1"), ("vcfrec", "S128"), ("ref_bases", "u1", (201,)),
+                          ("col100", "u1", (200,)), ("col101", "u1", (200,))])
+assert SIDECAR_DTYPE.itemsize == SIDECAR_BYTES
+
+
+def record_sidecars(raw) -> np.ndarray:
+    """(n, RECORD_BYTES) uint8 records -> (n, SIDECAR_BYTES) sidecars, cut by the library (`dan_record_sidecars`), which alone knows
+    which bytes the header pass reads."""
+    from . import _lib
+    raw = np.ascontiguousarray(raw)
+    out = np.empty((len(raw), SIDECAR_BYTES), np.uint8)
+    lib = _lib.load_library()
+    lib.dan_record_sidecars.argtypes = [C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]
+    _lib.check(lib.dan_record_sidecars(raw.ctypes.data, RECORD_BYTES, len(raw), out.ctypes.data), "dan_record_sidecars")
+    return out
+
+
+def _raw_rows(a) -> np.ndarray:
+    a = np.asarray(a)
+    if a.dtype == RECORD_DTYPE:
+        return np.ascontiguousarray(a).reshape(-1).view(np.uint8).reshape(-1, RECORD_BYTES)
+    if a.dtype == np.uint8 and a.ndim == 2 and a.shape[1] == RECORD_BYTES:
+        return np.ascontiguousarray(a)
+    raise ValueError(f"records must be RECORD_DTYPE or (n, {RECORD_BYTES}) uint8, not {a.dtype} {a.shape}")
+
+
+def _source_chunks(source, chunk=256):
+    if isinstance(source, RecordFile):
+        for lo in range(0, len(source), chunk):
+            yield source.raw[lo:lo + chunk]
+    elif isinstance(source, np.ndarray):
+        raw = _raw_rows(source)
+        for lo in range(0, len(raw), chunk):
+            yield raw[lo:lo + chunk]
+    else:
+        for a in source:
+            yield _raw_rows(a)
+
+
+def write_compressed_records(path, source, level: int = 6, threads: int | None = None) -> int:
+    """Write records as a compressed record file: one zlib stream (standard-library zlib, `level`) per record, compressed on a pool
+    of `threads` threads (zlib releases the GIL). `source` is a RecordFile, a RECORD_DTYPE array, or an iterable of such arrays (e.g.
+    slices of an HDF5 dataset), which is consumed once and never held whole. Returns the number of records written."""
+    import shutil
+    import tempfile
+    from concurrent.futures import ThreadPoolExecutor
+    path = os.fspath(path)
+    index, count, data_bytes = [], 0, 0
+    pad = lambda f, k: f.write(b"\0" * (-k % 16)) and None
+    with open(path, "wb") as f, tempfile.TemporaryFile(dir=os.path.dirname(os.path.abspath(path))) as side, \
+            ThreadPoolExecutor(threads or min(32, os.cpu_count() or 1)) as pool:
+        f.write(b"\0" * 64)
+        for raw in _source_chunks(source):
+            streams = list(pool.map(lambda r: zlib.compress(r.data, level), raw))
+            lens = np.array([len(z) for z in streams], dtype=np.uint64)
+            entry = np.empty(len(streams), _CZ_INDEX)
+            entry["offset"] = data_bytes + np.concatenate(([0], np.cumsum(lens)[:-1])).astype(np.uint64) if len(streams) else []
+            entry["length"] = lens
+            index.append(entry)
+            f.write(b"".join(streams))
+            side.write(record_sidecars(raw).tobytes())
+            data_bytes += int(lens.sum())
+            count += len(streams)
+        pad(f, data_bytes)
+        sidecar_off = 64 + data_bytes + (-data_bytes % 16)
+        side.seek(0)
+        shutil.copyfileobj(side, f)
+        pad(f, count * SIDECAR_BYTES)
+        index_off = sidecar_off + count * SIDECAR_BYTES + (-(count * SIDECAR_BYTES) % 16)
+        f.write((np.concatenate(index) if index else np.zeros(0, _CZ_INDEX)).tobytes())
+        h = np.zeros(1, _CZ_HEADER)
+        h[0] = (COMPRESSED_MAGIC, 1, RECORD_BYTES, count, index_off, sidecar_off, 64, data_bytes, SIDECAR_BYTES, 0)
+        f.seek(0)
+        f.write(h.tobytes())
+    return count
+
+
+class CompressedRecordFile:
+    """A compressed record file (write_compressed_records). Opening it checks the header and every index entry against the file's
+    size and raises ValueError on a malformed file, before any record is read. The header pass runs on the sidecars; the records
+    themselves are inflated on the GPU by decode_records_device, or on the host by `records`."""
+
+    def __init__(self, path):
+        self.path = os.fspath(path)
+        size = os.path.getsize(self.path)
+        if size < 64:
+            raise ValueError(f"{self.path}: {size} bytes, shorter than the 64-byte header of a compressed record file")
+        mm = np.memmap(self.path, dtype=np.uint8, mode="r")
+        h = mm[:64].view(_CZ_HEADER)[0]
+        if bytes(h["magic"]) != COMPRESSED_MAGIC:
+            raise ValueError(f"{self.path}: not a compressed record file (magic {bytes(h['magic'])!r})")
+        if int(h["version"]) != 1 or int(h["record_bytes"]) != RECORD_BYTES or int(h["sidecar_bytes"]) != SIDECAR_BYTES:
+            raise ValueError(f"{self.path}: version {int(h['version'])}, {int(h['record_bytes'])}-byte records, {int(h['sidecar_bytes'])}-byte "
+                             f"sidecars; this reader takes version 1, {RECORD_BYTES} and {SIDECAR_BYTES}")
+        n = int(h["count"])
+        for name, off, nbytes in (("index", int(h["index_off"]), n * _CZ_INDEX.itemsize), ("sidecar", int(h["sidecar_off"]), n * SIDECAR_BYTES),
+                                  ("data", int(h["data_off"]), int(h["data_bytes"]))):
+            if off < 64 or off > size or nbytes > size - off:
+                raise ValueError(f"{self.path}: {name} section [{off}, +{nbytes}) lies outside the file's {size} bytes (truncated?)")
+        ix = int(h["index_off"])
+        index = np.frombuffer(mm[ix:ix + n * _CZ_INDEX.itemsize].tobytes(), _CZ_INDEX)
+        self.offsets, self.lengths = index["offset"].astype(np.uint64), index["length"].astype(np.uint32)
+        db = np.uint64(h["data_bytes"])
+        bad = np.flatnonzero((self.offsets > db) | (self.lengths.astype(np.uint64) > db - np.minimum(self.offsets, db)))
+        if len(bad):
+            raise ValueError(f"{self.path}: index entry of record {int(bad[0])} points past the data section's end ({len(bad)} such entries)")
+        so, do = int(h["sidecar_off"]), int(h["data_off"])
+        self.sidecars = mm[so:so + n * SIDECAR_BYTES].reshape(n, SIDECAR_BYTES)
+        self.data = mm[do:do + int(db)]
+        self.max_stream_bytes = int(self.lengths.max()) if n else 0
+
+    def __len__(self):
+        return len(self.offsets)
+
+    def stream(self, i) -> memoryview:
+        o = int(self.offsets[i])
+        return memoryview(self.data[o:o + int(self.lengths[i])])
+
+    def field(self, idx, name):
+        if name in ("name", "num_reads", "label", "vcfrec", "ref_bases"):
+            return self.sidecars[idx].view(SIDECAR_DTYPE)[0][name]
+        return self.records([idx])[0][name]
+
+    def records(self, indices) -> np.ndarray:
+        """Host inflate of `indices` (standard-library zlib) -> RECORD_DTYPE array. ValueError on a corrupt record."""
+        idx = _record_indices(self, indices)
+        out = np.empty(len(idx), RECORD_DTYPE)
+        raw = out.view(np.uint8).reshape(len(idx), RECORD_BYTES)
+        for k, i in enumerate(idx):
+            try:
+                rec = zlib.decompress(self.stream(int(i)))
+            except zlib.error as e:
+                raise ValueError(f"record {int(i)}: {e}") from None
+            if len(rec) != RECORD_BYTES:
+                raise ValueError(f"record {int(i)} inflates to {len(rec)} bytes, not {RECORD_BYTES}")
+            raw[k] = np.frombuffer(rec, np.uint8)
+        return out
+
+    def unpack(self, path, chunk: int = 256):
+        """Write the records back as a raw record file (RecordFile's format)."""
+        with open(os.fspath(path), "wb") as f:
+            for lo in range(0, len(self), chunk):
+                f.write(self.records(np.arange(lo, min(len(self), lo + chunk))).tobytes())
+
+
+def open_record_file(path):
+    """A RecordFile, or a CompressedRecordFile when the file starts with the compressed magic."""
+    with open(os.fspath(path), "rb") as f:
+        head = f.read(len(COMPRESSED_MAGIC))
+    return CompressedRecordFile(path) if head == COMPRESSED_MAGIC else RecordFile(os.fspath(path))
+
+
+def inflate_device(src: torch.Tensor, offsets: torch.Tensor, lengths: torch.Tensor, slot_bytes: int, stream=None):
+    """Inflate n zlib streams on the GPU (`dan_inflate_device`): stream i is src[offsets[i] : offsets[i] + lengths[i]] of the CUDA uint8
+    tensor `src`; -> (dst (n, slot_bytes) uint8, status (n,) int32), CUDA tensors. status[i] == 0 (INFLATE_STATUS) means stream i
+    inflated to exactly slot_bytes and passed its Adler-32 check; a failed stream leaves an all-zero row."""
+    from . import _lib
+    if not src.is_cuda or src.dtype != torch.uint8 or src.dim() != 1:
+        raise ValueError("src must be a 1-D CUDA uint8 tensor")
+    off = offsets.to(device=src.device, dtype=torch.int64).contiguous()
+    ln = lengths.to(device=src.device, dtype=torch.int32).contiguous()
+    n = off.numel()
+    if ln.numel() != n:
+        raise ValueError("one length per offset")
+    o, l = off.cpu().numpy(), ln.cpu().numpy()
+    if n and (o.min() < 0 or l.min() < 0 or (o + l).max() > src.numel()):
+        raise ValueError("a stream lies outside src")
+    dst = torch.empty((n, slot_bytes), dtype=torch.uint8, device=src.device)
+    status = torch.empty(n, dtype=torch.int32, device=src.device)
+    lib = _lib.load_library()
+    lib.dan_inflate_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
+    with torch.cuda.device(src.device):
+        st = (stream if stream is not None else torch.cuda.current_stream(src.device)).cuda_stream
+        _lib.check(lib.dan_inflate_device(src.data_ptr(), off.data_ptr(), ln.data_ptr(), n, dst.data_ptr(), slot_bytes, status.data_ptr(), st),
+                   "dan_inflate_device")
+    return dst, status
 
 
 class _FeederCfg(C.Structure):
@@ -366,10 +561,11 @@ def decode_records(records: RecordFile, indices, batch: HostBatch | None = None,
     return batch, sc
 
 
-def decode_record_headers(records: RecordFile, indices, use_q_scores=True, use_strands=True, keep_candidate_af=False, seed=0, max_reads=100,
+def decode_record_headers(records, indices, use_q_scores=True, use_strands=True, keep_candidate_af=False, seed=0, max_reads=100,
                           store_max_reads=200):
     """The header pass of the decode alone (`dan_decode_record_headers`, host code): -> (headers, scalars, ref_masks, var_masks).
-    headers is a RECORD_HEADER_DTYPE array; scalars and masks are what decode_records returns for the same arguments."""
+    headers is a RECORD_HEADER_DTYPE array; scalars and masks are what decode_records returns for the same arguments. On a
+    CompressedRecordFile the pass runs over the sidecars (`dan_decode_sidecar_headers`) with the same results."""
     from . import _lib
     lib = _lib.load_library()
     idx = _record_indices(records, indices)
@@ -379,8 +575,12 @@ def decode_record_headers(records: RecordFile, indices, use_q_scores=True, use_s
     hdr = np.zeros(n, RECORD_HEADER_DTYPE)
     out = _batch_struct((None, None, None, None, rm, vm), sc)
     cfg = _feeder_cfg(max_reads, store_max_reads, use_q_scores, use_strands, keep_candidate_af, seed)
-    lib.dan_decode_record_headers.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(_FeederCfg), C.POINTER(_RecordBatchC), C.c_void_p]
-    rc = lib.dan_decode_record_headers(records.raw.ctypes.data, RECORD_BYTES, idx.ctypes.data, n, C.byref(cfg), C.byref(out), hdr.ctypes.data)
+    if isinstance(records, CompressedRecordFile):
+        lib.dan_decode_sidecar_headers.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(_FeederCfg), C.POINTER(_RecordBatchC), C.c_void_p]
+        rc = lib.dan_decode_sidecar_headers(records.sidecars.ctypes.data, idx.ctypes.data, n, C.byref(cfg), C.byref(out), hdr.ctypes.data)
+    else:
+        lib.dan_decode_record_headers.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(_FeederCfg), C.POINTER(_RecordBatchC), C.c_void_p]
+        rc = lib.dan_decode_record_headers(records.raw.ctypes.data, RECORD_BYTES, idx.ctypes.data, n, C.byref(cfg), C.byref(out), hdr.ctypes.data)
     if rc < 0 and not sc["status"].any():
         _lib.check(rc, "dan_decode_record_headers")
     return hdr, sc, rm, vm
@@ -398,17 +598,49 @@ def _staging_bytes(n, max_reads):
     return need
 
 
+def _compressed_sizes(n, max_stream_bytes):
+    from . import _lib
+    lib = _lib.load_library()
+    for f in (lib.dan_decode_compressed_records_device_staging_bytes, lib.dan_decode_compressed_records_device_workspace_bytes):
+        f.argtypes, f.restype = [C.c_int, C.c_size_t], C.c_size_t
+    return (int(lib.dan_decode_compressed_records_device_staging_bytes(n, max_stream_bytes)),
+            int(lib.dan_decode_compressed_records_device_workspace_bytes(n, max_stream_bytes)))
+
+
+def _compressed_layout(n):
+    """Offsets of the compressed staging regions for n records, as dan_decode_compressed_records_device lays them out
+    (include/dan_b200.h): sidecars, stream offsets, stream lengths, headers, ref masks, var masks, streams."""
+    a16 = lambda x: (x + 15) & ~15
+    off = a16(n * SIDECAR_BYTES)
+    ln = off + 8 * n
+    hdr = a16(ln + 4 * n)
+    rm = hdr + n * RECORD_HEADER_DTYPE.itemsize
+    vm = rm + n * 201
+    return dict(side=0, off=off, len=ln, hdr=hdr, rm=rm, vm=vm, data=a16(vm + n * 201))
+
+
 class DeviceBatch:
     """Decoded batch on the GPU (`dan_decode_records_device`): device uint8 tiles in the layout dan_forward takes, the pinned host
     staging buffer the raw records are read into, and the device workspace they are copied to. The decoded tiles exist only on
-    the device."""
+    the device.
 
-    def __init__(self, capacity: int, num_reads: int = 100, device=None, read_len: int = 201):
+    With `max_stream_bytes` (a CompressedRecordFile's largest stream) the batch decodes compressed records
+    (`dan_decode_compressed_records_device`): the staging buffer holds sidecars and zlib streams, sized for `capacity` streams of
+    that size, and `inflate_status` is a device int32 tensor with each record's inflate status (INFLATE_STATUS) of the last decode."""
+
+    def __init__(self, capacity: int, num_reads: int = 100, device=None, read_len: int = 201, max_stream_bytes: int | None = None):
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.capacity, self.num_reads, self.device, self.size = capacity, num_reads, dev, 0
-        nbytes = _staging_bytes(capacity, num_reads)
+        self.max_stream_bytes = max_stream_bytes
+        if max_stream_bytes is None:
+            nbytes = wbytes = _staging_bytes(capacity, num_reads)
+            self.inflate_status = None
+        else:
+            _staging_bytes(capacity, num_reads)          # checks max_reads
+            nbytes, wbytes = _compressed_sizes(capacity, max_stream_bytes)
+            self.inflate_status = torch.zeros(capacity, dtype=torch.int32, device=dev)
         self.staging = torch.empty(nbytes, dtype=torch.uint8).pin_memory()
-        self.workspace = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        self.workspace = torch.empty(wbytes, dtype=torch.uint8, device=dev)
         mk = lambda *shape: torch.empty(shape, dtype=torch.uint8, device=dev)
         self.reads, self.q, self.strands = (mk(capacity, read_len, num_reads) for _ in range(3))
         self.ref, self.ref_masks, self.var_masks = (mk(capacity, read_len) for _ in range(3))
@@ -421,27 +653,41 @@ class DeviceBatch:
     def headers(self):
         """Header-pass descriptors of the last decode (RECORD_HEADER_DTYPE, a view into the staging buffer)."""
         n = self.size
-        off = (n * RECORD_BYTES + 15) & ~15
+        off = (n * RECORD_BYTES + 15) & ~15 if self.max_stream_bytes is None else _compressed_layout(n)["hdr"]
         return self.staging.numpy()[off:off + n * RECORD_HEADER_DTYPE.itemsize].view(RECORD_HEADER_DTYPE)
 
 
-def decode_records_device(records: RecordFile, indices, batch: DeviceBatch | None = None, use_q_scores=True, use_strands=True,
+def decode_records_device(records, indices, batch: DeviceBatch | None = None, use_q_scores=True, use_strands=True,
                           keep_candidate_af=False, seed=0, max_reads=100, store_max_reads=200, strict=True, stream=None):
     """decode_records with the tile pass on the GPU (`dan_decode_records_device`). The records go into the batch's pinned staging
     buffer (one memcpy from the file for a contiguous ascending range, an index gather otherwise), the header pass runs on the host,
     then one H2D copy and the tile kernel run on `stream` (default: the current stream). Returns (batch, scalars) with the same
     outputs as decode_records, byte for byte. Asynchronous: the batch's tensors are ready once `stream` has passed the call, and
-    the batch may be decoded into again only after that."""
+    the batch may be decoded into again only after that.
+
+    `records` is a RecordFile, a CompressedRecordFile or a path (opened by its magic). For a compressed file the zlib streams are
+    staged instead of the records, the header pass runs over the sidecars, and the records are inflated on the GPU before the tile
+    pass (`dan_decode_compressed_records_device`); the batch must be a compressed DeviceBatch (default: one sized for the file). The
+    call does not wait for the inflate: `batch.inflate_status` holds each record's status once `stream` has passed the call, and a
+    record whose stream is corrupt decodes to all-zero tiles and masks."""
     from . import _lib
     lib = _lib.load_library()
+    if not isinstance(records, (RecordFile, CompressedRecordFile)):
+        records = open_record_file(records)
+    compressed = isinstance(records, CompressedRecordFile)
     idx = _record_indices(records, indices)
     n = len(idx)
     if batch is None:
-        batch = DeviceBatch(max(n, 1), num_reads=max_reads)
+        batch = DeviceBatch(max(n, 1), num_reads=max_reads, max_stream_bytes=records.max_stream_bytes if compressed else None)
     if n > batch.capacity:
         raise ValueError(f"{n} records > capacity {batch.capacity}")
     if batch.num_reads != max_reads:
         raise ValueError(f"batch holds {batch.num_reads} reads per candidate, max_reads is {max_reads}")
+    if compressed != (batch.max_stream_bytes is not None):
+        raise ValueError("a compressed record file needs a DeviceBatch with max_stream_bytes, a raw one a DeviceBatch without")
+    if compressed:
+        return _decode_compressed_device(records, idx, batch, _feeder_cfg(max_reads, store_max_reads, use_q_scores, use_strands,
+                                                                           keep_candidate_af, seed), strict, stream)
     if n and np.all(np.diff(idx) == 1):
         records.read_block(int(idx[0]), n, batch.staging)
     else:
@@ -471,19 +717,70 @@ def decode_records_device(records: RecordFile, indices, batch: DeviceBatch | Non
 _VCF_OFFSET = RECORD_DTYPE.fields["vcfrec"][1]
 
 
+def _stage_streams(rf: CompressedRecordFile, idx, dst: np.ndarray):
+    """Copy the streams of records idx back to back into dst; -> their offsets in dst. A contiguous ascending range whose streams
+    lie back to back in the file (as write_compressed_records lays them out) is one copy."""
+    n = len(idx)
+    off, ln = rf.offsets[idx], rf.lengths[idx].astype(np.uint64)
+    if n and np.all(np.diff(idx) == 1) and np.all(off[1:] == off[:-1] + ln[:-1]):
+        span = int(off[-1] + ln[-1] - off[0])
+        if span > dst.size:
+            raise ValueError(f"{n} streams of {span} bytes exceed the batch's {dst.size}-byte stream region")
+        dst[:span] = rf.data[int(off[0]):int(off[0]) + span]
+        return off - off[0]
+    pos = np.concatenate(([0], np.cumsum(ln))).astype(np.uint64)
+    if n and int(pos[-1]) > dst.size:
+        raise ValueError(f"{n} streams of {int(pos[-1])} bytes exceed the batch's {dst.size}-byte stream region")
+    for k, i in enumerate(idx):
+        o = int(rf.offsets[i])
+        dst[int(pos[k]):int(pos[k + 1])] = rf.data[o:o + int(rf.lengths[i])]
+    return pos[:n]
+
+
+def _decode_compressed_device(rf: CompressedRecordFile, idx, batch: DeviceBatch, cfg, strict, stream):
+    from . import _lib
+    lib = _lib.load_library()
+    n = len(idx)
+    lay = _compressed_layout(n)
+    st = batch.staging.numpy()
+    st[:n * SIDECAR_BYTES].reshape(n, SIDECAR_BYTES)[:] = rf.sidecars[idx]
+    st[lay["off"]:lay["off"] + 8 * n].view(np.uint64)[:] = _stage_streams(rf, idx, st[lay["data"]:])
+    st[lay["len"]:lay["len"] + 4 * n].view(np.uint32)[:] = rf.lengths[idx]
+    sc = _scalars(n)
+    out = _batch_struct((batch.reads, batch.q, batch.strands, batch.ref, batch.ref_masks, batch.var_masks), sc)
+    lib.dan_decode_compressed_records_device.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(_FeederCfg),
+                                                         C.POINTER(_RecordBatchC), C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]
+    with torch.cuda.device(batch.device):
+        s = (stream if stream is not None else torch.cuda.current_stream(batch.device)).cuda_stream
+        rc = lib.dan_decode_compressed_records_device(batch.staging.data_ptr(), batch.staging.numel(), idx.ctypes.data, n, C.byref(cfg),
+                                                      C.byref(out), batch.workspace.data_ptr(), batch.workspace.numel(),
+                                                      batch.inflate_status.data_ptr(), s)
+    batch.size = n
+    side = st[:n * SIDECAR_BYTES].view(SIDECAR_DTYPE)
+    batch.meta = [(a.decode(), b.decode()) for a, b in zip(side["name"].tolist(), side["vcfrec"].tolist())]
+    if rc == -1 and sc["status"].any():
+        if strict:
+            _raise_failed(idx, sc)
+    else:
+        _lib.check(rc, "dan_decode_compressed_records_device")
+    return batch, sc
+
+
 class _CallSlot:
     """One ring slot of call_record_file: a DeviceBatch plus the pinned buffers of its allele lengths and results."""
 
-    def __init__(self, capacity, num_reads, dev):
-        self.batch = DeviceBatch(capacity, num_reads, dev)
+    def __init__(self, capacity, num_reads, dev, max_stream_bytes=None):
+        self.batch = DeviceBatch(capacity, num_reads, dev, max_stream_bytes=max_stream_bytes)
         pin = lambda shape, dt: torch.empty(shape, dtype=dt).pin_memory()
         self.ref_len, self.var_len = pin(capacity, torch.int32), pin(capacity, torch.int32)
         self.scores, self.gt, self.q = pin((capacity, 4), torch.float32), pin(capacity, torch.int8), pin(capacity, torch.int32)
+        self.inflate_status = None if max_stream_bytes is None else pin(capacity, torch.int32)
 
 
 def call_record_file(model, records, start=0, stop=None, batch_size=1036, depth=2, thresholds=None, strict=True, failed=None, seed=0,
                      store_max_reads=200, keep_candidate_af=False):
-    """Stream records [start, stop) of a record file (path or RecordFile) to scored VCF records and genotype calls: the whole path of
+    """Stream records [start, stop) of a record file (a path, opened by its magic, a RecordFile or a CompressedRecordFile) to scored VCF
+    records and genotype calls: the whole path of
     the reference's inference (main.py --test_file -> trainer.test -> append_vcf_records -> tools/format_vcf.py's thresholds) in one call.
 
     Yields, per batch of up to `batch_size` records in file order, (names, vcf_lines, gt, q): record names, the VCF records with the
@@ -495,9 +792,12 @@ def call_record_file(model, records, start=0, stop=None, batch_size=1036, depth=
     scores (16 bytes) and gt / q per record come back. `depth` slots rotate, so the host work of batch k+1 overlaps the GPU work of
     batch k; a slot is reused only after its batch's results have been yielded.
     Records the reference's loader raises on (status != 0): strict=True raises naming them; strict=False leaves them out and appends
-    (record index, status) to `failed` when a list is given."""
-    import os
-    rf = records if isinstance(records, RecordFile) else RecordFile(os.fspath(records))
+    (record index, status) to `failed` when a list is given.
+    From a compressed file the streams are staged and inflated on the device; a record whose stream is corrupt gets status
+    REC_CORRUPT and is handled the same way. Its inflate status is known only once the batch's device work has finished, so a strict
+    raise for it comes when that batch is finished (after the batches before it have been yielded), not when it is submitted."""
+    rf = records if isinstance(records, (RecordFile, CompressedRecordFile)) else open_record_file(records)
+    msb = rf.max_stream_bytes if isinstance(rf, CompressedRecordFile) else None
     stop = len(rf) if stop is None else int(stop)
     start = int(start)
     if not 0 <= start <= stop <= len(rf):
@@ -512,7 +812,7 @@ def call_record_file(model, records, start=0, stop=None, batch_size=1036, depth=
                 max_reads=model.num_single_reads, store_max_reads=store_max_reads)
     with torch.cuda.device(dev):
         main, side = torch.cuda.current_stream(dev), torch.cuda.Stream(dev)
-        free = deque(_CallSlot(min(batch_size, max(stop - start, 1)), model.num_single_reads, dev) for _ in range(depth))
+        free = deque(_CallSlot(min(batch_size, max(stop - start, 1)), model.num_single_reads, dev, msb) for _ in range(depth))
         side.wait_stream(main)          # the slots' device memory may be blocks the current stream freed with work still queued on them
         pending = deque()
 
@@ -537,6 +837,8 @@ def call_record_file(model, records, start=0, stop=None, batch_size=1036, depth=
                 slot.scores[:n].copy_(scores, non_blocking=True)
                 slot.gt[:n].copy_(gt, non_blocking=True)
                 slot.q[:n].copy_(q, non_blocking=True)
+                if slot.inflate_status is not None:
+                    slot.inflate_status[:n].copy_(batch.inflate_status[:n], non_blocking=True)
                 ev = torch.cuda.Event()
                 ev.record(main)
             pending.append((slot, idx, sc["status"].copy(), batch.meta, ev))
@@ -545,6 +847,11 @@ def call_record_file(model, records, start=0, stop=None, batch_size=1036, depth=
             slot, idx, status, meta, ev = pending.popleft()
             ev.synchronize()
             n = len(idx)
+            if slot.inflate_status is not None:
+                status = np.where((status == 0) & (slot.inflate_status[:n].numpy() != 0), REC_CORRUPT, status)
+                if strict and (status == REC_CORRUPT).any():
+                    free.append(slot)
+                    _raise_failed(idx, {"status": status})
             good = status == 0
             if failed is not None:
                 failed.extend((int(idx[b]), int(status[b])) for b in np.flatnonzero(~good))

@@ -290,6 +290,49 @@ size_t dan_decode_records_device_workspace_bytes(int n, const dan_feeder_config*
 int dan_decode_records_device(void* staging, size_t staging_bytes, const int64_t* indices, int n, const dan_feeder_config* cfg,
                               const dan_record_batch* out, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- compressed record files ------------------------------------------------------------------------------------------------------
+ * File layout (all fields little-endian; written and opened by dl4vc_b200/feeder.py):
+ *   header, 64 bytes: magic "DL4VCZR1", u32 version = 1, u32 record_bytes = DAN_RECORD_BYTES, u64 count, u64 index_off,
+ *                     u64 sidecar_off, u64 data_off, u64 data_bytes, u32 sidecar_bytes = DAN_SIDECAR_BYTES, u32 reserved = 0;
+ *   index   at index_off:   count entries of 12 bytes, u64 offset into the data section + u32 compressed length;
+ *   sidecar at sidecar_off: count sidecars of DAN_SIDECAR_BYTES (dan_record_sidecars);
+ *   data    at data_off:    data_bytes of RFC 1950 zlib streams, one per record holding its DAN_RECORD_BYTES, in record order.
+ * A sidecar holds exactly the record bytes the header pass reads, plus the name: [name 16][num_reads 4][label 1][vcfrec 128]
+ * [ref_bases 201][single_reads column 100 of stored rows 0..199][column 101 of rows 0..199]. The header pass over a record's sidecar
+ * gives the same headers, scalars and masks as over the record. */
+#define DAN_SIDECAR_BYTES 750
+int dan_record_sidecars(const void* records, size_t record_stride, int n, void* out);
+
+/* dan_decode_record_headers over sidecars (DAN_SIDECAR_BYTES apart): sidecar indices[i] decodes into entry i, keyed by indices[i]. */
+int dan_decode_sidecar_headers(const void* sidecars, const int64_t* indices, int n, const dan_feeder_config* cfg, const dan_record_batch* out,
+                               dan_record_header* headers);
+
+/* Batched zlib inflate on the device: stream i is src[offsets[i], offsets[i] + lengths[i]) and inflates into
+ * dst[i * slot_bytes, (i + 1) * slot_bytes). Stored, fixed- and dynamic-Huffman blocks, 32 KB window, zlib header and Adler-32 trailer.
+ * status[i] = DAN_INFLATE_OK only when the stream inflated to exactly slot_bytes and its Adler-32 matched; any other status leaves an
+ * all-zero slot. Every read stays inside its stream and every write inside its slot, so a bad stream never affects another.
+ * All pointers are DEVICE pointers; asynchronous on `stream`. */
+enum { DAN_INFLATE_OK = 0, DAN_INFLATE_E_HEADER = 1, DAN_INFLATE_E_BLOCK = 2, DAN_INFLATE_E_CODES = 3, DAN_INFLATE_E_DISTANCE = 4,
+       DAN_INFLATE_E_INPUT = 5, DAN_INFLATE_E_OUTPUT_LONG = 6, DAN_INFLATE_E_OUTPUT_SHORT = 7, DAN_INFLATE_E_ADLER = 8 };
+int dan_inflate_device(const void* src, const uint64_t* offsets, const uint32_t* lengths, int n, void* dst, uint64_t slot_bytes,
+                       int32_t* status, void* stream);
+
+/* Device decode of compressed records. `staging` (pinned HOST, dan_decode_compressed_records_device_staging_bytes(capacity,
+ * max_stream_bytes) bytes) holds, for the n records of the call, at offsets that depend only on n (each region 16-byte aligned):
+ *   [n sidecars][n u64 stream offsets][n u32 stream lengths][n dan_record_header][n*201 ref masks][n*201 var masks][streams]
+ * The caller fills the sidecars, the index and the streams (offsets relative to the start of the streams region); the header pass
+ * over the sidecars writes the headers and masks. One cudaMemcpyAsync moves everything from the index to the end of the last stream into
+ * `workspace` behind n record images; dan_inflate_device fills the images, and the tile pass of dan_decode_records_device runs over
+ * them. inflate_status (DEVICE, n int32) receives the inflate status; a record whose stream fails gets all-zero tiles, ref and masks.
+ * For records that inflate, every output equals dan_decode_records' on the raw records byte for byte. DAN_E_WORKSPACE (no copy, no
+ * launch) if a buffer is too small; DAN_E_INVALID (no copy) if an index entry leaves the streams region, and with per-record status as
+ * dan_decode_records. Asynchronous: neither buffer may be reused before the stream has passed this call. */
+size_t dan_decode_compressed_records_device_staging_bytes(int n, size_t max_stream_bytes);
+size_t dan_decode_compressed_records_device_workspace_bytes(int n, size_t max_stream_bytes);
+int dan_decode_compressed_records_device(void* staging, size_t staging_bytes, const int64_t* indices, int n, const dan_feeder_config* cfg,
+                                         const dan_record_batch* out, void* workspace, size_t workspace_bytes, int32_t* inflate_status,
+                                         void* stream);
+
 /* Test hook for the bit-exact integer/encoding work (dl4vc/model.py:450-627,719): writes the conv-1 input in the
  * reference's logical order (batch, Cin, num_reads, read_len) fp32, DEVICE pointer. */
 int dan_encode(dan_model* m, const uint8_t* reads, const uint8_t* q_scores, const uint8_t* strands,
