@@ -23,7 +23,7 @@ LIB_PATH = os.environ.get("DAN_B200_LIB") or os.path.join(os.path.dirname(os.pat
 EXPORTED_SYMBOLS = (
     "dan_last_error", "dan_version", "dan_model_create", "dan_model_destroy", "dan_model_load_weights",
     "dan_model_set_pass_candidates", "dan_workspace_bytes", "dan_forward", "dan_workspace_bytes_host",
-    "dan_forward_host", "dan_scores", "dan_genotype_calls", "dan_format_vcf_info", "dan_make_mask_vectors", "dan_encode", "dan_encode_bf16", "dan_model_set_flags", "dan_model_bf16_route", "dan_train_tape_bytes", "dan_train_forward", "dan_backward", "dan_losses", "dan_close_table_update", "dan_decode_records", "dan_decode_record_headers", "dan_decode_records_device", "dan_decode_records_device_workspace_bytes", "dan_record_sidecars", "dan_decode_sidecar_headers", "dan_inflate_device", "dan_decode_compressed_records_device", "dan_decode_compressed_records_device_staging_bytes", "dan_decode_compressed_records_device_workspace_bytes", "dan_debug_fc_input", "dan_last_launch_count", "dan_measure_fma_tflops",
+    "dan_forward_host", "dan_scores", "dan_genotype_calls", "dan_format_vcf_info", "dan_make_mask_vectors", "dan_encode", "dan_encode_bf16", "dan_model_set_flags", "dan_model_bf16_route", "dan_train_tape_bytes", "dan_train_forward", "dan_backward", "dan_losses", "dan_close_table_update", "dan_decode_records", "dan_decode_record_headers", "dan_decode_records_device", "dan_decode_records_device_workspace_bytes", "dan_record_sidecars", "dan_decode_sidecar_headers", "dan_inflate_device", "dan_deflate_bound", "dan_deflate_device", "dan_deflate_compact", "dan_decode_compressed_records_device", "dan_decode_compressed_records_device_staging_bytes", "dan_decode_compressed_records_device_workspace_bytes", "dan_debug_fc_input", "dan_last_launch_count", "dan_measure_fma_tflops",
     "dan_profile_enable", "dan_profile_read", "dan_profile_class_name",
 )
 PROF_NUM_CLASSES = 4

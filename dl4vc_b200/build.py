@@ -14,7 +14,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libdan_b200.so")
-SOURCES = ["dan_capi.cu", "dan_fp32.cu", "dan_bf16.cu", "dan_train.cu", "dan_losses.cu", "dan_feeder.cu", "dan_inflate.cu"]
+SOURCES = ["dan_capi.cu", "dan_fp32.cu", "dan_bf16.cu", "dan_train.cu", "dan_losses.cu", "dan_feeder.cu", "dan_inflate.cu", "dan_deflate.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "--use_fast_math=false",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "--expt-relaxed-constexpr", "-Xptxas", "-v"]
 NVCC_FLAGS.remove("--use_fast_math=false")

@@ -12,13 +12,13 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 #include "dan_internal.h"
+#include "dan_zlib.cuh"
 
 namespace {
 
 constexpr int kWarps = 4;                  // streams per CTA
 constexpr int kLitBits = 10, kDistBits = 8;
 constexpr int kMaxBits = 15;
-constexpr uint32_t kAdlerMod = 65521;
 
 struct Huff {                              // one decode table set
   uint16_t count[kMaxBits + 1];            // codes of each length
@@ -31,13 +31,6 @@ struct WarpSmem {
   uint8_t lens[288 + 32];                  // code lengths of the current block: literal/length at [0, 288), distance at [288, 320)
   uint8_t cl[19];                          // code-length code lengths of a dynamic block
 };
-
-__constant__ uint16_t kLenBase[29] = {3, 4, 5, 6, 7, 8, 9, 10, 11, 13, 15, 17, 19, 23, 27, 31, 35, 43, 51, 59, 67, 83, 99, 115, 131, 163, 195, 227, 258};
-__constant__ uint8_t kLenExtra[29] = {0, 0, 0, 0, 0, 0, 0, 0, 1, 1, 1, 1, 2, 2, 2, 2, 3, 3, 3, 3, 4, 4, 4, 4, 5, 5, 5, 5, 0};
-__constant__ uint16_t kDistBase[30] = {1, 2, 3, 4, 5, 7, 9, 13, 17, 25, 33, 49, 65, 97, 129, 193, 257, 385, 513, 769, 1025, 1537, 2049, 3073, 4097,
-                                       6145, 8193, 12289, 16385, 24577};
-__constant__ uint8_t kDistExtra[30] = {0, 0, 0, 0, 1, 1, 2, 2, 3, 3, 4, 4, 5, 5, 6, 6, 7, 7, 8, 8, 9, 9, 10, 10, 11, 11, 12, 12, 13, 13};
-__constant__ uint8_t kClOrder[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
 
 // Warp-uniform LSB-first bit reader over src[0, len).
 struct Bits {
@@ -238,19 +231,11 @@ __global__ void __launch_bounds__(kWarps * 32) inflate_kernel(const uint8_t* __r
     else if (o != slot_bytes) st = DAN_INFLATE_E_OUTPUT_SHORT;
     else {
       __syncwarp();
-      // Adler-32 over 32 chunks: chunk [s, s + m) adds S1 = sum b_k to A and (n - s) S1 - sum k b_k to B (k local)
+      // Adler-32 over 32 chunks, one per lane
       const uint64_t chunk = (slot_bytes + 31) / 32, s = min((uint64_t)lane * chunk, slot_bytes), m = min(chunk, slot_bytes - s);
-      uint64_t s1 = 0, s2 = 0;
-      for (uint64_t k = 0; k < m; ++k) {
-        const uint32_t x = out[s + k];
-        s1 += x; s2 += (k % kAdlerMod) * x;
-        if ((k & 4095) == 4095) { s1 %= kAdlerMod; s2 %= kAdlerMod; }
-      }
-      s1 %= kAdlerMod; s2 %= kAdlerMod;
-      uint64_t bb = ((slot_bytes - s) % kAdlerMod * s1 + kAdlerMod - s2) % kAdlerMod;
-      for (int d = 16; d; d >>= 1) { s1 += __shfl_xor_sync(0xffffffffu, s1, d); bb += __shfl_xor_sync(0xffffffffu, bb, d); }
-      const uint32_t A = (uint32_t)((1 + s1) % kAdlerMod), B = (uint32_t)((slot_bytes % kAdlerMod + bb) % kAdlerMod);
-      if (((B << 16) | A) != ((a0 << 24) | (a1 << 16) | (a2 << 8) | a3)) st = DAN_INFLATE_E_ADLER;
+      AdlerPart ad = adler_chunk(out, slot_bytes, s, m);
+      for (int d = 16; d; d >>= 1) { ad.a += __shfl_xor_sync(0xffffffffu, ad.a, d); ad.b += __shfl_xor_sync(0xffffffffu, ad.b, d); }
+      if (adler_value(ad.a, ad.b, slot_bytes) != ((a0 << 24) | (a1 << 16) | (a2 << 8) | a3)) st = DAN_INFLATE_E_ADLER;
     }
   }
   __syncwarp();

@@ -14,7 +14,8 @@ RecordFile / decode_records  raw fixed-record pileup file (the reference's HDF5 
 decode_records_device  the same decode with the tile pass on the GPU (`dan_decode_records_device`): host header pass (parse, sampling,
                    masks), one H2D copy of the staged raw records, a kernel that writes the device tiles `dan_forward` reads.
 CompressedRecordFile  the same records as one zlib stream each, with an index and per-record sidecars (the bytes the header pass
-                   reads); write_compressed_records writes one, decode_records_device inflates the records on the GPU (`dan_inflate_device`).
+                   reads); write_compressed_records writes one, with host zlib or on the GPU (`dan_deflate_device`), and
+                   decode_records_device inflates the records on the GPU (`dan_inflate_device`).
 call_record_file   record file -> scored VCF lines and genotype calls, streamed in batches through a ring of pinned slots.
 format_vcf_info    the `BP=..;NV=..;HV=..;OV=..` field `utils.append_vcf_records` splices into VCF column 3 (`utils.py:162-178`).
 """
@@ -353,30 +354,47 @@ def _source_chunks(source, chunk=256):
             yield _raw_rows(a)
 
 
-def write_compressed_records(path, source, level: int = 6, threads: int | None = None) -> int:
-    """Write records as a compressed record file: one zlib stream (standard-library zlib, `level`) per record, compressed on a pool
-    of `threads` threads (zlib releases the GIL). `source` is a RecordFile, a RECORD_DTYPE array, or an iterable of such arrays (e.g.
-    slices of an HDF5 dataset), which is consumed once and never held whole. Returns the number of records written."""
+def write_compressed_records(path, source, level: int | None = None, threads: int | None = None, device=None) -> int:
+    """Write records as a compressed record file: one zlib stream per record. `source` is a RecordFile, a RECORD_DTYPE array, or an
+    iterable of such arrays (e.g. slices of an HDF5 dataset), which is consumed once and never held whole. Returns the number of
+    records written.
+
+    device=None: standard-library zlib at `level` (default 6) on a pool of `threads` threads (zlib releases the GIL).
+    device=<CUDA device>: the records are compressed on that GPU (`dan_deflate_device`, see deflate_device); `level` and `threads`
+    do not apply and raise ValueError when given. The file's layout is the same either way; the streams differ, and both inflate to
+    the records."""
+    path = os.fspath(path)
+    if device is None:
+        chunks = _host_deflate_chunks(source, 6 if level is None else level, threads)
+    else:
+        dev = torch.device(device)
+        if dev.type != "cuda":
+            raise ValueError(f"device must be a CUDA device, not {dev}")
+        if level is not None or threads is not None:
+            raise ValueError("level and threads apply to host compression (device=None); the GPU deflate has one setting")
+        chunks = _device_deflate_chunks(source, dev)
+    return _write_compressed(path, chunks)
+
+
+def _write_compressed(path, chunks) -> int:
+    """The file around the streams: `chunks` yields (stream bytes back to back, their lengths, the chunk's sidecars)."""
+    import contextlib
     import shutil
     import tempfile
-    from concurrent.futures import ThreadPoolExecutor
-    path = os.fspath(path)
     index, count, data_bytes = [], 0, 0
     pad = lambda f, k: f.write(b"\0" * (-k % 16)) and None
-    with open(path, "wb") as f, tempfile.TemporaryFile(dir=os.path.dirname(os.path.abspath(path))) as side, \
-            ThreadPoolExecutor(threads or min(32, os.cpu_count() or 1)) as pool:
+    with contextlib.closing(chunks), open(path, "wb") as f, tempfile.TemporaryFile(dir=os.path.dirname(os.path.abspath(path))) as side:
         f.write(b"\0" * 64)
-        for raw in _source_chunks(source):
-            streams = list(pool.map(lambda r: zlib.compress(r.data, level), raw))
-            lens = np.array([len(z) for z in streams], dtype=np.uint64)
-            entry = np.empty(len(streams), _CZ_INDEX)
-            entry["offset"] = data_bytes + np.concatenate(([0], np.cumsum(lens)[:-1])).astype(np.uint64) if len(streams) else []
+        for data, lens, sidecars in chunks:
+            lens = np.asarray(lens, dtype=np.uint64)
+            entry = np.empty(len(lens), _CZ_INDEX)
+            entry["offset"] = data_bytes + np.concatenate(([0], np.cumsum(lens)[:-1])).astype(np.uint64) if len(lens) else []
             entry["length"] = lens
             index.append(entry)
-            f.write(b"".join(streams))
-            side.write(record_sidecars(raw).tobytes())
+            f.write(data)
+            side.write(sidecars.tobytes())
             data_bytes += int(lens.sum())
-            count += len(streams)
+            count += len(lens)
         pad(f, data_bytes)
         sidecar_off = 64 + data_bytes + (-data_bytes % 16)
         side.seek(0)
@@ -389,6 +407,91 @@ def write_compressed_records(path, source, level: int = 6, threads: int | None =
         f.seek(0)
         f.write(h.tobytes())
     return count
+
+
+def _host_deflate_chunks(source, level, threads):
+    from concurrent.futures import ThreadPoolExecutor
+    with ThreadPoolExecutor(threads or min(32, os.cpu_count() or 1)) as pool:
+        for raw in _source_chunks(source):
+            streams = list(pool.map(lambda r: zlib.compress(r.data, level), raw))
+            yield b"".join(streams), [len(z) for z in streams], record_sidecars(raw)
+
+
+class _DeflateSlot:
+    """One chunk in flight on the GPU: pinned staging of the raw records, the device input, stream slots and packed output, and
+    pinned landing buffers for the lengths / status and the packed streams."""
+
+    def __init__(self, capacity, dev):
+        bound = deflate_bound(RECORD_BYTES)
+        self.capacity = capacity
+        self.host_in = torch.empty(capacity * RECORD_BYTES, dtype=torch.uint8, pin_memory=True)
+        self.dev_in = torch.empty(capacity * RECORD_BYTES, dtype=torch.uint8, device=dev)
+        self.slots = torch.empty(capacity * bound, dtype=torch.uint8, device=dev)
+        self.packed = torch.empty(capacity * bound, dtype=torch.uint8, device=dev)
+        self.meta = torch.empty(2 * capacity, dtype=torch.int32, device=dev)            # lengths, then status
+        self.offsets = torch.empty(capacity + 1, dtype=torch.int64, device=dev)
+        self.host_meta = torch.empty(2 * capacity, dtype=torch.int32, pin_memory=True)
+        self.host_out = torch.empty(capacity * bound, dtype=torch.uint8, pin_memory=True)
+        self.done = torch.cuda.Event()
+        self.job = None                                                                   # (first record, count, sidecars)
+
+
+def _device_deflate_chunks(source, dev, depth=2):
+    """GPU compression of _source_chunks(source). Per chunk: the records into a pinned slot, one H2D copy, dan_deflate_device,
+    dan_deflate_compact, one D2H copy of lengths and status; once those have landed, one D2H copy of exactly the compressed bytes.
+    `depth` slots rotate, so reading chunk k + 1 and cutting its sidecars on the host overlap the GPU work of chunk k."""
+    from . import _lib
+    lib = _deflate_lib()
+    stream, copy_stream = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
+    slots, first = [], 0
+
+    def finish(slot):
+        start, n, sidecars = slot.job
+        slot.job = None
+        slot.done.synchronize()
+        lens, status = slot.host_meta[:n].numpy().view(np.uint32).copy(), slot.host_meta[slot.capacity:slot.capacity + n].numpy()
+        bad = np.flatnonzero(status != 0)
+        if len(bad):
+            raise RuntimeError(f"record #{start + int(bad[0])}: GPU deflate failed with status {int(status[bad[0]])}")
+        total = int(lens.sum(dtype=np.uint64))
+        with torch.cuda.stream(copy_stream):
+            copy_stream.wait_event(slot.done)
+            slot.host_out[:total].copy_(slot.packed[:total], non_blocking=True)
+        copy_stream.synchronize()
+        return memoryview(slot.host_out[:total].numpy()), lens, sidecars
+
+    try:
+        with torch.cuda.device(dev):
+            stream.wait_stream(torch.cuda.current_stream(dev))
+            for k, raw in enumerate(_source_chunks(source)):
+                n = len(raw)
+                if len(slots) < depth:
+                    slots.append(None)
+                slot = slots[k % depth]
+                if slot is not None and slot.job is not None:
+                    yield finish(slot)
+                if slot is None or slot.capacity < n:
+                    slot = slots[k % depth] = _DeflateSlot(max(n, 1), dev)
+                    stream.wait_stream(torch.cuda.current_stream(dev))
+                if n:
+                    np.copyto(slot.host_in[:n * RECORD_BYTES].numpy(), raw.reshape(-1))
+                with torch.cuda.stream(stream):
+                    slot.dev_in[:n * RECORD_BYTES].copy_(slot.host_in[:n * RECORD_BYTES], non_blocking=True)
+                    st = stream.cuda_stream
+                    _lib.check(lib.dan_deflate_device(slot.dev_in.data_ptr(), n, RECORD_BYTES, slot.slots.data_ptr(), slot.meta.data_ptr(),
+                                                      slot.meta.data_ptr() + 4 * slot.capacity, st), "dan_deflate_device")
+                    _lib.check(lib.dan_deflate_compact(slot.slots.data_ptr(), slot.meta.data_ptr(), n, RECORD_BYTES, slot.packed.data_ptr(),
+                                                       slot.offsets.data_ptr(), st), "dan_deflate_compact")
+                    slot.host_meta.copy_(slot.meta, non_blocking=True)
+                    slot.done.record(stream)
+                slot.job = (first, n, record_sidecars(raw))
+                first += n
+            pending = sorted((s for s in slots if s is not None and s.job is not None), key=lambda s: s.job[0])
+            for slot in pending:
+                yield finish(slot)
+    finally:
+        stream.synchronize()
+        copy_stream.synchronize()
 
 
 class CompressedRecordFile:
@@ -490,6 +593,51 @@ def inflate_device(src: torch.Tensor, offsets: torch.Tensor, lengths: torch.Tens
         _lib.check(lib.dan_inflate_device(src.data_ptr(), off.data_ptr(), ln.data_ptr(), n, dst.data_ptr(), slot_bytes, status.data_ptr(), st),
                    "dan_inflate_device")
     return dst, status
+
+
+def _deflate_lib():
+    from . import _lib
+    lib = _lib.load_library()
+    lib.dan_deflate_bound.argtypes = [C.c_uint64]
+    lib.dan_deflate_bound.restype = C.c_size_t
+    lib.dan_deflate_device.argtypes = [C.c_void_p, C.c_int, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.dan_deflate_compact.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]
+    return lib
+
+
+def deflate_bound(slot_bytes: int) -> int:
+    """Bytes of one output slot of dan_deflate_device: the stored-block encoding of slot_bytes, which no stream exceeds."""
+    return int(_deflate_lib().dan_deflate_bound(slot_bytes))
+
+
+def deflate_device(src: torch.Tensor, stream=None):
+    """Compress the n rows of the CUDA uint8 tensor `src` (n, slot) on the GPU (`dan_deflate_device`), each into one standard zlib
+    stream that zlib.decompress and inflate_device both take; the mirror of inflate_device. -> (streams, offsets, lengths, status),
+    CUDA tensors: the streams packed back to back in one uint8 tensor, stream i at streams[offsets[i] : offsets[i] + lengths[i]]
+    (int64 / int32), and status[i] == 0 (DAN_DEFLATE_OK) for each. Waits for the device to learn the packed size."""
+    from . import _lib
+    if not isinstance(src, torch.Tensor) or not src.is_cuda or src.dtype != torch.uint8 or src.dim() != 2:
+        raise ValueError("src must be a 2-D (n, slot) CUDA uint8 tensor")
+    src = src.contiguous()
+    n, slot = src.shape
+    lib = _deflate_lib()
+    bound = int(lib.dan_deflate_bound(slot))
+    dev = src.device
+    slots = torch.empty(n * bound, dtype=torch.uint8, device=dev)
+    packed = torch.empty(n * bound, dtype=torch.uint8, device=dev)
+    lengths = torch.empty(n, dtype=torch.int32, device=dev)
+    status = torch.empty(n, dtype=torch.int32, device=dev)
+    offsets = torch.empty(n + 1, dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        stream = stream if stream is not None else torch.cuda.current_stream(dev)
+        st = stream.cuda_stream
+        _lib.check(lib.dan_deflate_device(src.data_ptr(), n, slot, slots.data_ptr(), lengths.data_ptr(), status.data_ptr(), st),
+                   "dan_deflate_device")
+        _lib.check(lib.dan_deflate_compact(slots.data_ptr(), lengths.data_ptr(), n, slot, packed.data_ptr(), offsets.data_ptr(), st),
+                   "dan_deflate_compact")
+        stream.synchronize()
+        total = int(offsets[n].item())
+    return packed[:total], offsets[:n], lengths, status
 
 
 class _FeederCfg(C.Structure):

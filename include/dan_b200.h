@@ -317,6 +317,26 @@ enum { DAN_INFLATE_OK = 0, DAN_INFLATE_E_HEADER = 1, DAN_INFLATE_E_BLOCK = 2, DA
 int dan_inflate_device(const void* src, const uint64_t* offsets, const uint32_t* lengths, int n, void* dst, uint64_t slot_bytes,
                        int32_t* status, void* stream);
 
+/* Batched zlib deflate on the device, the inverse of dan_inflate_device: input i is src[i * slot_bytes, (i + 1) * slot_bytes) and
+ * becomes one complete RFC 1950 stream (2-byte header, deflate blocks, big-endian Adler-32) in dst[i * B, (i + 1) * B) with
+ * B = dan_deflate_bound(slot_bytes) = slot_bytes + 5 * max(1, ceil(slot_bytes / 65535)) + 6, the size of the stored-block encoding (an
+ * empty input still needs one block). lengths[i] receives the stream's length and status[i] DAN_DEFLATE_OK. The streams hold
+ * dynamic-Huffman blocks, or stored blocks when those would be larger; no write leaves its slot. Distances stay within 32768 bytes and
+ * the input, matches within 258 bytes. A stream's bytes depend only on its input: not on n, its position in the batch, the launch or
+ * the device. All pointers are DEVICE pointers; asynchronous on `stream`. Before any launch: DAN_E_INVALID for n < 0 or a null
+ * pointer, DAN_E_UNSUPPORTED for slot_bytes above DAN_DEFLATE_MAX_SLOT (the input must fit in one CTA's shared memory). n = 0
+ * launches nothing. */
+#define DAN_DEFLATE_MAX_SLOT 131072
+enum { DAN_DEFLATE_OK = 0, DAN_DEFLATE_E_UNSUPPORTED = 1 };
+size_t dan_deflate_bound(uint64_t slot_bytes);
+int dan_deflate_device(const void* src, int n, uint64_t slot_bytes, void* dst, uint32_t* lengths, int32_t* status, void* stream);
+
+/* Packs the n streams of dan_deflate_device back to back: offsets (DEVICE, n + 1 u64) receives the exclusive prefix sum of lengths
+ * (offsets[n] = the total) and stream i moves from its slot in `slots` (stride dan_deflate_bound(slot_bytes)) to dst + offsets[i]. dst
+ * (DEVICE) must hold the total; n * dan_deflate_bound(slot_bytes) bytes always do. Asynchronous on `stream`, so that a single
+ * cudaMemcpyAsync of offsets[n] bytes carries only the compressed bytes to the host. */
+int dan_deflate_compact(const void* slots, const uint32_t* lengths, int n, uint64_t slot_bytes, void* dst, uint64_t* offsets, void* stream);
+
 /* Device decode of compressed records. `staging` (pinned HOST, dan_decode_compressed_records_device_staging_bytes(capacity,
  * max_stream_bytes) bytes) holds, for the n records of the call, at offsets that depend only on n (each region 16-byte aligned):
  *   [n sidecars][n u64 stream offsets][n u32 stream lengths][n dan_record_header][n*201 ref masks][n*201 var masks][streams]
