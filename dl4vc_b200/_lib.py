@@ -23,10 +23,12 @@ LIB_PATH = os.environ.get("DAN_B200_LIB") or os.path.join(os.path.dirname(os.pat
 EXPORTED_SYMBOLS = (
     "dan_last_error", "dan_version", "dan_model_create", "dan_model_destroy", "dan_model_load_weights",
     "dan_model_set_pass_candidates", "dan_workspace_bytes", "dan_forward", "dan_workspace_bytes_host",
-    "dan_forward_host", "dan_scores", "dan_genotype_calls", "dan_format_vcf_info", "dan_make_mask_vectors", "dan_encode", "dan_encode_bf16", "dan_model_set_flags", "dan_model_bf16_route", "dan_train_tape_bytes", "dan_train_forward", "dan_backward", "dan_losses", "dan_close_table_update", "dan_decode_records", "dan_decode_record_headers", "dan_decode_records_device", "dan_decode_records_device_workspace_bytes", "dan_record_sidecars", "dan_decode_sidecar_headers", "dan_inflate_device", "dan_deflate_bound", "dan_deflate_device", "dan_deflate_compact", "dan_decode_compressed_records_device", "dan_decode_compressed_records_device_staging_bytes", "dan_decode_compressed_records_device_workspace_bytes", "dan_debug_fc_input", "dan_last_launch_count", "dan_measure_fma_tflops",
+    "dan_forward_host", "dan_scores", "dan_genotype_calls", "dan_format_vcf_info", "dan_make_mask_vectors", "dan_encode", "dan_encode_bf16", "dan_model_set_flags", "dan_model_bf16_route", "dan_train_tape_bytes", "dan_train_forward", "dan_backward", "dan_losses", "dan_close_table_update", "dan_decode_records", "dan_decode_record_headers", "dan_record_sidecars", "dan_decode_sidecar_headers", "dan_inflate_device", "dan_deflate_bound", "dan_deflate_device", "dan_deflate_compact", "dan_decode_layout", "dan_decode_records_device", "dan_debug_fc_input", "dan_last_launch_count", "dan_measure_fma_tflops",
     "dan_profile_enable", "dan_profile_read", "dan_profile_class_name",
 )
 PROF_NUM_CLASSES = 4
+RECORDS_RAW = 0         # DAN_RECORDS_RAW / DAN_RECORDS_ZLIB: the two record formats of dan_decode_records_device
+RECORDS_ZLIB = 1
 
 
 class DanLibraryError(RuntimeError):
@@ -44,6 +46,21 @@ class DanConfigC(C.Structure):
         ("num_fc", C.c_int32), ("fc_sizes", C.c_int32 * DAN_MAX_FC),
         ("num_reads", C.c_int32), ("read_len", C.c_int32),
     ]
+
+
+class DanFeederConfigC(C.Structure):
+    _fields_ = [("max_reads", C.c_int32), ("store_max_reads", C.c_int32), ("use_q_scores", C.c_int32), ("use_strands", C.c_int32),
+                ("keep_candidate_af", C.c_int32), ("seed", C.c_uint64)]
+
+
+class DanRecordBatchC(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("reads", "q_scores", "strands", "ref", "ref_masks", "var_masks", "label", "num_reads", "is_snp",
+                                          "var_type", "allele_freq", "coverage", "var_base_enum", "var_ref_enum", "blacklist", "status")]
+
+
+class DanStagingLayoutC(C.Structure):
+    _fields_ = [(n, C.c_size_t) for n in ("sidecars", "records", "stream_offsets", "stream_lengths", "headers", "ref_masks", "var_masks",
+                                          "streams", "staging_bytes", "workspace_bytes")]
 
 
 _PL = C.c_void_p * DAN_MAX_LAYERS
@@ -103,6 +120,18 @@ def load_library(path: str | None = None):
     lib.dan_genotype_calls.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp]
     lib.dan_format_vcf_info.argtypes = [vp, i32, vp, sz]
     lib.dan_make_mask_vectors.argtypes = [vp, vp, vp, i32, vp, vp, vp]
+    cfgp, batchp = C.POINTER(DanFeederConfigC), C.POINTER(DanRecordBatchC)
+    lib.dan_decode_records.argtypes = [vp, sz, vp, i32, cfgp, batchp]
+    lib.dan_decode_record_headers.argtypes = [vp, sz, vp, i32, cfgp, batchp, vp]
+    lib.dan_record_sidecars.argtypes = [vp, sz, i32, vp]
+    lib.dan_decode_sidecar_headers.argtypes = [vp, vp, i32, cfgp, batchp, vp]
+    lib.dan_decode_layout.argtypes = [i32, i32, sz, C.POINTER(DanStagingLayoutC)]
+    lib.dan_decode_records_device.argtypes = [i32, vp, sz, vp, i32, cfgp, batchp, vp, sz, vp, vp]
+    lib.dan_inflate_device.argtypes = [vp, vp, vp, i32, vp, C.c_uint64, vp, vp]
+    lib.dan_deflate_bound.argtypes = [C.c_uint64]
+    lib.dan_deflate_bound.restype = sz
+    lib.dan_deflate_device.argtypes = [vp, i32, C.c_uint64, vp, vp, vp, vp]
+    lib.dan_deflate_compact.argtypes = [vp, vp, i32, C.c_uint64, vp, vp, vp]
     lib.dan_last_launch_count.restype = i32
     lib.dan_measure_fma_tflops.argtypes = [C.c_double, vp]
     lib.dan_measure_fma_tflops.restype = C.c_double

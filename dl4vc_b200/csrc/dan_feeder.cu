@@ -217,36 +217,65 @@ void host_tiles(const uint8_t* rec, const dan_record_header& h, const dan_feeder
   memcpy(out->ref + (size_t)i * kRecP, rec + kOffRefBases, kRecP);
 }
 
-int check_feeder_config(const dan_feeder_config* cfg, int* R, int* S) {
+// The checks every batch entry point starts with: the count, the pointers (`pointers` is false if one is NULL), the record stride
+// and the config, whose read counts go to R / S. Nothing is checked past the count when n == 0.
+int check_batch(int n, bool pointers, const dan_feeder_config* cfg, int* R, int* S, size_t record_stride = DAN_RECORD_BYTES) {
+  if (n < 0) { dan_set_error("negative record count"); return DAN_E_INVALID; }
+  if (n == 0) return DAN_OK;
+  if (!pointers || !cfg) { dan_set_error("null pointer"); return DAN_E_INVALID; }
+  if (record_stride < DAN_RECORD_BYTES) { dan_set_error("record stride %zu below the %d-byte record", record_stride, DAN_RECORD_BYTES); return DAN_E_INVALID; }
   *R = cfg->max_reads; *S = cfg->store_max_reads < kRecRows ? cfg->store_max_reads : kRecRows;
   if (*R < 1 || *R > kRecRows || *S < 1) { dan_set_error("max_reads %d / store_max_reads %d out of range", *R, cfg->store_max_reads); return DAN_E_INVALID; }
   return DAN_OK;
 }
 
+// The header pass over n records, record i read through view(i) and keyed by indices[i]; its masks go to rm / vm + i * 201 and its
+// header to headers[i].
+template <class View>
+int header_passes(View view, const int64_t* indices, int n, const dan_feeder_config* cfg, int R, int S, const dan_record_batch* out,
+                  uint8_t* rm, uint8_t* vm, dan_record_header* headers) {
+  int failed = 0;
+  for (int i = 0; i < n; ++i)
+    if (header_pass(view(i), indices[i], cfg, R, S, out, i, rm + (size_t)i * kRecP, vm + (size_t)i * kRecP, headers + i) != DAN_REC_OK) ++failed;
+  if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
+  return DAN_OK;
+}
+
 // ---- device tile pass ------------------------------------------------------------------------------------------------------------
-// Layout of the device workspace, and of the pinned host staging buffer it is copied from in one piece:
-//   [n records, DAN_RECORD_BYTES apart][pad to 16][n dan_record_header][n*201 ref_masks][n*201 var_masks]
-struct StagingLayout { size_t hdr, rm, vm, total; };
-StagingLayout staging_layout(int n) {
-  StagingLayout l;
-  l.hdr = ((size_t)n * kRecBytes + 15) & ~(size_t)15;
-  l.rm = l.hdr + (size_t)n * sizeof(dan_record_header);
-  l.vm = l.rm + (size_t)n * kRecP;
-  l.total = ((l.vm + (size_t)n * kRecP) + 15) & ~(size_t)15;
+constexpr size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
+
+// The staging layout of include/dan_b200.h. The device workspace holds the n record images (for ZLIB; for RAW they are the copied
+// records region) followed by the staging buffer from the records region on, so every copied region keeps its 16-byte alignment.
+dan_staging_layout staging_layout(int format, int n, size_t max_stream_bytes) {
+  const bool zlib = format == DAN_RECORDS_ZLIB;
+  dan_staging_layout l;
+  size_t at = 0;
+  auto region = [&](size_t bytes) { const size_t o = at; at = align16(at + bytes); return o; };
+  l.sidecars = region(zlib ? (size_t)n * kSideBytes : 0);
+  l.records = region(zlib ? 0 : (size_t)n * kRecBytes);
+  l.stream_offsets = region(zlib ? (size_t)n * 8 : 0);
+  l.stream_lengths = region(zlib ? (size_t)n * 4 : 0);
+  l.headers = region((size_t)n * sizeof(dan_record_header));
+  l.ref_masks = region((size_t)n * kRecP);
+  l.var_masks = region((size_t)n * kRecP);
+  l.streams = at;
+  l.staging_bytes = align16(l.streams + (zlib ? (size_t)n * max_stream_bytes : 0));
+  l.workspace_bytes = (zlib ? align16((size_t)n * kRecBytes) : 0) + l.staging_bytes - l.records;
   return l;
 }
 
 constexpr int kTileThreads = 256;
 
-// grid (n, 3): block (i, t) writes tile t (0 reads, 1 q-scores, 2 strands) of record i. The chosen rows are gathered into a
-// [position][read] image of the tile in shared memory (zero past num_rows, or everywhere for a tile the config leaves unused),
-// placed at the output address's offset mod 16, so the tile leaves shared memory in aligned 16-byte stores; only the bytes before
-// the first and after the last 16-byte boundary of the record's range go out one by one. Blocks of tile 0 also copy ref_bases
-// and the header pass's masks.
-__global__ void decode_tiles_kernel(const uint8_t* __restrict__ ws, int n, int R, int use_q, int use_s,
-                                                                      size_t hdr_off, size_t rm_off, size_t vm_off,
-                                                                      uint8_t* __restrict__ reads, uint8_t* __restrict__ q, uint8_t* __restrict__ sd,
-                                                                      uint8_t* __restrict__ ref, uint8_t* __restrict__ ref_masks, uint8_t* __restrict__ var_masks) {
+// grid (n, 3): block (i, t) writes tile t (0 reads, 1 q-scores, 2 strands) of record i from its image images + i * DAN_RECORD_BYTES.
+// The chosen rows are gathered into a [position][read] image of the tile in shared memory (zero past num_rows, or everywhere for a
+// tile the config leaves unused), placed at the output address's offset mod 16, so the tile leaves shared memory in aligned 16-byte
+// stores; only the bytes before the first and after the last 16-byte boundary of the record's range go out one by one. Blocks of
+// tile 0 also copy ref_bases and the header pass's masks. A record whose inflate_status (NULL for raw records) is not DAN_INFLATE_OK
+// decodes to nothing: no tile rows and all-zero masks (its image, ref_bases included, is already all zero).
+__global__ void decode_tiles_kernel(const uint8_t* __restrict__ images, const dan_record_header* __restrict__ headers,
+                                    const uint8_t* __restrict__ rm, const uint8_t* __restrict__ vm, const int32_t* __restrict__ inflate_status,
+                                    int R, int use_q, int use_s, uint8_t* __restrict__ reads, uint8_t* __restrict__ q, uint8_t* __restrict__ sd,
+                                    uint8_t* __restrict__ ref, uint8_t* __restrict__ ref_masks, uint8_t* __restrict__ var_masks) {
   extern __shared__ uint4 tile_smem[];
   __shared__ uint8_t rows[kRecRows];
   const int i = blockIdx.x, t = blockIdx.y, tid = threadIdx.x;
@@ -256,14 +285,16 @@ __global__ void decode_tiles_kernel(const uint8_t* __restrict__ ws, int n, int R
   uint8_t* dst = dst_base + (size_t)i * T;
   const int mis = (int)((uintptr_t)dst & 15);
   uint8_t* s = reinterpret_cast<uint8_t*>(tile_smem) + mis;
-  const dan_record_header* h = reinterpret_cast<const dan_record_header*>(ws + hdr_off) + i;
-  const int num_rows = h->num_rows;
+  const dan_record_header* h = headers + i;
+  const bool ok = !inflate_status || inflate_status[i] == DAN_INFLATE_OK;
+  const int num_rows = ok ? h->num_rows : 0;
   const bool fill = t == 0 || (t == 1 && use_q) || (t == 2 && use_s);
   for (int k = tid; k < (T + 31) / 16; k += kTileThreads) tile_smem[k] = make_uint4(0, 0, 0, 0);
   if (tid < num_rows) rows[tid] = h->rows[tid];
   __syncthreads();
+  const uint8_t* rec = images + (size_t)i * kRecBytes;
   if (fill) {
-    const uint8_t* src = ws + (size_t)i * kRecBytes + (t == 0 ? kOffSingle : t == 1 ? kOffQ : kOffStrand);
+    const uint8_t* src = rec + (t == 0 ? kOffSingle : t == 1 ? kOffQ : kOffStrand);
     for (int e = tid; e < num_rows * kRecP; e += kTileThreads) {        // consecutive threads read consecutive bytes of one stored row
       const int j = e / kRecP, p = e - j * kRecP;
       s[p * R + j] = src[rows[j] * kRecP + p];
@@ -278,38 +309,13 @@ __global__ void decode_tiles_kernel(const uint8_t* __restrict__ ws, int n, int R
   for (int k = tid; k < chunks; k += kTileThreads) d4[k] = s4[k];
   for (int k = head + chunks * 16 + tid; k < T; k += kTileThreads) dst[k] = s[k];
   if (t == 0) {
-    const uint8_t* rb = ws + (size_t)i * kRecBytes + kOffRefBases;
+    const size_t o = (size_t)i * kRecP;
     for (int k = tid; k < kRecP; k += kTileThreads) {
-      ref[(size_t)i * kRecP + k] = rb[k];
-      ref_masks[(size_t)i * kRecP + k] = ws[rm_off + (size_t)i * kRecP + k];
-      var_masks[(size_t)i * kRecP + k] = ws[vm_off + (size_t)i * kRecP + k];
+      ref[o + k] = rec[kOffRefBases + k];
+      ref_masks[o + k] = ok ? rm[o + k] : 0;
+      var_masks[o + k] = ok ? vm[o + k] : 0;
     }
   }
-}
-
-// ---- compressed records ------------------------------------------------------------------------------------------------------------
-// Staging layout for n records (include/dan_b200.h). The device workspace holds [n record images][pad to 16] followed by the staging
-// buffer from `off` on, so every offset past `off` keeps its 16-byte alignment.
-struct CompressedLayout { size_t side, off, len, hdr, rm, vm, data; };
-CompressedLayout compressed_layout(int n) {
-  CompressedLayout l;
-  l.side = 0;
-  l.off = ((size_t)n * kSideBytes + 15) & ~(size_t)15;
-  l.len = l.off + (size_t)n * 8;
-  l.hdr = (l.len + (size_t)n * 4 + 15) & ~(size_t)15;
-  l.rm = l.hdr + (size_t)n * sizeof(dan_record_header);
-  l.vm = l.rm + (size_t)n * kRecP;
-  l.data = (l.vm + (size_t)n * kRecP + 15) & ~(size_t)15;
-  return l;
-}
-size_t images_bytes(int n) { return ((size_t)n * kRecBytes + 15) & ~(size_t)15; }
-
-// a record whose stream failed decodes to nothing: no tile rows (its image is already all zero) and all-zero masks
-__global__ void clear_failed_kernel(uint8_t* ws, int n, size_t hdr_off, size_t rm_off, size_t vm_off, const int32_t* __restrict__ inflate_status) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n || inflate_status[i] == DAN_INFLATE_OK) return;
-  reinterpret_cast<dan_record_header*>(ws + hdr_off)[i].num_rows = 0;
-  for (int k = 0; k < kRecP; ++k) { ws[rm_off + (size_t)i * kRecP + k] = 0; ws[vm_off + (size_t)i * kRecP + k] = 0; }
 }
 
 }  // namespace
@@ -317,69 +323,23 @@ __global__ void clear_failed_kernel(uint8_t* ws, int n, size_t hdr_off, size_t r
 extern "C" {
 
 int dan_decode_records(const void* records, size_t record_stride, const int64_t* indices, int n, const dan_feeder_config* cfg, const dan_record_batch* out) {
-  if (n < 0) { dan_set_error("negative record count"); return DAN_E_INVALID; }
-  if (n == 0) return DAN_OK;
-  if (!records || !indices || !cfg || !out || !out->reads || !out->ref || !out->ref_masks || !out->var_masks) { dan_set_error("null pointer"); return DAN_E_INVALID; }
-  if (record_stride < DAN_RECORD_BYTES) { dan_set_error("record stride %zu below the %d-byte record", record_stride, DAN_RECORD_BYTES); return DAN_E_INVALID; }
   int R, S;
-  if (check_feeder_config(cfg, &R, &S) != DAN_OK) return DAN_E_INVALID;
-  int failed = 0;
-  for (int i = 0; i < n; ++i) {
-    const uint8_t* rec = static_cast<const uint8_t*>(records) + (size_t)indices[i] * record_stride;
-    dan_record_header h;
-    if (header_pass(raw_view(rec), indices[i], cfg, R, S, out, i, out->ref_masks + (size_t)i * kRecP, out->var_masks + (size_t)i * kRecP, &h) != DAN_REC_OK) ++failed;
-    host_tiles(rec, h, cfg, R, out, i);
-  }
-  if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
-  return DAN_OK;
+  const int rc = check_batch(n, records && indices && out && out->reads && out->ref && out->ref_masks && out->var_masks, cfg, &R, &S, record_stride);
+  if (rc != DAN_OK || n == 0) return rc;
+  const auto rec = [&](int i) { return static_cast<const uint8_t*>(records) + (size_t)indices[i] * record_stride; };
+  std::vector<dan_record_header> h(n);
+  const int failed = header_passes([&](int i) { return raw_view(rec(i)); }, indices, n, cfg, R, S, out, out->ref_masks, out->var_masks, h.data());
+  for (int i = 0; i < n; ++i) host_tiles(rec(i), h[i], cfg, R, out, i);
+  return failed;
 }
 
 int dan_decode_record_headers(const void* records, size_t record_stride, const int64_t* indices, int n, const dan_feeder_config* cfg,
                               const dan_record_batch* out, dan_record_header* headers) {
-  if (n < 0) { dan_set_error("negative record count"); return DAN_E_INVALID; }
-  if (n == 0) return DAN_OK;
-  if (!records || !indices || !cfg || !out || !out->ref_masks || !out->var_masks || !headers) { dan_set_error("null pointer"); return DAN_E_INVALID; }
-  if (record_stride < DAN_RECORD_BYTES) { dan_set_error("record stride %zu below the %d-byte record", record_stride, DAN_RECORD_BYTES); return DAN_E_INVALID; }
   int R, S;
-  if (check_feeder_config(cfg, &R, &S) != DAN_OK) return DAN_E_INVALID;
-  int failed = 0;
-  for (int i = 0; i < n; ++i) {
-    const uint8_t* rec = static_cast<const uint8_t*>(records) + (size_t)indices[i] * record_stride;
-    if (header_pass(raw_view(rec), indices[i], cfg, R, S, out, i, out->ref_masks + (size_t)i * kRecP, out->var_masks + (size_t)i * kRecP, headers + i) != DAN_REC_OK) ++failed;
-  }
-  if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
-  return DAN_OK;
-}
-
-size_t dan_decode_records_device_workspace_bytes(int n, const dan_feeder_config* cfg) {
-  int R, S;
-  if (n < 0 || !cfg || check_feeder_config(cfg, &R, &S) != DAN_OK) return 0;
-  return staging_layout(n).total;
-}
-
-int dan_decode_records_device(void* staging, size_t staging_bytes, const int64_t* indices, int n, const dan_feeder_config* cfg,
-                              const dan_record_batch* out, void* workspace, size_t workspace_bytes, void* stream) {
-  if (n < 0) { dan_set_error("negative record count"); return DAN_E_INVALID; }
-  if (n == 0) return DAN_OK;
-  if (!staging || !indices || !cfg || !out || !out->reads || !out->ref || !out->ref_masks || !out->var_masks || !workspace) { dan_set_error("null pointer"); return DAN_E_INVALID; }
-  int R, S;
-  if (check_feeder_config(cfg, &R, &S) != DAN_OK) return DAN_E_INVALID;
-  const StagingLayout l = staging_layout(n);
-  if (staging_bytes < l.total) { dan_set_error("staging buffer of %zu bytes is below the %zu bytes %d records need", staging_bytes, l.total, n); return DAN_E_WORKSPACE; }
-  if (workspace_bytes < l.total) { dan_set_error("device workspace of %zu bytes is below the %zu bytes %d records need", workspace_bytes, l.total, n); return DAN_E_WORKSPACE; }
-  uint8_t* st = static_cast<uint8_t*>(staging);
-  dan_record_header* hdr = reinterpret_cast<dan_record_header*>(st + l.hdr);
-  int failed = 0;
-  for (int i = 0; i < n; ++i)
-    if (header_pass(raw_view(st + (size_t)i * kRecBytes), indices[i], cfg, R, S, out, i, st + l.rm + (size_t)i * kRecP, st + l.vm + (size_t)i * kRecP, hdr + i) != DAN_REC_OK) ++failed;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  DAN_CUDA_TRY(cudaMemcpyAsync(workspace, staging, l.total, cudaMemcpyHostToDevice, s));
-  const int smem = ((kRecP * R + 31) / 16) * 16;
-  decode_tiles_kernel<<<dim3(n, 3), kTileThreads, smem, s>>>(static_cast<const uint8_t*>(workspace), n, R, cfg->use_q_scores != 0, cfg->use_strands != 0,
-                                                             l.hdr, l.rm, l.vm, out->reads, out->q_scores, out->strands, out->ref, out->ref_masks, out->var_masks);
-  DAN_CUDA_TRY(cudaGetLastError());
-  if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
-  return DAN_OK;
+  const int rc = check_batch(n, records && indices && out && out->ref_masks && out->var_masks && headers, cfg, &R, &S, record_stride);
+  if (rc != DAN_OK || n == 0) return rc;
+  return header_passes([&](int i) { return raw_view(static_cast<const uint8_t*>(records) + (size_t)indices[i] * record_stride); }, indices, n, cfg,
+                       R, S, out, out->ref_masks, out->var_masks, headers);
 }
 
 int dan_record_sidecars(const void* records, size_t record_stride, int n, void* out) {
@@ -405,77 +365,70 @@ int dan_record_sidecars(const void* records, size_t record_stride, int n, void* 
 
 int dan_decode_sidecar_headers(const void* sidecars, const int64_t* indices, int n, const dan_feeder_config* cfg, const dan_record_batch* out,
                                dan_record_header* headers) {
-  if (n < 0) { dan_set_error("negative record count"); return DAN_E_INVALID; }
-  if (n == 0) return DAN_OK;
-  if (!sidecars || !indices || !cfg || !out || !out->ref_masks || !out->var_masks || !headers) { dan_set_error("null pointer"); return DAN_E_INVALID; }
   int R, S;
-  if (check_feeder_config(cfg, &R, &S) != DAN_OK) return DAN_E_INVALID;
-  int failed = 0;
-  for (int i = 0; i < n; ++i) {
-    const uint8_t* sc = static_cast<const uint8_t*>(sidecars) + (size_t)indices[i] * kSideBytes;
-    if (header_pass(sidecar_view(sc), indices[i], cfg, R, S, out, i, out->ref_masks + (size_t)i * kRecP, out->var_masks + (size_t)i * kRecP, headers + i) != DAN_REC_OK) ++failed;
-  }
-  if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
+  const int rc = check_batch(n, sidecars && indices && out && out->ref_masks && out->var_masks && headers, cfg, &R, &S);
+  if (rc != DAN_OK || n == 0) return rc;
+  return header_passes([&](int i) { return sidecar_view(static_cast<const uint8_t*>(sidecars) + (size_t)indices[i] * kSideBytes); }, indices, n,
+                       cfg, R, S, out, out->ref_masks, out->var_masks, headers);
+}
+
+int dan_decode_layout(int format, int n, size_t max_stream_bytes, dan_staging_layout* out) {
+  if (format != DAN_RECORDS_RAW && format != DAN_RECORDS_ZLIB) { dan_set_error("unknown record format %d", format); return DAN_E_INVALID; }
+  if (n < 0) { dan_set_error("negative record count"); return DAN_E_INVALID; }
+  if (!out) { dan_set_error("null pointer"); return DAN_E_INVALID; }
+  *out = staging_layout(format, n, max_stream_bytes);
   return DAN_OK;
 }
 
-size_t dan_decode_compressed_records_device_staging_bytes(int n, size_t max_stream_bytes) {
-  if (n < 0) return 0;
-  return (compressed_layout(n).data + (size_t)n * max_stream_bytes + 15) & ~(size_t)15;
-}
-
-size_t dan_decode_compressed_records_device_workspace_bytes(int n, size_t max_stream_bytes) {
-  if (n < 0) return 0;
-  return images_bytes(n) + dan_decode_compressed_records_device_staging_bytes(n, max_stream_bytes) - compressed_layout(n).off;
-}
-
-int dan_decode_compressed_records_device(void* staging, size_t staging_bytes, const int64_t* indices, int n, const dan_feeder_config* cfg,
-                                         const dan_record_batch* out, void* workspace, size_t workspace_bytes, int32_t* inflate_status,
-                                         void* stream) {
-  if (n < 0) { dan_set_error("negative record count"); return DAN_E_INVALID; }
-  if (n == 0) return DAN_OK;
-  if (!staging || !indices || !cfg || !out || !out->reads || !out->ref || !out->ref_masks || !out->var_masks || !workspace || !inflate_status) {
-    dan_set_error("null pointer"); return DAN_E_INVALID;
-  }
+int dan_decode_records_device(int format, void* staging, size_t staging_bytes, const int64_t* indices, int n, const dan_feeder_config* cfg,
+                              const dan_record_batch* out, void* workspace, size_t workspace_bytes, int32_t* inflate_status, void* stream) {
+  if (format != DAN_RECORDS_RAW && format != DAN_RECORDS_ZLIB) { dan_set_error("unknown record format %d", format); return DAN_E_INVALID; }
+  const bool zlib = format == DAN_RECORDS_ZLIB;
   int R, S;
-  if (check_feeder_config(cfg, &R, &S) != DAN_OK) return DAN_E_INVALID;
-  const CompressedLayout l = compressed_layout(n);
-  if (staging_bytes < l.data) { dan_set_error("staging buffer of %zu bytes is below the %zu bytes %d records need", staging_bytes, l.data, n); return DAN_E_WORKSPACE; }
+  int rc = check_batch(n, staging && indices && out && out->reads && out->ref && out->ref_masks && out->var_masks && workspace && (!zlib || inflate_status),
+                       cfg, &R, &S);
+  if (rc != DAN_OK || n == 0) return rc;
+  const dan_staging_layout l = staging_layout(format, n, 0);      // the streams region is what the caller's buffer has room for
+  if (staging_bytes < l.staging_bytes) {
+    dan_set_error("staging buffer of %zu bytes is below the %zu bytes %d records need", staging_bytes, l.staging_bytes, n); return DAN_E_WORKSPACE;
+  }
   uint8_t* st = static_cast<uint8_t*>(staging);
-  const uint64_t* off = reinterpret_cast<const uint64_t*>(st + l.off);
-  const uint32_t* len = reinterpret_cast<const uint32_t*>(st + l.len);
-  const size_t cap = staging_bytes - l.data;
-  size_t used = 0;
-  for (int i = 0; i < n; ++i) {
+  const uint64_t* off = reinterpret_cast<const uint64_t*>(st + l.stream_offsets);
+  const uint32_t* len = reinterpret_cast<const uint32_t*>(st + l.stream_lengths);
+  const size_t cap = staging_bytes - l.streams;
+  size_t used = 0;                                                // bytes of the streams region the copy carries
+  for (int i = 0; zlib && i < n; ++i) {
     if (off[i] > cap || len[i] > cap - off[i]) {
       dan_set_error("stream %d ([%llu, +%u)) leaves the %zu-byte streams region of the staging buffer", i, (unsigned long long)off[i], len[i], cap);
       return DAN_E_INVALID;
     }
     if (off[i] + len[i] > used) used = off[i] + len[i];
   }
-  const size_t copy = l.data - l.off + used, images = images_bytes(n);
-  if (workspace_bytes < images + copy) { dan_set_error("device workspace of %zu bytes is below the %zu bytes %d records need", workspace_bytes, images + copy, n); return DAN_E_WORKSPACE; }
-  dan_record_header* hdr = reinterpret_cast<dan_record_header*>(st + l.hdr);
-  int failed = 0;
-  for (int i = 0; i < n; ++i)
-    if (header_pass(sidecar_view(st + l.side + (size_t)i * kSideBytes), indices[i], cfg, R, S, out, i, st + l.rm + (size_t)i * kRecP,
-                    st + l.vm + (size_t)i * kRecP, hdr + i) != DAN_REC_OK) ++failed;
+  if (workspace_bytes < l.workspace_bytes + used) {
+    dan_set_error("device workspace of %zu bytes is below the %zu bytes %d records need", workspace_bytes, l.workspace_bytes + used, n);
+    return DAN_E_WORKSPACE;
+  }
+  dan_record_header* hdr = reinterpret_cast<dan_record_header*>(st + l.headers);
+  const int failed = zlib ? header_passes([&](int i) { return sidecar_view(st + l.sidecars + (size_t)i * kSideBytes); }, indices, n, cfg, R, S, out,
+                                          st + l.ref_masks, st + l.var_masks, hdr)
+                          : header_passes([&](int i) { return raw_view(st + l.records + (size_t)i * kRecBytes); }, indices, n, cfg, R, S, out,
+                                          st + l.ref_masks, st + l.var_masks, hdr);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
-  const size_t base = images - l.off;                 // workspace offset of staging byte b (b >= l.off) is base + b
-  DAN_CUDA_TRY(cudaMemcpyAsync(ws + images, st + l.off, copy, cudaMemcpyHostToDevice, s));
-  const int rc = dan_inflate_launch(ws + base + l.data, reinterpret_cast<const uint64_t*>(ws + base + l.off),
-                                    reinterpret_cast<const uint32_t*>(ws + base + l.len), n, ws, kRecBytes, inflate_status, s);
-  if (rc != DAN_OK) return rc;
-  clear_failed_kernel<<<(n + 127) / 128, 128, 0, s>>>(ws, n, base + l.hdr, base + l.rm, base + l.vm, inflate_status);
-  DAN_CUDA_TRY(cudaGetLastError());
+  uint8_t* ws = static_cast<uint8_t*>(workspace);               // the record images
+  uint8_t* dev = ws + (l.workspace_bytes - l.staging_bytes);    // the device copy of staging byte b (b >= l.records) is dev + b
+  DAN_CUDA_TRY(cudaMemcpyAsync(dev + l.records, st + l.records, l.streams - l.records + used, cudaMemcpyHostToDevice, s));
+  if (zlib) {
+    rc = dan_inflate_launch(dev + l.streams, reinterpret_cast<const uint64_t*>(dev + l.stream_offsets),
+                            reinterpret_cast<const uint32_t*>(dev + l.stream_lengths), n, ws, kRecBytes, inflate_status, s);
+    if (rc != DAN_OK) return rc;
+  }
   const int smem = ((kRecP * R + 31) / 16) * 16;
-  decode_tiles_kernel<<<dim3(n, 3), kTileThreads, smem, s>>>(ws, n, R, cfg->use_q_scores != 0, cfg->use_strands != 0, base + l.hdr, base + l.rm,
-                                                             base + l.vm, out->reads, out->q_scores, out->strands, out->ref, out->ref_masks,
-                                                             out->var_masks);
+  decode_tiles_kernel<<<dim3(n, 3), kTileThreads, smem, s>>>(ws, reinterpret_cast<const dan_record_header*>(dev + l.headers), dev + l.ref_masks,
+                                                             dev + l.var_masks, zlib ? inflate_status : nullptr, R, cfg->use_q_scores != 0,
+                                                             cfg->use_strands != 0, out->reads, out->q_scores, out->strands, out->ref,
+                                                             out->ref_masks, out->var_masks);
   DAN_CUDA_TRY(cudaGetLastError());
-  if (failed) { dan_set_error("%d of %d records raise in the reference loader (see status[])", failed, n); return DAN_E_INVALID; }
-  return DAN_OK;
+  return failed;
 }
 
 }  // extern "C"

@@ -326,9 +326,7 @@ def record_sidecars(raw) -> np.ndarray:
     from . import _lib
     raw = np.ascontiguousarray(raw)
     out = np.empty((len(raw), SIDECAR_BYTES), np.uint8)
-    lib = _lib.load_library()
-    lib.dan_record_sidecars.argtypes = [C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]
-    _lib.check(lib.dan_record_sidecars(raw.ctypes.data, RECORD_BYTES, len(raw), out.ctypes.data), "dan_record_sidecars")
+    _lib.check(_lib.load_library().dan_record_sidecars(raw.ctypes.data, RECORD_BYTES, len(raw), out.ctypes.data), "dan_record_sidecars")
     return out
 
 
@@ -441,7 +439,7 @@ def _device_deflate_chunks(source, dev, depth=2):
     dan_deflate_compact, one D2H copy of lengths and status; once those have landed, one D2H copy of exactly the compressed bytes.
     `depth` slots rotate, so reading chunk k + 1 and cutting its sidecars on the host overlap the GPU work of chunk k."""
     from . import _lib
-    lib = _deflate_lib()
+    lib = _lib.load_library()
     stream, copy_stream = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
     slots, first = [], 0
 
@@ -586,28 +584,17 @@ def inflate_device(src: torch.Tensor, offsets: torch.Tensor, lengths: torch.Tens
         raise ValueError("a stream lies outside src")
     dst = torch.empty((n, slot_bytes), dtype=torch.uint8, device=src.device)
     status = torch.empty(n, dtype=torch.int32, device=src.device)
-    lib = _lib.load_library()
-    lib.dan_inflate_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
     with torch.cuda.device(src.device):
         st = (stream if stream is not None else torch.cuda.current_stream(src.device)).cuda_stream
-        _lib.check(lib.dan_inflate_device(src.data_ptr(), off.data_ptr(), ln.data_ptr(), n, dst.data_ptr(), slot_bytes, status.data_ptr(), st),
+        _lib.check(_lib.load_library().dan_inflate_device(src.data_ptr(), off.data_ptr(), ln.data_ptr(), n, dst.data_ptr(), slot_bytes, status.data_ptr(), st),
                    "dan_inflate_device")
     return dst, status
 
 
-def _deflate_lib():
-    from . import _lib
-    lib = _lib.load_library()
-    lib.dan_deflate_bound.argtypes = [C.c_uint64]
-    lib.dan_deflate_bound.restype = C.c_size_t
-    lib.dan_deflate_device.argtypes = [C.c_void_p, C.c_int, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
-    lib.dan_deflate_compact.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]
-    return lib
-
-
 def deflate_bound(slot_bytes: int) -> int:
     """Bytes of one output slot of dan_deflate_device: the stored-block encoding of slot_bytes, which no stream exceeds."""
-    return int(_deflate_lib().dan_deflate_bound(slot_bytes))
+    from . import _lib
+    return int(_lib.load_library().dan_deflate_bound(slot_bytes))
 
 
 def deflate_device(src: torch.Tensor, stream=None):
@@ -620,7 +607,7 @@ def deflate_device(src: torch.Tensor, stream=None):
         raise ValueError("src must be a 2-D (n, slot) CUDA uint8 tensor")
     src = src.contiguous()
     n, slot = src.shape
-    lib = _deflate_lib()
+    lib = _lib.load_library()
     bound = int(lib.dan_deflate_bound(slot))
     dev = src.device
     slots = torch.empty(n * bound, dtype=torch.uint8, device=dev)
@@ -640,17 +627,8 @@ def deflate_device(src: torch.Tensor, stream=None):
     return packed[:total], offsets[:n], lengths, status
 
 
-class _FeederCfg(C.Structure):
-    _fields_ = [("max_reads", C.c_int32), ("store_max_reads", C.c_int32), ("use_q_scores", C.c_int32), ("use_strands", C.c_int32),
-                ("keep_candidate_af", C.c_int32), ("seed", C.c_uint64)]
-
-
 _SCALARS = (("label", np.uint8), ("num_reads", np.int32), ("is_snp", np.uint8), ("var_type", np.int32), ("allele_freq", np.float32),
             ("coverage", np.int32), ("var_base_enum", np.int32), ("var_ref_enum", np.int32), ("blacklist", np.uint8), ("status", np.int32))
-
-
-class _RecordBatchC(C.Structure):
-    _fields_ = [(n, C.c_void_p) for n in ("reads", "q_scores", "strands", "ref", "ref_masks", "var_masks")] + [(n, C.c_void_p) for n, _ in _SCALARS]
 
 
 # dan_record_header (include/dan_b200.h): tile column j < num_rows of every tile is stored row rows[j]
@@ -660,7 +638,8 @@ assert RECORD_HEADER_DTYPE.itemsize == 216
 
 
 def _feeder_cfg(max_reads, store_max_reads, use_q_scores, use_strands, keep_candidate_af, seed):
-    return _FeederCfg(max_reads, store_max_reads, int(use_q_scores), int(use_strands), int(keep_candidate_af), int(seed))
+    from . import _lib
+    return _lib.DanFeederConfigC(max_reads, store_max_reads, int(use_q_scores), int(use_strands), int(keep_candidate_af), int(seed))
 
 
 def _record_indices(records, indices):
@@ -675,8 +654,9 @@ def _scalars(n):
 
 
 def _batch_struct(tiles, sc):
+    from . import _lib
     ptr = lambda t: None if t is None else t.data_ptr() if isinstance(t, torch.Tensor) else t.ctypes.data
-    return _RecordBatchC(*[ptr(t) for t in tiles], *[sc[k].ctypes.data for k, _ in _SCALARS])
+    return _lib.DanRecordBatchC(*[ptr(t) for t in tiles], *[sc[k].ctypes.data for k, _ in _SCALARS])
 
 
 def _raise_failed(idx, sc):
@@ -700,7 +680,6 @@ def decode_records(records: RecordFile, indices, batch: HostBatch | None = None,
     sc = _scalars(n)
     out = _batch_struct((batch.reads, batch.q, batch.strands, batch.ref, batch.ref_masks, batch.var_masks), sc)
     cfg = _feeder_cfg(max_reads, store_max_reads, use_q_scores, use_strands, keep_candidate_af, seed)
-    lib.dan_decode_records.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(_FeederCfg), C.POINTER(_RecordBatchC)]
     rc = lib.dan_decode_records(records.raw.ctypes.data, RECORD_BYTES, idx.ctypes.data, n, C.byref(cfg), C.byref(out))
     batch.size = n
     batch.meta = [(bytes(records.field(int(i), "name")).decode(), bytes(records.field(int(i), "vcfrec")).decode()) for i in idx]
@@ -724,71 +703,43 @@ def decode_record_headers(records, indices, use_q_scores=True, use_strands=True,
     out = _batch_struct((None, None, None, None, rm, vm), sc)
     cfg = _feeder_cfg(max_reads, store_max_reads, use_q_scores, use_strands, keep_candidate_af, seed)
     if isinstance(records, CompressedRecordFile):
-        lib.dan_decode_sidecar_headers.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(_FeederCfg), C.POINTER(_RecordBatchC), C.c_void_p]
         rc = lib.dan_decode_sidecar_headers(records.sidecars.ctypes.data, idx.ctypes.data, n, C.byref(cfg), C.byref(out), hdr.ctypes.data)
     else:
-        lib.dan_decode_record_headers.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(_FeederCfg), C.POINTER(_RecordBatchC), C.c_void_p]
         rc = lib.dan_decode_record_headers(records.raw.ctypes.data, RECORD_BYTES, idx.ctypes.data, n, C.byref(cfg), C.byref(out), hdr.ctypes.data)
     if rc < 0 and not sc["status"].any():
         _lib.check(rc, "dan_decode_record_headers")
     return hdr, sc, rm, vm
 
 
-def _staging_bytes(n, max_reads):
+def _decode_layout(fmt, n, max_stream_bytes=0):
+    """The staging layout of n records of format fmt (_lib.RECORDS_RAW / RECORDS_ZLIB), as dan_decode_layout reports it."""
     from . import _lib
-    lib = _lib.load_library()
-    lib.dan_decode_records_device_workspace_bytes.argtypes = [C.c_int, C.POINTER(_FeederCfg)]
-    lib.dan_decode_records_device_workspace_bytes.restype = C.c_size_t
-    cfg = _feeder_cfg(max_reads, 200, 1, 1, 0, 0)
-    need = int(lib.dan_decode_records_device_workspace_bytes(n, C.byref(cfg)))
-    if need == 0 and n > 0:
-        raise ValueError(f"max_reads {max_reads} out of range 1..200")
-    return need
-
-
-def _compressed_sizes(n, max_stream_bytes):
-    from . import _lib
-    lib = _lib.load_library()
-    for f in (lib.dan_decode_compressed_records_device_staging_bytes, lib.dan_decode_compressed_records_device_workspace_bytes):
-        f.argtypes, f.restype = [C.c_int, C.c_size_t], C.c_size_t
-    return (int(lib.dan_decode_compressed_records_device_staging_bytes(n, max_stream_bytes)),
-            int(lib.dan_decode_compressed_records_device_workspace_bytes(n, max_stream_bytes)))
-
-
-def _compressed_layout(n):
-    """Offsets of the compressed staging regions for n records, as dan_decode_compressed_records_device lays them out
-    (include/dan_b200.h): sidecars, stream offsets, stream lengths, headers, ref masks, var masks, streams."""
-    a16 = lambda x: (x + 15) & ~15
-    off = a16(n * SIDECAR_BYTES)
-    ln = off + 8 * n
-    hdr = a16(ln + 4 * n)
-    rm = hdr + n * RECORD_HEADER_DTYPE.itemsize
-    vm = rm + n * 201
-    return dict(side=0, off=off, len=ln, hdr=hdr, rm=rm, vm=vm, data=a16(vm + n * 201))
+    lay = _lib.DanStagingLayoutC()
+    _lib.check(_lib.load_library().dan_decode_layout(fmt, n, max_stream_bytes, C.byref(lay)), "dan_decode_layout")
+    return lay
 
 
 class DeviceBatch:
     """Decoded batch on the GPU (`dan_decode_records_device`): device uint8 tiles in the layout dan_forward takes, the pinned host
-    staging buffer the raw records are read into, and the device workspace they are copied to. The decoded tiles exist only on
-    the device.
+    staging buffer the records are read into, and the device workspace they are copied to. The decoded tiles exist only on the
+    device.
 
-    With `max_stream_bytes` (a CompressedRecordFile's largest stream) the batch decodes compressed records
-    (`dan_decode_compressed_records_device`): the staging buffer holds sidecars and zlib streams, sized for `capacity` streams of
-    that size, and `inflate_status` is a device int32 tensor with each record's inflate status (INFLATE_STATUS) of the last decode."""
+    With `max_stream_bytes` (a CompressedRecordFile's largest stream) the batch decodes compressed records: the staging buffer holds
+    sidecars and zlib streams, sized for `capacity` streams of that size, and `inflate_status` is a device int32 tensor with each
+    record's inflate status (INFLATE_STATUS) of the last decode."""
 
     def __init__(self, capacity: int, num_reads: int = 100, device=None, read_len: int = 201, max_stream_bytes: int | None = None):
+        from . import _lib
+        if not 1 <= num_reads <= 200:
+            raise ValueError(f"max_reads {num_reads} out of range 1..200")
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.capacity, self.num_reads, self.device, self.size = capacity, num_reads, dev, 0
         self.max_stream_bytes = max_stream_bytes
-        if max_stream_bytes is None:
-            nbytes = wbytes = _staging_bytes(capacity, num_reads)
-            self.inflate_status = None
-        else:
-            _staging_bytes(capacity, num_reads)          # checks max_reads
-            nbytes, wbytes = _compressed_sizes(capacity, max_stream_bytes)
-            self.inflate_status = torch.zeros(capacity, dtype=torch.int32, device=dev)
-        self.staging = torch.empty(nbytes, dtype=torch.uint8).pin_memory()
-        self.workspace = torch.empty(wbytes, dtype=torch.uint8, device=dev)
+        self.format = _lib.RECORDS_RAW if max_stream_bytes is None else _lib.RECORDS_ZLIB
+        lay = _decode_layout(self.format, capacity, max_stream_bytes or 0)
+        self.inflate_status = None if max_stream_bytes is None else torch.zeros(capacity, dtype=torch.int32, device=dev)
+        self.staging = torch.empty(lay.staging_bytes, dtype=torch.uint8).pin_memory()
+        self.workspace = torch.empty(lay.workspace_bytes, dtype=torch.uint8, device=dev)
         mk = lambda *shape: torch.empty(shape, dtype=torch.uint8, device=dev)
         self.reads, self.q, self.strands = (mk(capacity, read_len, num_reads) for _ in range(3))
         self.ref, self.ref_masks, self.var_masks = (mk(capacity, read_len) for _ in range(3))
@@ -801,7 +752,7 @@ class DeviceBatch:
     def headers(self):
         """Header-pass descriptors of the last decode (RECORD_HEADER_DTYPE, a view into the staging buffer)."""
         n = self.size
-        off = (n * RECORD_BYTES + 15) & ~15 if self.max_stream_bytes is None else _compressed_layout(n)["hdr"]
+        off = _decode_layout(self.format, n).headers
         return self.staging.numpy()[off:off + n * RECORD_HEADER_DTYPE.itemsize].view(RECORD_HEADER_DTYPE)
 
 
@@ -815,11 +766,10 @@ def decode_records_device(records, indices, batch: DeviceBatch | None = None, us
 
     `records` is a RecordFile, a CompressedRecordFile or a path (opened by its magic). For a compressed file the zlib streams are
     staged instead of the records, the header pass runs over the sidecars, and the records are inflated on the GPU before the tile
-    pass (`dan_decode_compressed_records_device`); the batch must be a compressed DeviceBatch (default: one sized for the file). The
-    call does not wait for the inflate: `batch.inflate_status` holds each record's status once `stream` has passed the call, and a
-    record whose stream is corrupt decodes to all-zero tiles and masks."""
+    pass; the batch must be a compressed DeviceBatch (default: one sized for the file). The call does not wait for the inflate:
+    `batch.inflate_status` holds each record's status once `stream` has passed the call, and a record whose stream is corrupt
+    decodes to all-zero tiles and masks."""
     from . import _lib
-    lib = _lib.load_library()
     if not isinstance(records, (RecordFile, CompressedRecordFile)):
         records = open_record_file(records)
     compressed = isinstance(records, CompressedRecordFile)
@@ -833,36 +783,35 @@ def decode_records_device(records, indices, batch: DeviceBatch | None = None, us
         raise ValueError(f"batch holds {batch.num_reads} reads per candidate, max_reads is {max_reads}")
     if compressed != (batch.max_stream_bytes is not None):
         raise ValueError("a compressed record file needs a DeviceBatch with max_stream_bytes, a raw one a DeviceBatch without")
+    lay = _decode_layout(batch.format, n)
+    st = batch.staging.numpy()
     if compressed:
-        return _decode_compressed_device(records, idx, batch, _feeder_cfg(max_reads, store_max_reads, use_q_scores, use_strands,
-                                                                           keep_candidate_af, seed), strict, stream)
-    if n and np.all(np.diff(idx) == 1):
-        records.read_block(int(idx[0]), n, batch.staging)
+        st[lay.sidecars:lay.sidecars + n * SIDECAR_BYTES].reshape(n, SIDECAR_BYTES)[:] = records.sidecars[idx]
+        st[lay.stream_offsets:lay.stream_offsets + 8 * n].view(np.uint64)[:] = _stage_streams(records, idx, st[lay.streams:])
+        st[lay.stream_lengths:lay.stream_lengths + 4 * n].view(np.uint32)[:] = records.lengths[idx]
+        rows = st[lay.sidecars:lay.sidecars + n * SIDECAR_BYTES].view(SIDECAR_DTYPE)
     else:
-        records.gather(idx, batch.staging)
+        if n and np.all(np.diff(idx) == 1):
+            records.read_block(int(idx[0]), n, st[lay.records:])
+        else:
+            records.gather(idx, st[lay.records:])
+        rows = st[lay.records:lay.records + n * RECORD_BYTES].view(RECORD_DTYPE)
     sc = _scalars(n)
     out = _batch_struct((batch.reads, batch.q, batch.strands, batch.ref, batch.ref_masks, batch.var_masks), sc)
     cfg = _feeder_cfg(max_reads, store_max_reads, use_q_scores, use_strands, keep_candidate_af, seed)
-    lib.dan_decode_records_device.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(_FeederCfg), C.POINTER(_RecordBatchC),
-                                              C.c_void_p, C.c_size_t, C.c_void_p]
     with torch.cuda.device(batch.device):
-        st = (stream if stream is not None else torch.cuda.current_stream(batch.device)).cuda_stream
-        rc = lib.dan_decode_records_device(batch.staging.data_ptr(), batch.staging.numel(), idx.ctypes.data, n, C.byref(cfg), C.byref(out),
-                                           batch.workspace.data_ptr(), batch.workspace.numel(), st)
+        s = (stream if stream is not None else torch.cuda.current_stream(batch.device)).cuda_stream
+        rc = _lib.load_library().dan_decode_records_device(batch.format, batch.staging.data_ptr(), batch.staging.numel(), idx.ctypes.data, n,
+                                                           C.byref(cfg), C.byref(out), batch.workspace.data_ptr(), batch.workspace.numel(),
+                                                           None if batch.inflate_status is None else batch.inflate_status.data_ptr(), s)
     batch.size = n
-    raw = batch.staging.numpy()[:n * RECORD_BYTES].reshape(n, RECORD_BYTES)
-    names = raw[:, :16].copy().view("S16").reshape(-1)
-    vcfrecs = raw[:, _VCF_OFFSET:_VCF_OFFSET + 128].copy().view("S128").reshape(-1)
-    batch.meta = [(a.decode(), b.decode()) for a, b in zip(names.tolist(), vcfrecs.tolist())]
+    batch.meta = [(a.decode(), b.decode()) for a, b in zip(rows["name"].tolist(), rows["vcfrec"].tolist())]
     if rc == -1 and sc["status"].any():          # DAN_E_INVALID with per-record status: records the reference raises on
         if strict:
             _raise_failed(idx, sc)
     else:
         _lib.check(rc, "dan_decode_records_device")
     return batch, sc
-
-
-_VCF_OFFSET = RECORD_DTYPE.fields["vcfrec"][1]
 
 
 def _stage_streams(rf: CompressedRecordFile, idx, dst: np.ndarray):
@@ -883,35 +832,6 @@ def _stage_streams(rf: CompressedRecordFile, idx, dst: np.ndarray):
         o = int(rf.offsets[i])
         dst[int(pos[k]):int(pos[k + 1])] = rf.data[o:o + int(rf.lengths[i])]
     return pos[:n]
-
-
-def _decode_compressed_device(rf: CompressedRecordFile, idx, batch: DeviceBatch, cfg, strict, stream):
-    from . import _lib
-    lib = _lib.load_library()
-    n = len(idx)
-    lay = _compressed_layout(n)
-    st = batch.staging.numpy()
-    st[:n * SIDECAR_BYTES].reshape(n, SIDECAR_BYTES)[:] = rf.sidecars[idx]
-    st[lay["off"]:lay["off"] + 8 * n].view(np.uint64)[:] = _stage_streams(rf, idx, st[lay["data"]:])
-    st[lay["len"]:lay["len"] + 4 * n].view(np.uint32)[:] = rf.lengths[idx]
-    sc = _scalars(n)
-    out = _batch_struct((batch.reads, batch.q, batch.strands, batch.ref, batch.ref_masks, batch.var_masks), sc)
-    lib.dan_decode_compressed_records_device.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(_FeederCfg),
-                                                         C.POINTER(_RecordBatchC), C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]
-    with torch.cuda.device(batch.device):
-        s = (stream if stream is not None else torch.cuda.current_stream(batch.device)).cuda_stream
-        rc = lib.dan_decode_compressed_records_device(batch.staging.data_ptr(), batch.staging.numel(), idx.ctypes.data, n, C.byref(cfg),
-                                                      C.byref(out), batch.workspace.data_ptr(), batch.workspace.numel(),
-                                                      batch.inflate_status.data_ptr(), s)
-    batch.size = n
-    side = st[:n * SIDECAR_BYTES].view(SIDECAR_DTYPE)
-    batch.meta = [(a.decode(), b.decode()) for a, b in zip(side["name"].tolist(), side["vcfrec"].tolist())]
-    if rc == -1 and sc["status"].any():
-        if strict:
-            _raise_failed(idx, sc)
-    else:
-        _lib.check(rc, "dan_decode_compressed_records_device")
-    return batch, sc
 
 
 class _CallSlot:

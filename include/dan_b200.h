@@ -278,18 +278,6 @@ typedef struct dan_record_header {
 int dan_decode_record_headers(const void* records, size_t record_stride, const int64_t* indices, int n, const dan_feeder_config* cfg,
                               const dan_record_batch* out, dan_record_header* headers);
 
-/* Device decode. `staging` is a pinned HOST buffer of dan_decode_records_device_workspace_bytes(n, cfg) bytes whose first
- * n * DAN_RECORD_BYTES bytes hold the n records back to back, record i decoding into candidate i; indices[i] is record i's index in its
- * file, which seeds the read draw exactly as in dan_decode_records. The call runs the header pass on the host, writing the headers and
- * masks into the rest of `staging` and the scalars of `out` (HOST pointers: label .. status, each may be NULL, valid on return), copies
- * the staging buffer to `workspace` (DEVICE, same size) in one cudaMemcpyAsync on `stream` and launches the tile pass there, which
- * writes out->reads / q_scores / strands / ref / ref_masks / var_masks (DEVICE pointers; q_scores / strands may be NULL). Every output
- * equals dan_decode_records' byte for byte. Asynchronous: neither buffer may be reused before the stream has passed this call.
- * DAN_E_WORKSPACE (no copy, no launch) if either buffer is too small; DAN_E_INVALID with per-record status as dan_decode_records. */
-size_t dan_decode_records_device_workspace_bytes(int n, const dan_feeder_config* cfg);
-int dan_decode_records_device(void* staging, size_t staging_bytes, const int64_t* indices, int n, const dan_feeder_config* cfg,
-                              const dan_record_batch* out, void* workspace, size_t workspace_bytes, void* stream);
-
 /* ---- compressed record files ------------------------------------------------------------------------------------------------------
  * File layout (all fields little-endian; written and opened by dl4vc_b200/feeder.py):
  *   header, 64 bytes: magic "DL4VCZR1", u32 version = 1, u32 record_bytes = DAN_RECORD_BYTES, u64 count, u64 index_off,
@@ -337,21 +325,38 @@ int dan_deflate_device(const void* src, int n, uint64_t slot_bytes, void* dst, u
  * cudaMemcpyAsync of offsets[n] bytes carries only the compressed bytes to the host. */
 int dan_deflate_compact(const void* slots, const uint32_t* lengths, int n, uint64_t slot_bytes, void* dst, uint64_t* offsets, void* stream);
 
-/* Device decode of compressed records. `staging` (pinned HOST, dan_decode_compressed_records_device_staging_bytes(capacity,
- * max_stream_bytes) bytes) holds, for the n records of the call, at offsets that depend only on n (each region 16-byte aligned):
- *   [n sidecars][n u64 stream offsets][n u32 stream lengths][n dan_record_header][n*201 ref masks][n*201 var masks][streams]
- * The caller fills the sidecars, the index and the streams (offsets relative to the start of the streams region); the header pass
- * over the sidecars writes the headers and masks. One cudaMemcpyAsync moves everything from the index to the end of the last stream into
- * `workspace` behind n record images; dan_inflate_device fills the images, and the tile pass of dan_decode_records_device runs over
- * them. inflate_status (DEVICE, n int32) receives the inflate status; a record whose stream fails gets all-zero tiles, ref and masks.
- * For records that inflate, every output equals dan_decode_records' on the raw records byte for byte. DAN_E_WORKSPACE (no copy, no
- * launch) if a buffer is too small; DAN_E_INVALID (no copy) if an index entry leaves the streams region, and with per-record status as
- * dan_decode_records. Asynchronous: neither buffer may be reused before the stream has passed this call. */
-size_t dan_decode_compressed_records_device_staging_bytes(int n, size_t max_stream_bytes);
-size_t dan_decode_compressed_records_device_workspace_bytes(int n, size_t max_stream_bytes);
-int dan_decode_compressed_records_device(void* staging, size_t staging_bytes, const int64_t* indices, int n, const dan_feeder_config* cfg,
-                                         const dan_record_batch* out, void* workspace, size_t workspace_bytes, int32_t* inflate_status,
-                                         void* stream);
+/* ---- device decode, of raw (DAN_RECORDS_RAW) or compressed (DAN_RECORDS_ZLIB) records --------------------------------------------
+ * The caller stages the n records of a call in one pinned HOST buffer, at the offsets dan_decode_layout reports. The regions come in
+ * this order, each 16-byte aligned, at offsets that depend only on (format, n); a region the format does not use is empty:
+ *   [sidecars][records][stream offsets][stream lengths][headers][ref masks][var masks][streams]
+ *   RAW:  records  = n records back to back, DAN_RECORD_BYTES apart;
+ *   ZLIB: sidecars = n sidecars, DAN_SIDECAR_BYTES apart; stream offsets / lengths = n u64 / n u32, an offset counting from the
+ *         start of the streams region; streams = room for n streams of up to max_stream_bytes.
+ *   both: headers = n dan_record_header, ref / var masks = n * 201 bytes each, written by the call's header pass.
+ * staging_bytes and workspace_bytes are the sizes of the staging buffer and of the DEVICE workspace for n records (and, for ZLIB, n
+ * streams of max_stream_bytes, so sizes taken for a capacity serve every call of up to that many records). DAN_E_INVALID for an
+ * unknown format or n < 0. */
+enum { DAN_RECORDS_RAW = 0, DAN_RECORDS_ZLIB = 1 };
+typedef struct dan_staging_layout {
+  size_t sidecars, records, stream_offsets, stream_lengths, headers, ref_masks, var_masks, streams;   /* staging offsets */
+  size_t staging_bytes, workspace_bytes;
+} dan_staging_layout;
+int dan_decode_layout(int format, int n, size_t max_stream_bytes, dan_staging_layout* out);
+
+/* Device decode. Record i of the staging buffer decodes into candidate i; indices[i] is its index in its file, which seeds the read
+ * draw exactly as in dan_decode_records. The call runs the header pass on the host (over the records, or over the sidecars for ZLIB),
+ * writing the headers and masks into the staging buffer and the scalars of `out` (HOST pointers: label .. status, each may be NULL,
+ * valid on return). One cudaMemcpyAsync on `stream` moves everything from the records region to the end of the last stream into
+ * `workspace` (DEVICE); for ZLIB, dan_inflate_device then inflates the streams into n record images in the workspace and writes each
+ * record's status to inflate_status (DEVICE, n int32; NULL for RAW). The tile pass then writes out->reads / q_scores / strands / ref /
+ * ref_masks / var_masks (DEVICE pointers; q_scores / strands may be NULL). Every output equals dan_decode_records' on the raw records
+ * byte for byte; a record whose stream fails to inflate gets all-zero tiles, ref and masks.
+ * Before any header pass, copy or launch: DAN_E_INVALID for bad arguments or config, DAN_E_WORKSPACE if the staging buffer is too
+ * small, DAN_E_INVALID if an index entry leaves the streams region, DAN_E_WORKSPACE if the workspace is too small for the streams
+ * actually staged. Records the reference's loader raises on return DAN_E_INVALID with per-record status, as dan_decode_records.
+ * Asynchronous: neither buffer may be reused before the stream has passed this call. */
+int dan_decode_records_device(int format, void* staging, size_t staging_bytes, const int64_t* indices, int n, const dan_feeder_config* cfg,
+                              const dan_record_batch* out, void* workspace, size_t workspace_bytes, int32_t* inflate_status, void* stream);
 
 /* Test hook for the bit-exact integer/encoding work (dl4vc/model.py:450-627,719): writes the conv-1 input in the
  * reference's logical order (batch, Cin, num_reads, read_len) fp32, DEVICE pointer. */

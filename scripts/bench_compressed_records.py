@@ -6,7 +6,7 @@ warm, and reports:
   * the compression ratio and bytes per record;
   * host microseconds per record of the device path's host work (staging copy + header pass + enqueue inside decode_records_device),
     compressed against raw, and the staging copy and the header pass (sidecars against raw records) alone;
-  * H2D bytes per record of one staging copy, computed from the staging layouts and the streams' lengths;
+  * H2D bytes per record of one staging copy, from the staging layout (dan_decode_layout) and the streams' lengths;
   * the inflate kernel alone (dan_inflate_device over one batch's streams already on the device): CUDA events around each launch,
     time per record and output GB/s, and, in a separate torch.profiler pass over the compressed device decode, the device time of
     inflate_kernel, decode_tiles_kernel and the H2D copy per record;
@@ -49,11 +49,11 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("bench_compressed_records.py measures on a CUDA device; none is visible")
     from bench_record_calls import power_limit_w, write_records
+    from dl4vc_b200 import _lib
     from dl4vc_b200.config import prod_config
     from dl4vc_b200.factory import build_model
-    from dl4vc_b200.feeder import (RECORD_BYTES, RECORD_HEADER_DTYPE, CompressedRecordFile, DeviceBatch, RecordFile, _compressed_layout,
-                                   _stage_streams, call_record_file, decode_record_headers, decode_records_device, inflate_device,
-                                   write_compressed_records)
+    from dl4vc_b200.feeder import (RECORD_BYTES, SIDECAR_BYTES, CompressedRecordFile, DeviceBatch, RecordFile, _decode_layout, _stage_streams,
+                                   call_record_file, decode_record_headers, decode_records_device, inflate_device, write_compressed_records)
     from dl4vc_b200.weights import synth_state_dict
 
     dev = torch.device("cuda", 0)
@@ -94,18 +94,24 @@ def main():
                 best = min(best, t)
             return round(best / N * 1e6, 2)
 
-        lay = lambda n: _compressed_layout(n)
+        lay = lambda n: _decode_layout(_lib.RECORDS_ZLIB, n)
+
+        def stage_compressed(s, n):
+            st, L = db_cz.staging.numpy(), lay(n)
+            st[L.sidecars:L.sidecars + n * SIDECAR_BYTES].reshape(n, SIDECAR_BYTES)[:] = cf.sidecars[s:s + n]
+            _stage_streams(cf, np.arange(s, s + n), st[L.streams:])
+
         result["host_us_per_record"] = {
             "device_path_host_work_raw": per_record_us(lambda s, n: decode_records_device(rf, np.arange(s, s + n), db_raw, strict=False)),
             "device_path_host_work_compressed": per_record_us(lambda s, n: decode_records_device(cf, np.arange(s, s + n), db_cz, strict=False)),
             "staging_copy_raw": per_record_us(lambda s, n: rf.read_block(s, n, db_raw.staging)),
-            "staging_copy_compressed": per_record_us(lambda s, n: (db_cz.staging.numpy()[:n * 750].reshape(n, 750).__setitem__(slice(None), cf.sidecars[s:s + n]),
-                                                                   _stage_streams(cf, np.arange(s, s + n), db_cz.staging.numpy()[lay(n)["data"]:]))),
+            "staging_copy_compressed": per_record_us(stage_compressed),
             "header_pass_raw": per_record_us(lambda s, n: decode_record_headers(rf, np.arange(s, s + n))),
             "header_pass_sidecar": per_record_us(lambda s, n: decode_record_headers(cf, np.arange(s, s + n))),
             "timing": "best of --passes passes, host clock around each call, device synchronised between calls"}
-        raw_h2d = sum(((n * RECORD_BYTES + 15) & ~15) + n * (RECORD_HEADER_DTYPE.itemsize + 2 * 201) for _, n in starts)
-        cz_h2d = sum(lay(n)["data"] - lay(n)["off"] + int(cf.lengths[s:s + n].sum()) for s, n in starts)
+        copied = lambda L: L.streams - L.records         # the one H2D copy: from the records region to the streams, plus the used streams
+        raw_h2d = sum(copied(_decode_layout(_lib.RECORDS_RAW, n)) for _, n in starts)
+        cz_h2d = sum(copied(lay(n)) + int(cf.lengths[s:s + n].sum()) for s, n in starts)
         result["h2d_bytes_per_record"] = {"raw": round(raw_h2d / N, 1), "compressed": round(cz_h2d / N, 1), "ratio": round(raw_h2d / cz_h2d, 2)}
 
         # ---- the inflate kernel alone, on one batch's streams resident on the device ----
@@ -140,7 +146,7 @@ def main():
                 for s, n in starts:
                     decode_records_device(cf, np.arange(s, s + n), db_cz, strict=False)
             torch.cuda.synchronize()
-        split = {"inflate_kernel": 0.0, "decode_tiles_kernel": 0.0, "clear_failed_kernel": 0.0, "Memcpy HtoD": 0.0}
+        split = {"inflate_kernel": 0.0, "decode_tiles_kernel": 0.0, "Memcpy HtoD": 0.0}
         for e in prof.key_averages():
             t = getattr(e, "device_time_total", None)
             t = e.cuda_time_total if t is None else t

@@ -63,8 +63,9 @@ def main():
         src = torch.from_numpy(np.array(rf.raw[:B])).to(dev)
         streams, offsets, lengths, status = deflate_device(src)
         assert not status.any().item(), "deflate failed"
-        from dl4vc_b200.feeder import _deflate_lib, deflate_bound
-        lib = _deflate_lib()
+        from dl4vc_b200 import _lib
+        from dl4vc_b200.feeder import deflate_bound
+        lib = _lib.load_library()
         bound = deflate_bound(RECORD_BYTES)
         slots = torch.empty(B * bound, dtype=torch.uint8, device=dev)
         ln, st = torch.empty(B, dtype=torch.int32, device=dev), torch.empty(B, dtype=torch.int32, device=dev)

@@ -91,9 +91,10 @@ def main():
     import torch
     if not torch.cuda.is_available():
         raise SystemExit("bench_record_calls.py measures on a CUDA device; none is visible")
+    from dl4vc_b200 import _lib
     from dl4vc_b200.config import prod_config
     from dl4vc_b200.factory import build_model
-    from dl4vc_b200.feeder import (RECORD_BYTES, DeviceBatch, HostBatch, RecordFile, call_record_file, decode_record_headers,
+    from dl4vc_b200.feeder import (RECORD_BYTES, DeviceBatch, HostBatch, RecordFile, _decode_layout, call_record_file, decode_record_headers,
                                    decode_records, decode_records_device)
     from dl4vc_b200.weights import synth_state_dict
 
@@ -114,7 +115,7 @@ def main():
         # ---- host microseconds per record ----
         hb = HostBatch(B, pin=True)
         db = DeviceBatch(B, device=dev)
-        stage = db.staging
+        stage = db.staging.numpy()[_decode_layout(_lib.RECORDS_RAW, B).records:]
 
         def per_record_us(fn):
             best = float("inf")
@@ -167,10 +168,12 @@ def main():
             elif "Memcpy HtoD" in name:
                 copy += t
         recs = N * args.passes
+        layouts = [_decode_layout(_lib.RECORDS_RAW, n) for _, n in starts]
+        h2d_bytes = args.passes * sum(L.streams - L.records for L in layouts)      # the one H2D copy of each call
         result["device_tile_pass"] = {"copy_plus_kernel_us_per_record_events": round(ev_ms * 1e3 / recs, 3),
                                       "kernel_us_per_record": round(kern / recs, 4), "launches": kcount,
                                       "staging_h2d_us_per_record": round(copy / recs, 3),
-                                      "h2d_gb_per_s": round(recs * db.staging.numel() / B / (copy * 1e3), 1) if copy else None,
+                                      "h2d_gb_per_s": round(h2d_bytes / (copy * 1e3), 1) if copy else None,
                                       "source": "copy_plus_kernel: CUDA events recorded around each call on its stream; kernel / copy split: "
                                                 "torch.profiler CUDA activities over --passes further passes"}
         del prof

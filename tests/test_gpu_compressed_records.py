@@ -105,31 +105,30 @@ def test_malformed_files_raise_on_open(tmp_path):
     assert len(opened(blob)) == 5
 
 
-def test_compressed_device_decode_checks_buffers_before_any_device_work(synth_pair):
+def test_zlib_device_decode_checks_buffers_before_any_device_work(synth_pair):
     """Staging or workspace too small returns DAN_E_WORKSPACE and an index entry outside the streams region DAN_E_INVALID, before
     the header pass, any copy or launch, so these run without a GPU."""
     from dl4vc_b200 import _lib
-    from dl4vc_b200.feeder import _batch_struct, _compressed_layout, _compressed_sizes, _feeder_cfg, _FeederCfg, _RecordBatchC, _scalars
+    from dl4vc_b200.feeder import _batch_struct, _decode_layout, _feeder_cfg, _scalars
     _, cf = synth_pair
     n, m = 3, cf.max_stream_bytes
-    need, ws_need = _compressed_sizes(n, m)
-    lay = _compressed_layout(n)
-    assert need == (lay["data"] + n * m + 15) & ~15 and ws_need == ((n * RECORD_BYTES + 15) & ~15) + need - lay["off"]
+    lay = _decode_layout(_lib.RECORDS_ZLIB, n, m)
+    need = lay.staging_bytes
     staging = np.zeros(need, np.uint8)
-    staging[lay["off"]:lay["off"] + 8 * n].view(np.uint64)[:] = np.arange(n) * m
-    staging[lay["len"]:lay["len"] + 4 * n].view(np.uint32)[:] = m
+    # the last stream ends at the end of the buffer, so the call needs the whole workspace
+    staging[lay.stream_offsets:lay.stream_offsets + 8 * n].view(np.uint64)[:] = need - lay.streams - (n - np.arange(n)) * m
+    staging[lay.stream_lengths:lay.stream_lengths + 4 * n].view(np.uint32)[:] = m
     sc = _scalars(n)
     out = _batch_struct([torch.zeros(1, dtype=torch.uint8) for _ in range(6)], sc)
     cfg, idx = _feeder_cfg(100, 200, 1, 1, 0, 0), np.arange(n, dtype=np.int64)
     ws, status = np.zeros(16, np.uint8), np.zeros(n, np.int32)
     lib = _lib.load_library()
-    f = lib.dan_decode_compressed_records_device
-    f.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(_FeederCfg), C.POINTER(_RecordBatchC), C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]
-    call = lambda sb, wb: f(staging.ctypes.data, sb, idx.ctypes.data, n, C.byref(cfg), C.byref(out), ws.ctypes.data, wb, status.ctypes.data, None)
-    assert call(lay["data"] - 1, ws_need) == -4 and b"staging buffer" in lib.dan_last_error()
-    used = ((n * RECORD_BYTES + 15) & ~15) + lay["data"] - lay["off"] + n * m            # what this call copies behind the images
-    assert call(need, used - 1) == -4 and b"device workspace" in lib.dan_last_error()
-    assert call(need - 16, ws_need) == -1 and b"leaves the" in lib.dan_last_error()      # the last stream no longer fits
+    call = lambda sb, wb, c=cfg: lib.dan_decode_records_device(_lib.RECORDS_ZLIB, staging.ctypes.data, sb, idx.ctypes.data, n, C.byref(c),
+                                                               C.byref(out), ws.ctypes.data, wb, status.ctypes.data, None)
+    assert call(lay.streams - 1, lay.workspace_bytes) == -4 and b"staging buffer" in lib.dan_last_error()
+    assert call(need, lay.workspace_bytes - 1) == -4 and b"device workspace" in lib.dan_last_error()
+    assert call(need - 16, lay.workspace_bytes) == -1 and b"leaves the" in lib.dan_last_error()      # the last stream no longer fits
+    assert call(need, lay.workspace_bytes, _feeder_cfg(201, 200, 1, 1, 0, 0)) == -1 and b"max_reads" in lib.dan_last_error()
     assert not sc["num_reads"].any(), "the header pass must not run before the checks"
 
 

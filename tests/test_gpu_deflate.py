@@ -68,11 +68,12 @@ def test_deflate_device_argument_checks():
             deflate_device(bad)
 
 
-def test_deflate_c_abi_checks_arguments_before_any_launch():
+def test_deflate_entry_points_check_arguments_before_any_launch():
     """n < 0, null pointers and slots beyond the shared-memory capacity fail, and n = 0 succeeds, all without a launch, so these
     run without a GPU."""
-    from dl4vc_b200.feeder import _deflate_lib, deflate_bound
-    lib = _deflate_lib()
+    from dl4vc_b200 import _lib
+    from dl4vc_b200.feeder import deflate_bound
+    lib = _lib.load_library()
     for s in (0, 1, 258, 65535, 65536, 65537, RECORD_BYTES, 131072):
         assert deflate_bound(s) == _bound(s), s
     p = C.c_void_p(16)

@@ -104,11 +104,11 @@ def test_record_blocks_read_and_gather_raw_bytes():
         rf.read_block(0, 9, np.zeros(3 * RECORD_BYTES, np.uint8))
 
 
-def test_device_decode_rejects_bad_arguments_before_any_device_work():
+def test_raw_device_decode_rejects_bad_arguments_before_any_device_work():
     """Out-of-range indices raise in Python; a staging buffer or workspace below the size the call needs returns DAN_E_WORKSPACE
     before any copy or launch, so both checks run without a GPU."""
     from dl4vc_b200 import _lib
-    from dl4vc_b200.feeder import _batch_struct, _feeder_cfg, _FeederCfg, _RecordBatchC, _scalars, _staging_bytes, decode_records_device
+    from dl4vc_b200.feeder import _batch_struct, _decode_layout, _feeder_cfg, _scalars, decode_records_device
     rf = RecordFile(make_records(3, seed=4, noise_rows=False))
     with pytest.raises(IndexError, match="out of range"):
         decode_records_device(rf, [0, 3])
@@ -116,26 +116,52 @@ def test_device_decode_rejects_bad_arguments_before_any_device_work():
         decode_records_device(rf, [-1])
     lib = _lib.load_library()
     n = 3
-    need = _staging_bytes(n, 100)
+    lay = _decode_layout(_lib.RECORDS_RAW, n)
+    need = lay.staging_bytes
     assert need >= n * RECORD_BYTES + n * (216 + 2 * 201)
     staging = np.zeros(need, np.uint8)
-    staging[:n * RECORD_BYTES] = rf.raw.reshape(-1)
+    staging[lay.records:lay.records + n * RECORD_BYTES] = rf.raw.reshape(-1)
     tiles = [torch.zeros(1, dtype=torch.uint8) for _ in range(6)]
     sc = _scalars(n)
     out = _batch_struct(tiles, sc)
     cfg = _feeder_cfg(100, 200, 1, 1, 0, 0)
     idx = np.arange(n, dtype=np.int64)
-    lib.dan_decode_records_device.argtypes = [C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.POINTER(_FeederCfg), C.POINTER(_RecordBatchC),
-                                              C.c_void_p, C.c_size_t, C.c_void_p]
     ws = np.zeros(16, np.uint8)
-    rc = lib.dan_decode_records_device(staging.ctypes.data, need - 1, idx.ctypes.data, n, C.byref(cfg), C.byref(out), ws.ctypes.data, need, None)
-    assert rc == -4 and b"staging buffer" in lib.dan_last_error()
-    rc = lib.dan_decode_records_device(staging.ctypes.data, need, idx.ctypes.data, n, C.byref(cfg), C.byref(out), ws.ctypes.data, need - 16, None)
-    assert rc == -4 and b"device workspace" in lib.dan_last_error()
+    call = lambda c, sb, wb: lib.dan_decode_records_device(_lib.RECORDS_RAW, staging.ctypes.data, sb, idx.ctypes.data, n, C.byref(c), C.byref(out),
+                                                           ws.ctypes.data, wb, None, None)
+    assert call(cfg, need - 1, lay.workspace_bytes) == -4 and b"staging buffer" in lib.dan_last_error()
+    assert call(cfg, need, lay.workspace_bytes - 1) == -4 and b"device workspace" in lib.dan_last_error()
     assert not sc["num_reads"].any(), "the header pass must not run before the size checks"
-    bad = _feeder_cfg(201, 200, 1, 1, 0, 0)
-    rc = lib.dan_decode_records_device(staging.ctypes.data, need, idx.ctypes.data, n, C.byref(bad), C.byref(out), ws.ctypes.data, need, None)
-    assert rc == -1 and b"max_reads" in lib.dan_last_error()
+    assert call(_feeder_cfg(201, 200, 1, 1, 0, 0), need, lay.workspace_bytes) == -1 and b"max_reads" in lib.dan_last_error()
+
+
+@pytest.mark.parametrize("n", [0, 1, 3, 1036])
+def test_decode_layout_regions(n):
+    """dan_decode_layout for both formats: each region 16-byte aligned, disjoint, inside the staging buffer, the streams last; the
+    sidecars before the copied range [records, streams + used streams); the copy carries the records (raw) or the index (compressed),
+    the headers and the masks, and besides them only alignment padding: the parent's packing, which left the two mask regions
+    unaligned, copied at most 32 bytes less, and exactly as many for the 1036-record batches of the benchmarks."""
+    from dl4vc_b200 import _lib
+    from dl4vc_b200.feeder import SIDECAR_BYTES, _decode_layout
+    a16 = lambda x: -(-x // 16) * 16
+    m = 1000
+    for fmt in (_lib.RECORDS_RAW, _lib.RECORDS_ZLIB):
+        z = fmt == _lib.RECORDS_ZLIB
+        lay = _decode_layout(fmt, n, m)
+        sizes = {"sidecars": z * n * SIDECAR_BYTES, "records": (not z) * n * RECORD_BYTES, "stream_offsets": z * 8 * n,
+                 "stream_lengths": z * 4 * n, "headers": 216 * n, "ref_masks": 201 * n, "var_masks": 201 * n, "streams": z * n * m}
+        spans = sorted((getattr(lay, k), getattr(lay, k) + v, k) for k, v in sizes.items())
+        assert all(lo % 16 == 0 for lo, _, _ in spans), spans
+        assert all(hi <= nxt for (_, hi, _), (nxt, _, _) in zip(spans, spans[1:])), spans
+        assert spans[-1][1] <= lay.staging_bytes and lay.streams >= max(hi for _, hi, k in spans if k != "streams")
+        assert lay.sidecars + sizes["sidecars"] <= lay.records
+        copied = [k for lo, hi, k in spans if lay.records <= lo and hi <= lay.streams and hi > lo]
+        assert copied == ([] if n == 0 else ["stream_offsets", "stream_lengths"] if z else ["records"]) + (["headers", "ref_masks", "var_masks"] if n else [])
+        copy = lay.streams - lay.records
+        index = a16(n * SIDECAR_BYTES)
+        before = a16(a16(index + 12 * n) + 618 * n) - index if z else a16(a16(n * RECORD_BYTES) + 618 * n)
+        assert before <= copy <= before + 32 and (n != 1036 or copy == before), (copy, before)
+        assert lay.workspace_bytes == (a16(n * RECORD_BYTES) if z else 0) + lay.staging_bytes - lay.records
 
 
 # ---- GPU: device decode == host decode, byte for byte ----------------------------------------------------------------------------
