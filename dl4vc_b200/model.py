@@ -513,9 +513,10 @@ class Basic2DNet(nn.Module):
                 self._u8(var_masks, dev) if self.use_reads_ref_var_mask else None)
 
     def _choose_removed(self, u8, rm_non_var_reads, rm_var_reads):
-        """Read-removal augmentation (model.py:633-716): per round, at most one read per candidate that agrees with the variant proposal
-        (rm_var_reads) / covers the centre column without agreeing (rm_non_var_reads) is replaced by the empty-read encoding. The
-        reference draws with torch.randperm; here: a uniform draw per candidate among its eligible reads. Returns (B, R) uint8 or None."""
+        """Read-removal augmentation (model.py:633-716): min(rm_var_reads, #eligible) distinct reads per candidate that agree with the
+        variant proposal, and min(rm_non_var_reads, #eligible) distinct reads that cover the centre column without agreeing, are replaced
+        by the empty-read encoding. The reference draws distinct reads with torch.randperm; here each round draws one read per candidate
+        uniformly among its eligible reads that are not yet removed. Returns (B, R) uint8 or None."""
         if not (rm_non_var_reads or rm_var_reads) or not self.use_reads_ref_var_mask:
             return None
         reads, var_masks = u8[0], u8[5]
@@ -525,6 +526,7 @@ class Basic2DNet(nn.Module):
         removed = torch.zeros_like(agree)
         for eligible, rounds in ((agree, int(rm_var_reads)), (has_read & ~agree, int(rm_non_var_reads))):
             for _ in range(rounds):
+                eligible = eligible & ~removed
                 score = torch.rand(eligible.shape, device=eligible.device).masked_fill(~eligible, -1.0)
                 pick = score.argmax(dim=1)
                 hit = eligible.any(dim=1)

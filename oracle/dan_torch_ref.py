@@ -1,10 +1,14 @@
 """ORACLE — the reference's op sequence in any dtype, on CPU or CUDA, in eval or training mode.  TEST INFRASTRUCTURE ONLY.
 
 The same torch library calls as oracle/dan_torch_cpu.py (dl4vc/model.py:450-627 encode, :719-778 conv stack, :824-861 pool /
-highway, :911-958 FC / heads), with three differences that make it a yardstick for the kernels rather than a benchmark baseline:
+highway, :911-958 FC / heads), with these differences that make it a yardstick for the kernels rather than a benchmark baseline:
   * any dtype (float64 for the truth) and any device — on CUDA the caller turns TF32 off (`no_tf32`);
-  * training mode: batch-statistics BatchNorm that updates the running statistics (momentum 0.1), parameters as autograd leaves,
-    Dropout p = 0 (the tests compare against kernels run with dropout off);
+  * training mode: batch-statistics BatchNorm that updates the running statistics (momentum 0.1), parameters as autograd leaves;
+  * the FC trunk's Dropout is the identity unless `dropout` gives p and the keep mask of every site, which the kernels draw from a
+    counter-based hash (`dropout_keep` / `dropout_masks` restate it, so the same masks can be applied here);
+  * `removed` replaces chosen reads by the empty-read encoding of the training kernels' read-removal augmentation, as the port documents
+    it at `encode_channel` (dl4vc_b200/csrc/dan_kernels_common.cuh): token 0 in the read half, the reference half unchanged, the q,
+    strand, ref-agreement, var-agreement and var_len channels zero;
   * the FC input is returned block by block (`fc_blocks`), in the reference's feature order, next to the heads.
 
 Only tests/ import this file; dan_torch_cpu.py stays the bench baseline.
@@ -72,6 +76,33 @@ class _KinkMaxReads(torch.autograd.Function):
         return torch.zeros(ctx.shape, dtype=g.dtype, device=g.device).scatter(2, idx, g), None, None
 
 
+def dropout_keep(p, seed, salt, rows, ld, width):
+    """(rows, width) bool: the elements dropout_kernel (dl4vc_b200/csrc/dan_train.cu) keeps at site `salt` for `seed` and probability
+    `p`, over a row-major activation of leading dimension `ld` (element index b * ld + k). The hash is splitmix64's finaliser in wrapping
+    uint64 arithmetic; an element is dropped when its upper 32 bits fall below min(float32(p) * 2^32, 4294967295.f) truncated to uint32."""
+    i = np.arange(rows, dtype=np.uint64)[:, None] * np.uint64(ld) + np.arange(width, dtype=np.uint64)[None, :]
+    x = np.uint64(seed) ^ (np.uint64(0x9E3779B97F4A7C15) * (i + np.uint64(1))) ^ (np.uint64(salt) << np.uint64(56))
+    x ^= x >> np.uint64(30)
+    x *= np.uint64(0xBF58476D1CE4E5B9)
+    x ^= x >> np.uint64(27)
+    x *= np.uint64(0x94D049BB133111EB)
+    x ^= x >> np.uint64(31)
+    p32 = np.float32(p)
+    if not p32 > 0:
+        return np.ones((rows, width), dtype=bool)
+    # 4294967295.f rounds to 2^32; the device's float-to-uint32 conversion saturates there
+    thr = min(int(min(p32 * np.float32(2.0 ** 32), np.float32(4294967295.0))), 0xFFFFFFFF)
+    return (x >> np.uint64(32)) >= np.uint64(thr)
+
+
+def dropout_masks(cfg: DanConfig, rows, p, seed):
+    """The `dropout` argument of forward for one training step of the kernels: (p, keep masks of sites 0 .. len(layer_sizes)). Site 0 is
+    the FC input (fc_in_features columns of rows padded to a multiple of 16, dan_capi.cu fcInPad), site j the output of FC layer j - 1."""
+    widths = [cfg.fc_in_features] + list(cfg.layer_sizes)
+    lds = [(cfg.fc_in_features + 15) // 16 * 16] + list(cfg.layer_sizes)
+    return p, [dropout_keep(p, seed, j, rows, ld, w) for j, (ld, w) in enumerate(zip(lds, widths))]
+
+
 def fc_blocks(cfg: DanConfig):
     """name -> column slice of the FC input (model.py:838-912), in order: "post_pool" (pool_combine_dimension > 0) or "max" (unless
     skip_final_maxpool) and "mean"; then "hw<l>" per conv layer (concatenated highway, 0-based l) or "hw" (averaged highway)."""
@@ -105,9 +136,14 @@ class RefResult:
     bufs: dict                # name -> BatchNorm running buffer (updated in place in training mode)
 
 
-def forward(cfg: DanConfig, sd, arrays, dtype=torch.float64, device="cpu", train=False, kink_side=None, kink_tol=3e-6) -> RefResult:
+def forward(cfg: DanConfig, sd, arrays, dtype=torch.float64, device="cpu", train=False, kink_side=None, kink_tol=3e-6,
+            removed=None, dropout=None) -> RefResult:
     """The reference's forward over `arrays` = (reads, q_scores, strands, ref, ref_masks, var_masks) (PileupBatch.arrays() order) with
     the weights of state dict `sd`, computed in `dtype` on `device`.
+
+    removed: optional (B, R) bool, reads replaced by the empty-read encoding (module docstring). dropout: optional (p, keep masks), the
+    masks of the nn.Dropout sites of conv2hidden in order (the FC input, then the output of every FC ReLU), each (B, width) bool
+    (dropout_masks); kept values are scaled by 1 / (1 - p).
 
     kink_side 0 / 1: same values, but every ReLU whose input is within kink_tol of zero (relative to its tensor's largest |input|), and
     the read-axis max where the runner-up read is within kink_tol of the maximum, backpropagates as if it sat on the off / on side of the
@@ -121,6 +157,9 @@ def forward(cfg: DanConfig, sd, arrays, dtype=torch.float64, device="cpu", train
     bufs = {k: torch.as_tensor(v).to(dev, dtype).clone() for k, v in sd.items() if "running_" in k}
     reads, q_scores, strands, ref, ref_masks, var_masks = (torch.from_numpy(np.ascontiguousarray(a)).to(dev) for a in arrays)
     reads, ref = reads.long(), ref.long()
+    gone = None if removed is None else torch.as_tensor(np.asarray(removed, dtype=bool)).to(dev)
+    if gone is not None:
+        reads = reads.masked_fill(gone.unsqueeze(1), 0)                                    # token 0: counted as padding
     E, pe = params["embeddings.weight"], torch.as_tensor(sd["pe"]).to(dev, dtype)
     B, P, R = reads.shape
     # ---- encode (model.py:450-627); nn.Embedding(padding_idx=0, scale_grad_by_freq=True) of model.py:143-145 ----
@@ -141,6 +180,9 @@ def forward(cfg: DanConfig, sd, arrays, dtype=torch.float64, device="cpu", train
             nzs.append(nz)
         chans.append(nzs[0].expand(-1, -1, R).to(dtype))                                       # var_len from the REF mask (sic)
         x = torch.cat([x] + [c.unsqueeze(3) for c in chans], dim=3)
+    if gone is not None:                       # every channel behind the two embedding halves is zero on a removed read, var_len too
+        D = E.shape[1]
+        x = torch.cat((x[..., :2 * D], x[..., 2 * D:] * (~gone).to(dtype)[:, None, :, None]), dim=3)
     h = x.permute(0, 3, 2, 1)                                                                  # (B, Cin, R, P), model.py:719
     # ---- conv stack (model.py:728-778) ----
     pool, hw, res_i = None, [], 0
@@ -177,10 +219,16 @@ def forward(cfg: DanConfig, sd, arrays, dtype=torch.float64, device="cpu", train
         hwv = torch.cat(hw, dim=1) if cfg.concat_hw_reads else torch.stack(hw, 0).mean(0)
         pooled = torch.cat((pooled, relu(hwv)), dim=1)
     fc_in = pooled
-    # ---- FC trunk + heads (model.py:911-958); Dropout is the identity (eval, or p = 0) ----
-    xh = fc_in
-    for idx in cfg.fc_indices:
-        xh = relu(F.linear(xh, params[f"conv2hidden.{idx}.weight"], params[f"conv2hidden.{idx}.bias"]))
+    # ---- FC trunk + heads (model.py:911-958); Dropout is the identity unless its masks are given ----
+    if dropout is not None:
+        p, keeps = dropout
+        assert len(keeps) == len(cfg.fc_indices) + 1, "one keep mask per Dropout site"
+        drop = lambda z, j: z * (torch.as_tensor(np.asarray(keeps[j], dtype=bool)).to(dev, dtype) / (1.0 - p))
+    else:
+        drop = lambda z, j: z
+    xh = drop(fc_in, 0)
+    for j, idx in enumerate(cfg.fc_indices):
+        xh = drop(relu(F.linear(xh, params[f"conv2hidden.{idx}.weight"], params[f"conv2hidden.{idx}.bias"])), j + 1)
     outs = [F.linear(xh, params[n + ".weight"], params[n + ".bias"]) for n in HEAD_NAMES]
     outs[2] = torch.sigmoid(outs[2])
     outs[3] = F.leaky_relu(outs[3], 0.01)
@@ -188,20 +236,20 @@ def forward(cfg: DanConfig, sd, arrays, dtype=torch.float64, device="cpu", train
     return RefResult(torch.cat(outs, dim=1), fc_in, blocks, params, bufs)
 
 
-def train_reference(cfg: DanConfig, sd, arrays, dtype, dev, kink_side=None):
-    """Training-mode forward (batch-statistics BatchNorm with running-statistics update, dropout 0) under torch autograd. Returns heads,
-    {name: leaf parameter} and {name: updated running buffer}."""
-    r = forward(cfg, sd, arrays, dtype=dtype, device=dev, train=True, kink_side=kink_side)
+def train_reference(cfg: DanConfig, sd, arrays, dtype, dev, kink_side=None, removed=None, dropout=None):
+    """Training-mode forward (batch-statistics BatchNorm with running-statistics update; dropout and read removal as forward takes them)
+    under torch autograd. Returns heads, {name: leaf parameter} and {name: updated running buffer}."""
+    r = forward(cfg, sd, arrays, dtype=dtype, device=dev, train=True, kink_side=kink_side, removed=removed, dropout=dropout)
     return r.heads, r.params, r.bufs
 
 
-def kink_bound(cfg: DanConfig, sd, arrays, dheads, dev):
+def kink_bound(cfg: DanConfig, sd, arrays, dheads, dev, removed=None, dropout=None):
     """name -> |grad(kink_side=1) - grad(kink_side=0)| in float64: how much the gradient of each parameter moves when the ReLUs and
     read-axis maxima that sit within rounding distance of their kink switch sides. A single such unit that an fp32 forward puts on the
     other side than float64 does moves a gradient tensor by exactly this much, which no arithmetic accuracy bounds."""
     g = []
     for side in (0, 1):
-        heads, params, _ = train_reference(cfg, sd, arrays, torch.float64, dev, kink_side=side)
+        heads, params, _ = train_reference(cfg, sd, arrays, torch.float64, dev, kink_side=side, removed=removed, dropout=dropout)
         (heads * dheads.to(heads.device, torch.float64)).sum().backward()
         g.append({k: v.grad for k, v in params.items() if v.grad is not None})
     return {k: (g[1][k] - g[0][k]).abs().cpu().numpy() for k in g[0]}

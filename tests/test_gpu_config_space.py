@@ -269,32 +269,34 @@ def _sampled(a, above=200_000, stride=97):
     return a.reshape(-1)[::stride] if a.size > above else a
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("name,cfg", TRAIN_CASES, ids=[c[0] for c in TRAIN_CASES])
-def test_training_step_matches_float64_autograd(name, cfg):
-    cfg = dataclasses.replace(cfg, hidden_dropout=0.0)          # the reference runs without dropout
-    seed = sum(map(ord, name))
-    sd = synth_state_dict(cfg, seed=seed)
-    arrays = tuple(a[[0, 1, 3, 5]] for a in _batch(cfg.num_reads, seed + 1))       # 2 Poisson, 1 full, 1 empty
-    B = len(arrays[0])
-    cw = np.random.default_rng(seed + 2).standard_normal((B, 27)).astype(np.float32)
+def _train_reference(cfg, sd, arrays, cw, removed=None, dropout=None):
+    """One training step of oracle/dan_torch_ref.py on the GPU (TF32 off) with d(loss)/d(heads) = cw: {dtype: (heads, gradients, running
+    buffers)} for float64 and float32, and the kink bound of every gradient. removed / dropout: as dan_torch_ref.forward takes them."""
     ref = {}
     with dan_torch_ref.no_tf32():
         for dtype in (torch.float64, torch.float32):
-            heads, params, bufs = dan_torch_ref.train_reference(cfg, sd, arrays, dtype, "cuda")
+            heads, params, bufs = dan_torch_ref.train_reference(cfg, sd, arrays, dtype, "cuda", removed=removed, dropout=dropout)
             (heads * torch.from_numpy(cw).to(heads.device, dtype)).sum().backward()
             grads = {k: v.grad.cpu().numpy() for k, v in params.items() if v.grad is not None}
             ref[dtype] = (heads.detach().cpu().numpy(), grads, {k: v.cpu().numpy() for k, v in bufs.items()})
-        kink = dan_torch_ref.kink_bound(cfg, sd, arrays, torch.from_numpy(cw), "cuda")
-    want_heads, want_grads, want_bufs = ref[torch.float64]
+        kink = dan_torch_ref.kink_bound(cfg, sd, arrays, torch.from_numpy(cw), "cuda", removed=removed, dropout=dropout)
+    return ref, kink
 
-    model = build_model(cfg, sd, precision="fp32").train()
+
+def _train_step(model, arrays, cw, **kw):
+    """One training step of the kernels through model(...) with d(loss)/d(heads) = cw; kw: rm_non_var_reads / rm_var_reads."""
     r, q, s, rf, rm, vm = (t.long() for t in _tensors(arrays))
-    dummy = torch.zeros(B, dtype=torch.long)
-    out = model(r, rf, q, s, dummy, dummy, dummy, dummy, rm, vm)
+    dummy = torch.zeros(len(arrays[0]), dtype=torch.long)
+    out = model(r, rf, q, s, dummy, dummy, dummy, dummy, rm, vm, **kw)
     heads = torch.cat([o.reshape(o.shape[0], -1) for o in out[:6]], dim=1)
     (heads * torch.from_numpy(cw).to(heads.device)).sum().backward()
-    assert rel_err(heads.detach().cpu().numpy(), want_heads) < FP32_TOL, "training-mode forward"
+    return heads.detach().cpu().numpy()
+
+
+def _check_train_step(name, model, heads, ref, kink):
+    """The heads, every gradient tensor and the running statistics of `model` after _train_step against _train_reference."""
+    want_heads, want_grads, want_bufs = ref[torch.float64]
+    assert rel_err(heads, want_heads) < FP32_TOL, "training-mode forward"
 
     # The gradient is discontinuous where a ReLU input or the read-axis max sits at its kink: a unit within rounding distance of it can
     # land on either side in fp32 and move a gradient tensor by 1e-2 of its maximum (measured: with 21 reads the kernels' layer-4 bottleneck
@@ -322,6 +324,19 @@ def test_training_step_matches_float64_autograd(name, cfg):
     for bname, b in model.named_buffers():
         if "running_" in bname:
             np.testing.assert_allclose(b.detach().cpu().numpy(), want_bufs[bname], rtol=2e-5, atol=1e-6, err_msg=bname)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("name,cfg", TRAIN_CASES, ids=[c[0] for c in TRAIN_CASES])
+def test_training_step_matches_float64_autograd(name, cfg):
+    cfg = dataclasses.replace(cfg, hidden_dropout=0.0)          # dropout: tests/test_gpu_train_dropout_removal.py
+    seed = sum(map(ord, name))
+    sd = synth_state_dict(cfg, seed=seed)
+    arrays = tuple(a[[0, 1, 3, 5]] for a in _batch(cfg.num_reads, seed + 1))       # 2 Poisson, 1 full, 1 empty
+    cw = np.random.default_rng(seed + 2).standard_normal((len(arrays[0]), 27)).astype(np.float32)
+    ref, kink = _train_reference(cfg, sd, arrays, cw)
+    model = build_model(cfg, sd, precision="fp32").train()
+    _check_train_step(name, model, _train_step(model, arrays, cw), ref, kink)
 
 
 @pytest.mark.gpu
