@@ -23,7 +23,7 @@ LIB_PATH = os.environ.get("DAN_B200_LIB") or os.path.join(os.path.dirname(os.pat
 EXPORTED_SYMBOLS = (
     "dan_last_error", "dan_version", "dan_model_create", "dan_model_destroy", "dan_model_load_weights",
     "dan_model_set_pass_candidates", "dan_workspace_bytes", "dan_forward", "dan_workspace_bytes_host",
-    "dan_forward_host", "dan_scores", "dan_genotype_calls", "dan_format_vcf_info", "dan_make_mask_vectors", "dan_encode", "dan_encode_bf16", "dan_model_set_flags", "dan_model_bf16_route", "dan_train_tape_bytes", "dan_train_forward", "dan_backward", "dan_losses", "dan_close_table_update", "dan_decode_records", "dan_decode_record_headers", "dan_record_sidecars", "dan_decode_sidecar_headers", "dan_inflate_device", "dan_deflate_bound", "dan_deflate_device", "dan_deflate_compact", "dan_decode_layout", "dan_decode_records_device", "dan_debug_fc_input", "dan_last_launch_count", "dan_measure_fma_tflops",
+    "dan_forward_host", "dan_scores", "dan_genotype_calls", "dan_format_vcf_info", "dan_make_mask_vectors", "dan_encode", "dan_encode_bf16", "dan_model_set_flags", "dan_model_bf16_route", "dan_train_tape_bytes", "dan_train_forward", "dan_backward", "dan_losses", "dan_close_table_update", "dan_decode_records", "dan_decode_record_headers", "dan_record_sidecars", "dan_decode_sidecar_headers", "dan_inflate_device", "dan_deflate_bound", "dan_deflate_device", "dan_deflate_compact", "dan_bgzf_compress_device", "dan_bgzf_compact", "dan_decode_layout", "dan_decode_records_device", "dan_debug_fc_input", "dan_last_launch_count", "dan_measure_fma_tflops",
     "dan_profile_enable", "dan_profile_read", "dan_profile_class_name",
 )
 PROF_NUM_CLASSES = 4
@@ -132,6 +132,8 @@ def load_library(path: str | None = None):
     lib.dan_deflate_bound.restype = sz
     lib.dan_deflate_device.argtypes = [vp, i32, C.c_uint64, vp, vp, vp, vp]
     lib.dan_deflate_compact.argtypes = [vp, vp, i32, C.c_uint64, vp, vp, vp]
+    lib.dan_bgzf_compress_device.argtypes = [vp, C.c_uint64, vp, vp, vp, vp]
+    lib.dan_bgzf_compact.argtypes = [vp, vp, i32, vp, vp, vp]
     lib.dan_last_launch_count.restype = i32
     lib.dan_measure_fma_tflops.argtypes = [C.c_double, vp]
     lib.dan_measure_fma_tflops.restype = C.c_double

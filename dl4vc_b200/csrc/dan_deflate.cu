@@ -1,5 +1,6 @@
 // dan_deflate.cu — batched zlib (RFC 1950 / 1951) deflate on the GPU: n inputs of slot_bytes each into n complete zlib streams, the
-// inverse of dan_inflate.cu.
+// inverse of dan_inflate.cu; and the same deflate in BGZF framing (gzip members, RFC 1952, of <= 64 KB with the BC extra subfield):
+// a buffer cut as bgzip cuts it, into 65280-byte pieces and a shorter last one, each piece one block with a CRC-32 and ISIZE.
 //
 // One CTA of 1024 threads per input. The input sits whole in shared memory beside a 2^14-entry hash table of 4-byte prefixes. The
 // CTA walks the input in steps of 1024 positions, one position per thread:
@@ -17,7 +18,8 @@
 // blocks; otherwise the second pass repeats the same matches and parse and writes the bits: a block-wide exclusive scan of the
 // tokens' bit counts places each token, every thread ORs its bits into a shared-memory window, and the window's whole bytes go to
 // the output slot after every step. Nothing depends on float arithmetic, atomic order or the batch, so a stream's bytes depend only
-// on its input.
+// on its input. The two containers differ only around the deflate blocks: the header, and an Adler-32 (chunk parts summed) or a CRC-32
+// (chunk CRCs combined pairwise in a fixed tree), computed by the same one-chunk-per-thread split.
 #include <cstdint>
 #include <cuda_runtime.h>
 #include "dan_internal.h"
@@ -56,6 +58,7 @@ struct Smem {
   uint16_t cl_code[19];
   uint32_t warp_sum[32];
   uint64_t adler_a[32], adler_b[32];
+  uint32_t crc_part[32], crc_len[32];                // CRC-32 of each warp's chunks and their length
   uint64_t total_bits;
   uint32_t carry, wbit, outpos, nrle, nlit, ndist;
 };
@@ -391,19 +394,29 @@ __device__ void deflate_pass(Smem& sm, uint32_t n, uint8_t* out, uint32_t cap) {
   }
 }
 
-__global__ void __launch_bounds__(kThreads, 1) deflate_kernel(const uint8_t* __restrict__ src, uint64_t slot_bytes, uint8_t* __restrict__ dst,
-                                                             uint64_t bound, uint32_t* __restrict__ lengths, int32_t* __restrict__ status) {
+// The container around the deflate blocks: a zlib stream (2-byte header, big-endian Adler-32) or a BGZF block (18-byte gzip header with
+// the BC subfield, little-endian CRC-32 and ISIZE).
+enum class Container { kZlib, kBgzf };
+
+// CTA i compresses src[i * in_stride, min((i + 1) * in_stride, in_total)) into dst + i * out_stride. The stream is written as stored
+// blocks when the deflate blocks would be longer, so out_stride >= the stored size of in_stride bytes keeps every write in the slot.
+template <Container kC>
+__global__ void __launch_bounds__(kThreads, 1) deflate_kernel(const uint8_t* __restrict__ src, uint64_t in_stride, uint64_t in_total,
+                                                             uint8_t* __restrict__ dst, uint64_t out_stride, uint32_t* __restrict__ lengths,
+                                                             int32_t* __restrict__ status) {
+  constexpr uint32_t kHead = kC == Container::kZlib ? 2 : 18, kTail = kC == Container::kZlib ? 4 : 8;
   extern __shared__ __align__(16) uint8_t smem_raw[];
   Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const uint64_t i = blockIdx.x;
-  if (slot_bytes > kMaxSlot) {                       // the launcher refuses these; kept so that no write can leave shared memory
+  if (in_stride > kMaxSlot) {                        // the launchers refuse these; kept so that no write can leave shared memory
     if (tid == 0) { lengths[i] = 0; status[i] = DAN_DEFLATE_E_UNSUPPORTED; }
     return;
   }
-  const uint32_t n = (uint32_t)slot_bytes;
-  const uint8_t* in_g = src + i * slot_bytes;
-  uint8_t* out = dst + i * bound;
+  const uint32_t n = (uint32_t)min(in_stride, in_total - i * in_stride);
+  const uint8_t* in_g = src + i * in_stride;
+  uint8_t* out = dst + i * out_stride;
+  uint8_t* body = out + (kHead - 2);                 // deflate_pass and the stored blocks write from body[2] on, behind the header
   for (uint32_t k = tid; k < n + 16; k += kThreads) sm.in[k] = k < n ? in_g[k] : 0;
   for (int e = tid; e < 512 + (int)kMaxMatch + 1; e += kThreads) {
     if (e < 512) {                                   // zlib's d_code: entry d - 1 for d <= 256, 256 + ((d - 1) >> 7) above
@@ -419,41 +432,69 @@ __global__ void __launch_bounds__(kThreads, 1) deflate_kernel(const uint8_t* __r
     }
   }
   __syncthreads();
-  // Adler-32: one chunk per thread
+  // the checksum: one chunk per thread; Adler-32 parts add up, CRC-32 parts combine pairwise in a fixed tree
   {
     const uint32_t chunk = (n + kThreads - 1) / kThreads, s = min(tid * chunk, n), m = min(chunk, n - s);
-    AdlerPart ad = adler_chunk(sm.in, n, s, m);
-    for (int d = 16; d; d >>= 1) { ad.a += __shfl_xor_sync(0xffffffffu, ad.a, d); ad.b += __shfl_xor_sync(0xffffffffu, ad.b, d); }
-    if (lane == 0) { sm.adler_a[warp] = ad.a; sm.adler_b[warp] = ad.b; }
+    if (kC == Container::kZlib) {
+      AdlerPart ad = adler_chunk(sm.in, n, s, m);
+      for (int d = 16; d; d >>= 1) { ad.a += __shfl_xor_sync(0xffffffffu, ad.a, d); ad.b += __shfl_xor_sync(0xffffffffu, ad.b, d); }
+      if (lane == 0) { sm.adler_a[warp] = ad.a; sm.adler_b[warp] = ad.b; }
+    } else {
+      uint32_t crc = crc32_chunk(sm.in, s, m), len = m;
+      for (int d = 1; d < 32; d <<= 1) {             // lane l (a multiple of 2d) takes on lanes [l + d, l + 2d)
+        const uint32_t c2 = __shfl_down_sync(0xffffffffu, crc, d), l2 = __shfl_down_sync(0xffffffffu, len, d);
+        if (!(lane & (2 * d - 1))) { crc = crc32_combine(crc, c2, l2); len += l2; }
+      }
+      if (lane == 0) { sm.crc_part[warp] = crc; sm.crc_len[warp] = len; }
+    }
   }
-  deflate_pass<false>(sm, n, out, 0);
-  uint32_t adler = 0;
-  if (tid == 0) {
-    uint64_t a = 0, b = 0;
-    for (int w = 0; w < 32; ++w) { a += sm.adler_a[w]; b += sm.adler_b[w]; }
-    adler = adler_value(a, b, n);
+  deflate_pass<false>(sm, n, body, 0);
+  uint32_t check = 0;
+  if (kC == Container::kZlib) {
+    if (tid == 0) {
+      uint64_t a = 0, b = 0;
+      for (int w = 0; w < 32; ++w) { a += sm.adler_a[w]; b += sm.adler_b[w]; }
+      check = adler_value(a, b, n);
+    }
+  } else if (warp == 0) {                            // the same tree over the 32 warps' parts
+    uint32_t crc = sm.crc_part[lane], len = sm.crc_len[lane];
+    for (int d = 1; d < 32; d <<= 1) {
+      const uint32_t c2 = __shfl_down_sync(0xffffffffu, crc, d), l2 = __shfl_down_sync(0xffffffffu, len, d);
+      if (!(lane & (2 * d - 1))) { crc = crc32_combine(crc, c2, l2); len += l2; }
+    }
+    check = crc;
   }
-  const uint64_t zbytes = 2 + (sm.total_bits + 7) / 8 + 4;
-  uint64_t len;
-  if (zbytes <= bound) {
-    deflate_pass<true>(sm, n, out, (uint32_t)(bound - 4));
+  const uint32_t nb = n ? (n + 65534) / 65535 : 1;   // stored blocks of the input
+  const uint64_t stored = kHead + 5ull * nb + n + kTail;
+  const uint64_t zbytes = kHead + (sm.total_bits + 7) / 8 + kTail;
+  uint64_t len;                                      // bytes of body: 2 + the deflate blocks
+  if (zbytes <= stored) {
+    deflate_pass<true>(sm, n, body, (uint32_t)(stored - kTail - (kHead - 2)));
     len = sm.outpos;
-    if (tid == 0 && sm.wbit) out[len] = (uint8_t)sm.win[0];
+    if (tid == 0 && sm.wbit) body[len] = (uint8_t)sm.win[0];
     len += sm.wbit ? 1 : 0;
   } else {                                           // stored blocks of <= 65535 bytes: BFINAL/BTYPE byte, LEN, NLEN, the bytes
-    const uint32_t nb = n ? (n + 65534) / 65535 : 1;
-    for (uint32_t k = tid; k < n; k += kThreads) out[2 + 5 * (k / 65535 + 1) + k] = sm.in[k];
+    for (uint32_t k = tid; k < n; k += kThreads) body[2 + 5 * (k / 65535 + 1) + k] = sm.in[k];
     if ((uint32_t)tid < nb) {
       const uint32_t ln = min(65535u, n - tid * 65535u), o = 2 + tid * (65535u + 5);
-      out[o] = tid == (int)nb - 1;
-      out[o + 1] = ln & 255; out[o + 2] = ln >> 8; out[o + 3] = ~ln & 255; out[o + 4] = (~ln >> 8) & 255;
+      body[o] = tid == (int)nb - 1;
+      body[o + 1] = ln & 255; body[o + 2] = ln >> 8; body[o + 3] = ~ln & 255; body[o + 4] = (~ln >> 8) & 255;
     }
     len = 2 + 5ull * nb + n;
   }
-  if (tid == 0) {                                    // zlib header (deflate, 32 KB window, FCHECK) and the big-endian Adler-32
-    out[0] = 0x78; out[1] = 0x01;
-    out[len] = adler >> 24; out[len + 1] = (adler >> 16) & 255; out[len + 2] = (adler >> 8) & 255; out[len + 3] = adler & 255;
-    lengths[i] = (uint32_t)(len + 4);
+  if (tid == 0) {
+    uint8_t* t = body + len;
+    if (kC == Container::kZlib) {                    // zlib header (deflate, 32 KB window, FCHECK) and the big-endian Adler-32
+      out[0] = 0x78; out[1] = 0x01;
+      t[0] = check >> 24; t[1] = (check >> 16) & 255; t[2] = (check >> 8) & 255; t[3] = check & 255;
+    } else {                                         // gzip header: deflate, FEXTRA, MTIME 0, XFL 0, OS 255, XLEN 6, BC, BSIZE
+      const uint32_t bsize = (uint32_t)(kHead - 2 + len + kTail - 1);
+      const uint8_t h[16] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0};
+      for (int k = 0; k < 16; ++k) out[k] = h[k];
+      out[16] = bsize & 255; out[17] = bsize >> 8;
+      for (int k = 0; k < 4; ++k) { t[k] = (check >> (8 * k)) & 255; t[4 + k] = (n >> (8 * k)) & 255; }
+    }
+    lengths[i] = (uint32_t)(kHead - 2 + len + kTail);
     status[i] = DAN_DEFLATE_OK;
   }
 }
@@ -478,16 +519,30 @@ __global__ void __launch_bounds__(1024) compact_offsets_kernel(const uint32_t* _
   if (tid == 0) offsets[n] = carry;
 }
 
-__global__ void compact_copy_kernel(const uint8_t* __restrict__ slots, uint64_t bound, const uint32_t* __restrict__ lengths,
+__global__ void compact_copy_kernel(const uint8_t* __restrict__ slots, uint64_t stride, const uint32_t* __restrict__ lengths,
                                     const uint64_t* __restrict__ offsets, uint8_t* __restrict__ dst) {
   const uint64_t i = blockIdx.x;
-  const uint8_t* s = slots + i * bound;
+  const uint8_t* s = slots + i * stride;
   uint8_t* d = dst + offsets[i];
-  const uint64_t len = min((uint64_t)lengths[i], bound);
+  const uint64_t len = min((uint64_t)lengths[i], stride);
   for (uint64_t k = threadIdx.x; k < len; k += blockDim.x) d[k] = s[k];
 }
 
-DanSmemAttr g_deflate_smem;
+// dan_deflate_compact and dan_bgzf_compact: the outputs of n slots `stride` bytes apart, back to back
+int compact(const void* slots, uint64_t stride, const uint32_t* lengths, int n, void* dst, uint64_t* offsets, void* stream) {
+  if (n < 0) { dan_set_error("negative stream count"); return DAN_E_INVALID; }
+  if (!offsets) { dan_set_error("null pointer"); return DAN_E_INVALID; }
+  if (n > 0 && (!slots || !lengths || !dst)) { dan_set_error("null pointer"); return DAN_E_INVALID; }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  compact_offsets_kernel<<<1, 1024, 0, st>>>(lengths, n, offsets);
+  DAN_CUDA_TRY(cudaGetLastError());
+  if (n == 0) return DAN_OK;
+  compact_copy_kernel<<<n, 256, 0, st>>>(static_cast<const uint8_t*>(slots), stride, lengths, offsets, static_cast<uint8_t*>(dst));
+  DAN_CUDA_TRY(cudaGetLastError());
+  return DAN_OK;
+}
+
+DanSmemAttr g_deflate_smem, g_bgzf_smem;
 
 }  // namespace
 
@@ -504,25 +559,34 @@ extern "C" int dan_deflate_device(const void* src, int n, uint64_t slot_bytes, v
   }
   if (n == 0) return DAN_OK;
   if ((!src && slot_bytes) || !dst || !lengths || !status) { dan_set_error("null pointer"); return DAN_E_INVALID; }
-  DAN_CUDA_TRY(g_deflate_smem.ensure(deflate_kernel, sizeof(Smem)));
-  deflate_kernel<<<n, kThreads, sizeof(Smem), static_cast<cudaStream_t>(stream)>>>(static_cast<const uint8_t*>(src), slot_bytes,
-                                                                                    static_cast<uint8_t*>(dst), dan_deflate_bound(slot_bytes),
-                                                                                    lengths, status);
+  DAN_CUDA_TRY(g_deflate_smem.ensure(deflate_kernel<Container::kZlib>, sizeof(Smem)));
+  deflate_kernel<Container::kZlib><<<n, kThreads, sizeof(Smem), static_cast<cudaStream_t>(stream)>>>(
+      static_cast<const uint8_t*>(src), slot_bytes, (uint64_t)n * slot_bytes, static_cast<uint8_t*>(dst), dan_deflate_bound(slot_bytes),
+      lengths, status);
   DAN_CUDA_TRY(cudaGetLastError());
   return DAN_OK;
 }
 
 extern "C" int dan_deflate_compact(const void* slots, const uint32_t* lengths, int n, uint64_t slot_bytes, void* dst, uint64_t* offsets,
                                    void* stream) {
-  if (n < 0) { dan_set_error("negative stream count"); return DAN_E_INVALID; }
-  if (!offsets) { dan_set_error("null pointer"); return DAN_E_INVALID; }
-  if (n > 0 && (!slots || !lengths || !dst)) { dan_set_error("null pointer"); return DAN_E_INVALID; }
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  compact_offsets_kernel<<<1, 1024, 0, st>>>(lengths, n, offsets);
-  DAN_CUDA_TRY(cudaGetLastError());
-  if (n == 0) return DAN_OK;
-  compact_copy_kernel<<<n, 256, 0, st>>>(static_cast<const uint8_t*>(slots), dan_deflate_bound(slot_bytes), lengths, offsets,
-                                         static_cast<uint8_t*>(dst));
+  return compact(slots, dan_deflate_bound(slot_bytes), lengths, n, dst, offsets, stream);
+}
+
+static_assert(DAN_BGZF_MAX_INPUT <= kMaxSlot && 18 + 5 + DAN_BGZF_MAX_INPUT + 8 <= DAN_BGZF_MAX_BLOCK,
+              "a BGZF piece must fit in shared memory and its stored encoding in one slot");
+
+extern "C" int dan_bgzf_compress_device(const void* src, uint64_t bytes, void* dst, uint32_t* block_lengths, int32_t* status, void* stream) {
+  if (bytes == 0) return DAN_OK;
+  if (!src || !dst || !block_lengths || !status) { dan_set_error("null pointer"); return DAN_E_INVALID; }
+  const uint64_t n = (bytes + DAN_BGZF_MAX_INPUT - 1) / DAN_BGZF_MAX_INPUT;
+  if (n > 0x7fffffffull) { dan_set_error("%llu bytes make more than 2^31 - 1 BGZF blocks", (unsigned long long)bytes); return DAN_E_INVALID; }
+  DAN_CUDA_TRY(g_bgzf_smem.ensure(deflate_kernel<Container::kBgzf>, sizeof(Smem)));
+  deflate_kernel<Container::kBgzf><<<(unsigned)n, kThreads, sizeof(Smem), static_cast<cudaStream_t>(stream)>>>(
+      static_cast<const uint8_t*>(src), DAN_BGZF_MAX_INPUT, bytes, static_cast<uint8_t*>(dst), DAN_BGZF_MAX_BLOCK, block_lengths, status);
   DAN_CUDA_TRY(cudaGetLastError());
   return DAN_OK;
+}
+
+extern "C" int dan_bgzf_compact(const void* slots, const uint32_t* lengths, int n, void* dst, uint64_t* offsets, void* stream) {
+  return compact(slots, DAN_BGZF_MAX_BLOCK, lengths, n, dst, offsets, stream);
 }

@@ -1,5 +1,5 @@
 // dan_zlib.cuh — what the inflate (dan_inflate.cu) and deflate (dan_deflate.cu) kernels share: the DEFLATE (RFC 1951) length / distance
-// base and extra-bit tables, the code-length code order, and the chunked Adler-32 (RFC 1950) of a buffer.
+// base and extra-bit tables, the code-length code order, the chunked Adler-32 (RFC 1950) and the chunked CRC-32 (RFC 1952) of a buffer.
 #pragma once
 #include <cstdint>
 
@@ -33,4 +33,38 @@ __device__ inline AdlerPart adler_chunk(const uint8_t* data, uint64_t total, uin
 __device__ inline uint32_t adler_value(uint64_t a_sum, uint64_t b_sum, uint64_t total) {
   const uint32_t A = (uint32_t)((1 + a_sum) % kAdlerMod), B = (uint32_t)((total % kAdlerMod + b_sum) % kAdlerMod);
   return (B << 16) | A;
+}
+
+// CRC-32 (IEEE 802.3, reflected, as gzip and zlib.crc32) of data[0, total) in independent chunks: each chunk's own CRC (crc32_chunk),
+// then, in a fixed order, crc(A B) = crc(A) * x^(8 |B|) mod P ^ crc(B) (crc32_combine, zlib's crc32_combine).
+constexpr uint32_t kCrcPoly = 0xedb88320u;
+
+__device__ inline uint32_t crc32_chunk(const uint8_t* data, uint64_t s, uint64_t m) {
+  uint32_t c = 0xffffffffu;
+  for (uint64_t k = 0; k < m; ++k) {
+    c ^= data[s + k];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) c = (c >> 1) ^ (kCrcPoly & (0u - (c & 1u)));
+  }
+  return ~c;
+}
+
+// a * b modulo P, in the reflected representation (bit 31 is x^0)
+__device__ inline uint32_t crc32_multmodp(uint32_t a, uint32_t b) {
+  uint32_t p = 0;
+  for (uint32_t m = 1u << 31; m; m >>= 1) {
+    if (a & m) { p ^= b; if (!(a & (m - 1))) break; }
+    b = (b & 1u) ? (b >> 1) ^ kCrcPoly : b >> 1;
+  }
+  return p;
+}
+
+// the CRC-32 of A followed by B from crc_a, crc_b and the length of B
+__device__ inline uint32_t crc32_combine(uint32_t crc_a, uint32_t crc_b, uint64_t len_b) {
+  uint32_t p = 1u << 31, sq = 1u << 23;                // x^0 and x^8
+  for (; len_b; len_b >>= 1) {                         // p = x^(8 len_b) by square-and-multiply
+    if (len_b & 1) p = crc32_multmodp(sq, p);
+    if (len_b > 1) sq = crc32_multmodp(sq, sq);
+  }
+  return crc32_multmodp(p, crc_a) ^ crc_b;
 }

@@ -325,6 +325,23 @@ int dan_deflate_device(const void* src, int n, uint64_t slot_bytes, void* dst, u
  * cudaMemcpyAsync of offsets[n] bytes carries only the compressed bytes to the host. */
 int dan_deflate_compact(const void* slots, const uint32_t* lengths, int n, uint64_t slot_bytes, void* dst, uint64_t* offsets, void* stream);
 
+/* BGZF compression on the device, with dan_deflate_device's kernel in gzip framing. src[0, bytes) is cut as bgzip cuts it: into
+ * n = ceil(bytes / DAN_BGZF_MAX_INPUT) pieces of DAN_BGZF_MAX_INPUT bytes, the last one shorter. Piece i becomes one complete BGZF block
+ * in dst + i * DAN_BGZF_MAX_BLOCK: the 18-byte gzip header (1f 8b 08 04, MTIME 0, XFL 0, OS ff, XLEN 6, subfield 'B' 'C' with SLEN 2 and
+ * BSIZE = block size - 1), raw DEFLATE (dynamic-Huffman blocks, or one stored block when that is smaller; at most 18 + 5 + 65280 + 8 =
+ * 65311 bytes in all), then the CRC-32 and ISIZE of the piece, all little-endian. block_lengths[i] receives the block's size and
+ * status[i] DAN_DEFLATE_OK. The CRC-32 is computed in chunks and combined in a fixed order, so a block's bytes depend only on its
+ * piece: not on the other pieces, the launch or the device. All pointers are DEVICE pointers (dst: n * DAN_BGZF_MAX_BLOCK bytes,
+ * block_lengths and status: n entries); asynchronous on `stream`. bytes = 0 makes no blocks and launches nothing; otherwise a null
+ * pointer returns DAN_E_INVALID before any launch. The 28-byte empty EOF block that ends a BGZF file is the caller's to append. */
+#define DAN_BGZF_MAX_INPUT 65280
+#define DAN_BGZF_MAX_BLOCK 65536
+int dan_bgzf_compress_device(const void* src, uint64_t bytes, void* dst, uint32_t* block_lengths, int32_t* status, void* stream);
+
+/* Packs the n blocks of dan_bgzf_compress_device back to back, as dan_deflate_compact does with slots DAN_BGZF_MAX_BLOCK apart:
+ * offsets (DEVICE, n + 1 u64) receives the exclusive prefix sum of lengths and block i moves to dst + offsets[i]. */
+int dan_bgzf_compact(const void* slots, const uint32_t* lengths, int n, void* dst, uint64_t* offsets, void* stream);
+
 /* ---- device decode, of raw (DAN_RECORDS_RAW) or compressed (DAN_RECORDS_ZLIB) records --------------------------------------------
  * The caller stages the n records of a call in one pinned HOST buffer, at the offsets dan_decode_layout reports. The regions come in
  * this order, each 16-byte aligned, at offsets that depend only on (format, n); a region the format does not use is empty:
